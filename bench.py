@@ -46,7 +46,32 @@ def parse():
                     help="multi-GPU restart loop: per-round balancing (hbegp_fit_runs_sharded) or a static split of the runs")
     ap.add_argument("--only", default="all", choices=["all", "fit-step", "predict"],
                     help="profiling aid: run just the timed fit steps or just the timed prediction, print a short line")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed fit step and the last timed prediction returned as DIR/<name>.npy "
+                         "(rank 0; with several ranks the prediction is rank 0's block of rows)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(directory, arrays):
+    """Writes each array as directory/<name>.npy in float64 (float32 results stay float32), DUMP_BYTES in all: an array
+    whose share would be exceeded is cut to a fixed, seeded sample of its rows, so that two builds run with the same
+    arguments are compared on the same entries."""
+    os.makedirs(directory, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if a.dtype not in (np.float32, np.float64):
+            a = a.astype(np.float64)
+        if a.nbytes > share:
+            rows = np.random.default_rng(0).choice(len(a), share // (a.nbytes // len(a)), replace=False)
+            a = a[np.sort(rows)]
+        np.save(os.path.join(directory, f"{name}.npy"), a)
 
 
 def synth(n, d, seed=1, A=np.float64):
@@ -268,8 +293,15 @@ def main():
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
+
+    def fit_outputs(gathered):
+        lml, grad, status = gathered
+        return {"lml": lml, "lml_grad": grad, "status": status}
+
     if args.only == "fit-step":
-        ms_step, launches, _ = timed(step_resident, args.steps, args.warmup)
+        ms_step, launches, gathered = timed(step_resident, args.steps, args.warmup)
+        if rank == 0 and args.dump_outputs:
+            dump_outputs(args.dump_outputs, fit_outputs(gathered))
         if rank == 0:
             print(json.dumps({"only": "fit-step", "ms_per_step": ms_step, "evals_per_s": B / (ms_step * 1e-3),
                               "gpu_launches": int(launches), "clocks": sampler.stop()}), flush=True)
@@ -308,6 +340,10 @@ def main():
 
     psteps = max(2, min(args.steps, 3))
     ms_pred, pred_launches, _ = timed(predict_resident, psteps, 1)
+    if rank == 0 and args.dump_outputs:
+        outputs = {} if args.only == "predict" else fit_outputs(gathered)
+        outputs.update({"predict_mean": mean_dev.cpu().numpy(), "predict_var": var_dev.cpu().numpy()})
+        dump_outputs(args.dump_outputs, outputs)
     ms_pred_mean, _, _ = timed(predict_mean_resident, psteps, 1)
     if args.only == "predict":
         if rank == 0:

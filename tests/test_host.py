@@ -155,6 +155,24 @@ def test_gpu_arm_of_bench_does_not_import_the_oracle():
             assert "oracle/" not in open(path).read(), fn
 
 
+def test_bench_dump_outputs_are_float_within_budget_and_sampled_the_same_way(tmp_path, monkeypatch):
+    import bench
+    monkeypatch.setattr(bench, "DUMP_BYTES", 1 << 20)
+    arrays = {"lml": np.arange(65.0), "status": np.zeros(65, dtype=np.int32),
+              "mean": np.random.default_rng(1).random(1 << 18), "var": np.random.default_rng(2).random(1 << 18).astype(np.float32)}
+    for sub in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / sub), arrays)
+    got = {f.stem: np.load(f) for f in (tmp_path / "a").iterdir()}
+    assert sorted(got) == sorted(arrays)
+    assert got["status"].dtype == np.float64 and got["var"].dtype == np.float32 and got["mean"].dtype == np.float64
+    np.testing.assert_array_equal(got["lml"], arrays["lml"])
+    assert sum(a.nbytes for a in got.values()) <= 1 << 20
+    rows = np.flatnonzero(np.isin(arrays["mean"], got["mean"]))  # a subset of the rows, in their order
+    np.testing.assert_array_equal(arrays["mean"][rows], got["mean"])
+    for name, a in got.items():
+        np.testing.assert_array_equal(np.load(tmp_path / "b" / f"{name}.npy"), a)
+
+
 def test_c_abi_rejects_bad_arguments_without_crashing():
     """Every entry point returns a status (< 0 with a message) instead of aborting (SURVEY 8 b4 / b6)."""
     from hbetune_rs_b200 import _lib
