@@ -1046,9 +1046,11 @@ struct ModelT : Model {
         if ((rc = part.ensure((size_t)chunk * (np / TILE) * sizeof(T)))) return rc;  // one partial per 64-wide column tile at most
         for (long row0 = 0; row0 < m; row0 += chunk) {
             const int rows = (int)std::min<long>(chunk, round_up(m - row0, 128));
-            // column-tile width of the variance GEMM: must be the one launch_gemm_auto picks for exactly this shape
-            const bool tf = gemm_uses_tf32<T>(rows, np, w_aligned128, 5);
-            const int bn = tf ? 128 : pick_gemm_tile<T>(128, np);  // rows are always a multiple of 128
+            // The variance kernel is chosen from np alone, never from the row count: a candidate's variance then has
+            // the same bits however many rows are predicted with it (f32: 3xTF32 or FFMA sum in different orders).
+            // rows is a multiple of 128, so the TF32 tiles are full in M even when rows < 256.
+            const bool tf = gemm_uses_tf32<T>(np, np, w_aligned128, 5);
+            const int bn = tf ? 128 : pick_gemm_tile<T>(128, np);
             const int ntile = (np + bn - 1) / bn;
             T* pm = nullptr;
             if (ns > 1) {
@@ -1068,7 +1070,10 @@ struct ModelT : Model {
             g.rowsumsq = (T*)part.p; g.ld_rs = ntile; g.s_rs = 0;
             // keep ~48 MB of k* rows resident in L2 while W streams (ncu before: 35 GB of DRAM reads per 1 GB chunk)
             g.raster_group = (int)std::max<size_t>(1, ((size_t)48 << 20) / ((size_t)bn * np * sizeof(T)));
-            CUDA_TRY((launch_gemm_auto<T, true, true>(g, 1, st, w_aligned128, 5)));
+            if constexpr (std::is_same<T, float>::value) {
+                if (tf) CUDA_TRY((tf32::launch<true, true>(g, 1, st)));
+                else CUDA_TRY((launch_gemm<T, true, true>(g, 1, st)));
+            } else CUDA_TRY((launch_gemm<T, true, true>(g, 1, st)));
             e->launches++;
             k_var_finish<T><<<(rows + 255) / 256, 256, 0, st>>>((const T*)part.p, ntile, ntile, rows, m, row0, (T)c, var, nb, pm, ns, rows, mean,
                                                                 (long*)warn_rows.p, (T*)warn_vals.p, kWarnCap);
