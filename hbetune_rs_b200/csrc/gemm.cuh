@@ -72,11 +72,6 @@ __device__ __forceinline__ void dmma884(double& c0, double& c1, double a, double
                  : "d"(a), "d"(b));
 }
 
-// 1: early-fragment main loop for f64 (default; +2..6 % on B200, probes/gemm_early.cu), 0: the plain loop
-#ifndef HBEGP_EARLY
-#define HBEGP_EARLY 1
-#endif
-
 template <typename T, int BM, int BN, int WM, int WN, bool A_KMAJOR, bool B_KMAJOR, int BK_ = HBEGP_BK, int STAGES_ = HBEGP_STAGES>
 struct GemmCfg {
     static constexpr int BK = BK_;
@@ -201,10 +196,10 @@ __global__ void __launch_bounds__(GemmCfg<T, BM, BN, WM, WN, A_KMAJOR, B_KMAJOR,
     // warp-tile-relative row of accumulator slot i / column of slot j (see the two micro-kernels below)
     auto row_of = [&](int i) { return (F64 || A_KMAJOR) ? i * 8 + lr : FM * lr + i; };
     auto col_of = [&](int j) { return F64 ? j * 8 + 2 * lc : (B_KMAJOR ? j * 4 + lc : FN * lc + j); };
-#if HBEGP_EARLY
-    // Early-fragment variant (f64): the barrier of iteration kt also publishes stage kt + 1, so the operand fragments
+    // Early-fragment main loop (f64): the barrier of iteration kt also publishes stage kt + 1, so the operand fragments
     // of the first k4 step of the next stage are fetched during this iteration and no shared-memory latency sits
-    // between the barrier and the first DMMA.
+    // between the barrier and the first DMMA.  Measured +2..6 % on B200 against a loop that loads every fragment after
+    // the barrier (profiles/r01_gemm_early_probe.log).
     T a_n[FM], b_n[FN];
     auto load_frag = [&](const T* sA, const T* sB, int ks, T* a, T* b) {
         const int k = ks * 4 + lc;
@@ -224,21 +219,15 @@ __global__ void __launch_bounds__(GemmCfg<T, BM, BN, WM, WN, A_KMAJOR, B_KMAJOR,
         __syncthreads();
         if (nk > 0) load_frag(smem, smem + Cfg::A_ELEMS, 0, a_n, b_n);
     }
-#endif
     for (int kt = 0; kt < nk; kt++) {
-#if HBEGP_EARLY
         if constexpr (F64) cp_async_wait<(STAGES >= 3 ? STAGES - 3 : 0)>();
         else cp_async_wait<STAGES - 2>();
-#else
-        cp_async_wait<STAGES - 2>();
-#endif
         __syncthreads();
         if (kt + STAGES - 1 < nk) issue(kt + STAGES - 1);
         cp_async_commit();
         const T* sA = smem + (kt % STAGES) * Cfg::STAGE_ELEMS;
         const T* sB = sA + Cfg::A_ELEMS;
         if constexpr (F64) {
-#if HBEGP_EARLY
 #pragma unroll
             for (int ks = 0; ks < BK / 4; ks++) {
                 T a[FM], b[FN];
@@ -259,27 +248,6 @@ __global__ void __launch_bounds__(GemmCfg<T, BM, BN, WM, WN, A_KMAJOR, B_KMAJOR,
                 const T* nA = smem + ((kt + 1) % STAGES) * Cfg::STAGE_ELEMS;
                 load_frag(nA, nA + Cfg::A_ELEMS, 0, a_n, b_n);
             }
-#else
-#pragma unroll
-            for (int ks = 0; ks < BK / 4; ks++) {
-                T a[FM], b[FN];
-                const int k = ks * 4 + lc;
-#pragma unroll
-                for (int i = 0; i < FM; i++) {
-                    int row = wm * WM + i * 8 + lr;
-                    a[i] = A_KMAJOR ? sA[row * Cfg::A_STRIDE + k] : sA[k * Cfg::A_STRIDE + row];
-                }
-#pragma unroll
-                for (int j = 0; j < FN; j++) {
-                    int col = wn * WN + j * 8 + lr;
-                    b[j] = B_KMAJOR ? sB[col * Cfg::B_STRIDE + k] : sB[k * Cfg::B_STRIDE + col];
-                }
-#pragma unroll
-                for (int i = 0; i < FM; i++)
-#pragma unroll
-                    for (int j = 0; j < FN; j++) dmma884(acc[i][j][0], acc[i][j][1], a[i], b[j]);
-            }
-#endif
         } else {
             // FP32 (FFMA): (WM/8) x (WN/4) outputs per thread — 4 x 8 for the 64x64 tile, 8 x 8 for 128x128 —
             // operands fetched four k at a time with 16-byte shared loads.  Thread-to-row/column mapping follows
@@ -402,31 +370,10 @@ inline cudaError_t launch_gemm_cfg(const GemmArgs<T>& a, int batch, cudaStream_t
 // CTA tile choice.  Measured on B200 (probes/gemm_bench.cu, profiles/r01_gemm_tile_probe.log): the 64x64 tile
 // (4 warps, 32x32 warp tiles, 60 KB of shared memory -> 3 CTAs per SM) sustains 33.2 TFLOP/s on 2048^3 x 4
 // against 31.0 for 128x128 (8 warps, 1 CTA per SM) and 35.6 for cuBLAS, and it quantises far better on the
-// small and triangular grids of the recursion, so it is the default; HBEGP_TILE=128 selects the large tile
-// where a problem tiles evenly.
-inline int& gemm_tile_pref() {
-    static int pref = 64;
-    return pref;
-}
-
-// f32: the 128x128 configuration (8 x 8 outputs per thread) has the better FFMA-to-load ratio on paper but
-// measures slower than 64x64 (north-star step 124.7 ms vs 113.8 ms, predict 455 vs 413 ms), so 64x64 is the
-// default here too; HBEGP_TILE32=128 selects the large tile.
-inline int& gemm_tile_pref_f32() {
-    static int pref = 64;
-    return pref;
-}
-
-template <typename T = double>
-inline int pick_gemm_tile(int M, int N) {
-    const int pref = std::is_same<T, float>::value ? gemm_tile_pref_f32() : gemm_tile_pref();
-    return (pref == 128 && M % 128 == 0 && N % 128 == 0) ? 128 : 64;
-}
-
-// warp-tile height of the 128x128 configuration: 64x32 warp tiles (f64: 8 x 4 DMMA tiles; f32: 8 x 8 per thread)
-template <typename T>
-constexpr int wm128() { return 64; }
-
+// small and triangular grids of the recursion.  In f32 the 128x128 configuration (8 x 8 outputs per thread) has the
+// better FFMA-to-load ratio on paper but measured slower as well (north-star step 124.7 ms vs 113.8 ms, predict 455
+// vs 413 ms).  So the large products run on 64x64 tiles in both precisions.
+//
 // Latency-bound products (the bottom levels of the recursion at small n, small batches): a 64x64 tile puts its whole k
 // loop on ONE SM's FP64 pipe (0.52 us per 16-k step) while most of the 148 SMs idle.  When the caller allows it
 // (GemmArgs::small_ctas) and the 64x64 grid would have at most that many CTAs, the product runs on 32x32 tiles instead
@@ -438,16 +385,13 @@ constexpr int wm128() { return 64; }
 // so the engine only allows it up to n = 1024.
 template <typename T, bool AK, bool BK_>
 inline cudaError_t launch_gemm(const GemmArgs<T>& a, int batch, cudaStream_t stream) {
-    if (pick_gemm_tile<T>(a.M, a.N) == 128) return launch_gemm_cfg<T, 128, 128, wm128<T>(), 32, AK, BK_>(a, batch, stream);
-    {
-        const long tm = a.M / 64, tn = a.N / 64;
-        const long tiles = a.lower_only ? tm * (tm + 1) / 2 : tm * tn;
-        if (a.rowsumsq == nullptr && a.raster_group == 0 && tiles * batch <= a.small_ctas) {
-            // f64: 4 warps of 16x16 (2 x 2 DMMA tiles); f32: 2 warps of 32x16 (4 x 4 outputs per thread, the smallest
-            // warp tile of the FFMA micro-kernel)
-            if constexpr (std::is_same<T, double>::value) return launch_gemm_cfg<T, 32, 32, 16, 16, AK, BK_>(a, batch, stream);
-            else return launch_gemm_cfg<T, 32, 32, 32, 16, AK, BK_>(a, batch, stream);
-        }
+    const long tm = a.M / 64, tn = a.N / 64;
+    const long tiles = a.lower_only ? tm * (tm + 1) / 2 : tm * tn;
+    if (a.rowsumsq == nullptr && a.raster_group == 0 && tiles * batch <= a.small_ctas) {
+        // f64: 4 warps of 16x16 (2 x 2 DMMA tiles); f32: 2 warps of 32x16 (4 x 4 outputs per thread, the smallest
+        // warp tile of the FFMA micro-kernel)
+        if constexpr (std::is_same<T, double>::value) return launch_gemm_cfg<T, 32, 32, 16, 16, AK, BK_>(a, batch, stream);
+        else return launch_gemm_cfg<T, 32, 32, 32, 16, AK, BK_>(a, batch, stream);
     }
     return launch_gemm_cfg<T, 64, 64, 32, 32, AK, BK_>(a, batch, stream);
 }

@@ -40,14 +40,10 @@ namespace tf32 {
 // (the tensor pipe itself needs 1250).  Measured and rejected on the way: eight transform warps (145 vs 151 TFLOP/s), eight
 // drain warps (107 vs 113 at the time), descriptors hoisted out of the issue loop (no change).
 // Stage depth: 32 k per stage (128-byte rows, three 64 KB stages).  A finer ring -- 16 k per stage, six 32 KB stages, 64-byte
-// rows with SWIZZLE_64B -- was measured as well (compile with -DHBEGP_TF32_BK=16): 120-125 TFLOP/s against 132-137 on
-// 4096^3; the doubled number of barrier hand-shakes costs more than the shorter slot residence gains.
-#ifndef HBEGP_TF32_BK
-#define HBEGP_TF32_BK 32
-#endif
-constexpr int BM = 128, BN = 128, BK = HBEGP_TF32_BK, STAGES = 192 / (BK * 2);
-static_assert(BK == 16 || BK == 32, "BK: 16 (64-byte rows, SWIZZLE_64B) or 32 (128-byte rows, SWIZZLE_128B)");
-constexpr int TILE_BYTES = BM * BK * 4;  // one operand tile (hi or lo): 8 KB (BK = 16) or 16 KB
+// rows with SWIZZLE_64B -- was measured as well: 120-125 TFLOP/s against 132-137 on 4096^3; the doubled number of barrier
+// hand-shakes costs more than the shorter slot residence gains.
+constexpr int BM = 128, BN = 128, BK = 32, STAGES = 3;
+constexpr int TILE_BYTES = BM * BK * 4;  // one operand tile (hi or lo): 16 KB
 constexpr int STAGE_BYTES = 4 * TILE_BYTES;  // A_hi, A_lo, B_hi, B_lo
 constexpr int MN_BOX_BYTES = 32 * BK * 4;    // one TMA box of a row-major operand: BK k-rows x 32 rows (128 bytes)
 constexpr int THREADS = 320;
@@ -273,9 +269,7 @@ __global__ void __launch_bounds__(THREADS, 1) gemm_tf32x3_kernel(const __grid_co
             // inside the swizzled row.
             // MN-major (per 32-row box: 32 k-rows x 128 bytes of rows): 32-row groups 4096 bytes apart (LBO), groups of
             // 4 k-rows 512 bytes apart (SBO); one k step of 8 = 1024 bytes.
-            // (BK = 16: K-major rows are 64 bytes, SWIZZLE_64B, 8-row groups 512 bytes apart; MN-major boxes hold 16 k-rows,
-            // so the 32-row groups are 2048 bytes apart.)
-            constexpr uint32_t k_sbo = 8 * BK * 4, k_lay = (BK == 32) ? 2 : 4;  // SWIZZLE_128B / SWIZZLE_64B
+            constexpr uint32_t k_sbo = 8 * BK * 4, k_lay = 2;  // SWIZZLE_128B
             constexpr uint32_t a_lbo = A_KMAJOR ? 16 : MN_BOX_BYTES, a_sbo = A_KMAJOR ? k_sbo : 512, a_kstep = A_KMAJOR ? 32 : 1024;
             constexpr uint32_t b_lbo = B_KMAJOR ? 16 : MN_BOX_BYTES, b_sbo = B_KMAJOR ? k_sbo : 512, b_kstep = B_KMAJOR ? 32 : 1024;
             constexpr uint32_t a_lay = A_KMAJOR ? k_lay : 1, b_lay = B_KMAJOR ? k_lay : 1;
@@ -339,7 +333,7 @@ __global__ void __launch_bounds__(THREADS, 1) gemm_tf32x3_kernel(const __grid_co
         // accumulation, always the same sign.  Accumulating k = 4096 in TMEM loses 2.7e-5 on positive data (probe), and
         // even 64-k chunks (2e-7, less than the FFMA kernel's random rounding error) cost the f32 Cholesky its
         // positive-definiteness margin, because a systematic error does not average out over the recursion
-        // (tests/probes/f32_pd_boundary2.py: K stopped factoring at 4x the noise level the FFMA path reaches).  So
+        // (a probe: K stopped factoring at 4x the noise level the FFMA path reaches).  So
         // (almost) nothing is accumulated in TMEM for the hi*hi term: every KS_PER_BUF k steps (k = 16) start a fresh product
         // in one of NBUF rotating buffers, which is added round-to-nearest into registers here while the tensor core
         // fills the next.
@@ -444,7 +438,7 @@ inline bool make_operand_map(CUtensorMap* map, const float* base, bool kmajor, i
     cuuint32_t estr[3] = {1, 1, 1};
     CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(base), dims, strides, box, estr,
                      CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     kmajor ? (BK == 32 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B) : CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B,
+                     kmajor ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B,
                      CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     return r == CUDA_SUCCESS;
@@ -476,39 +470,29 @@ inline cudaError_t launch(const GemmArgs<float>& a, int batch, cudaStream_t stre
     return launch_prio(gemm_tf32x3_kernel<AK, BKM>, grid, dim3(THREADS), SMEM_BYTES, stream, p);
 }
 
-// Policy (process-wide, set by hbegp_ctx_create from HBEGP_TF32 / HBEGP_TF32_MIN): whether f32 contractions go through
-// the tensor path, and the smallest min(M, N) for which they do (below it one 128 x 128 tile per CTA leaves the GPU
-// emptier than the 64 x 64 FFMA tiles and the per-CTA pipeline start-up dominates).
+// Policy (process-wide, set by hbegp_ctx_create from HBEGP_TF32): whether f32 contractions go through the tensor path.
 inline bool& enabled() {
     static bool on = true;
     return on;
 }
-// bit i set: GEMM class i may use the tensor path (0 panel solve, 1 T = L21 W11, 2 trailing update, 3 W21 = -W22 T,
-// 4 K^-1 = W^T W, 5 predictive variance); a diagnostic switch (HBEGP_TF32_MASK)
-inline int& class_mask() {
-    static int v = 0x3f;
-    return v;
-}
-inline int& min_extent() {
-    static int v = 256;
-    return v;
-}
+// The smallest min(M, N) for which they do: below it one 128 x 128 tile per CTA leaves the GPU emptier than the 64 x 64
+// FFMA tiles and the per-CTA pipeline start-up dominates.
+constexpr int MIN_EXTENT = 256;
 
 }  // namespace tf32
 
-// Dispatch used by the engine: f64 -> DMMA kernel; f32 -> tcgen05 3xTF32 when the policy allows and the operands meet
-// the 128-wide-tile invariant (`aligned128`: every 128-wide diagonal block of a triangular operand has exact zeros
-// above its diagonal), else the FFMA kernel.
+// Dispatch used by the engine: f64 -> DMMA kernel; f32 -> tcgen05 3xTF32 when the policy allows, else the FFMA kernel.
+// The tensor path relies on the 128-wide-tile invariant of the recursion: every 128-wide diagonal block of a triangular
+// operand has exact zeros above its diagonal (the bottom nodes write them).
 template <typename T>
-inline bool gemm_uses_tf32(int M, int N, bool aligned128, int cls) {
-    return std::is_same<T, float>::value && tf32::enabled() && aligned128 && (M < N ? M : N) >= tf32::min_extent() &&
-           ((tf32::class_mask() >> cls) & 1);
+inline bool gemm_uses_tf32(int M, int N) {
+    return std::is_same<T, float>::value && tf32::enabled() && (M < N ? M : N) >= tf32::MIN_EXTENT;
 }
 
 template <typename T, bool AK, bool BKM>
-inline cudaError_t launch_gemm_auto(const GemmArgs<T>& a, int batch, cudaStream_t stream, bool aligned128, int cls) {
+inline cudaError_t launch_gemm_auto(const GemmArgs<T>& a, int batch, cudaStream_t stream) {
     if constexpr (std::is_same<T, float>::value) {
-        if (gemm_uses_tf32<T>(a.M, a.N, aligned128, cls)) return tf32::launch<AK, BKM>(a, batch, stream);
+        if (gemm_uses_tf32<T>(a.M, a.N)) return tf32::launch<AK, BKM>(a, batch, stream);
     }
     return launch_gemm<T, AK, BKM>(a, batch, stream);
 }

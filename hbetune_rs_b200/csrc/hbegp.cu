@@ -145,16 +145,6 @@ struct EngineBase {
     std::vector<cudaEvent_t> side_a, side_b;
     cudaStream_t main_side = nullptr;
     cudaEvent_t main_a = nullptr, main_b = nullptr;
-    bool use_side = true;
-    int side_max_cnt = 4;  // also use the side stream at n > 2048 for groups of at most this many matrices
-    bool use_node128 = true;
-    long small_tile_ctas = 296;  // 32x32 GEMM tiles for grids of at most this many 64x64 CTAs ...
-    int small_tile_np = 1024;    // ... at n up to this (HBEGP_SMALL_TILE_CTAS, HBEGP_SMALL_TILE_NP; gemm.cuh launch_gemm)
-    bool use_graph_update = true;  // HBEGP_GRAPH_UPDATE
-    bool alpha_side = true;       // alpha on the side stream beside the K^-1 product (HBEGP_ALPHA_SIDE)
-    bool small_tile_kinv = true;  // also for K^-1 = W^T W (HBEGP_SMALL_TILE_KINV)
-    int group_min = 0;  // n <= 2048: fewest matrices per stream group (HBEGP_GROUP_MIN; 0 = by size)
-    int node_v = 2;  // bottom node: 2 = k_node128_v2 (register-resident panels + DMMA products, FP64 inside), 1 = k_node128
     cudaEvent_t fork_ev = nullptr;
     long n = 0;
     int d = 0, np = 0;
@@ -234,7 +224,6 @@ struct Model {
     // prm_h[0] is the unclamped value the fit evaluated (fit.rs:96 does not clamp); they differ only when the optimum
     // sits outside the noise bounds by rounding.
     double noise_clamped = 0.0;
-    bool w_aligned128 = false;  // W meets the 128-wide-tile invariant (Engine::aligned128)
     // Retained-model policy (SURVEY F10 / H6: the minimizer keeps EVERY generation's model, minimize.rs:331, :407): only
     // the newest few models of a context keep their n x n factor W = L^-1 on the device.  An older one gives W and its
     // prediction scratch back to the pool (O(n d) stays: X^T / l, alpha, the parameters) and refactorises on its next
@@ -319,9 +308,6 @@ struct Engine : EngineBase {
     // generation (src/core/minimize.rs:331-407), so the padded size changes only every sixth generation.
     unsigned graph_epoch = 0;
     std::map<std::tuple<int, int, int, int, int>, CachedGraph> graphs;
-    bool use_graphs = true;
-    bool pad_batches = true;
-    bool streams_forced = false;
     T* h_prm = nullptr;  // pinned staging
     double* h_out = nullptr;
     int* h_status = nullptr;
@@ -341,11 +327,11 @@ struct Engine : EngineBase {
     // multiple of 4 (copies of the last theta, results ignored: 33 distinct graphs -> 9, first fit 0.90 -> 0.27 s).
     // The padding is not free any more now that small batches keep the GPU busy (B = 33 -> 36: +5 % per call), so a
     // size that keeps coming back — a caller's steady loop, the first rounds of a fit — gets its exact graph after
-    // four consecutive requests (probes/pad_ab.py, profiles/r02_pad_ab.log).
+    // four consecutive requests (profiles/r02_pad_ab.log).
     std::vector<int> exact_sizes;
     int pad_last_cnt = -1, pad_repeat = 0;
     int padded_batch(int cnt) {
-        if (!(use_graphs && pad_batches && np <= 2048 && cnt > 4)) return cnt;
+        if (!(np <= 2048 && cnt > 4)) return cnt;
         const int padded = std::min(cap, (cnt + 3) / 4 * 4);
         if (padded == cnt) return cnt;
         if (std::find(exact_sizes.begin(), exact_sizes.end(), cnt) != exact_sizes.end()) return cnt;
@@ -377,10 +363,6 @@ struct Engine : EngineBase {
     Model* new_empty_model(int nu2, const std::vector<double>& prm_h, double noise_clamped) override;
 
     int p() const { return d + 2; }
-    // The recursion puts its 128-multiple blocks first (chol_inv) and k_node128 zeroes the (0,1) block of every bottom
-    // node, so with the fused node enabled every 128-wide diagonal tile of W has exact zeros above its diagonal -- the
-    // invariant the 128-wide GEMM tiles (f64 HBEGP_TILE=128, f32 tcgen05) need for their triangular k ranges.
-    bool aligned128() const { return use_node128; }
     long mstride() const { return (long)np * np; }
     int ntiles_lower() const { int t = np / TILE; return t * (t + 1) / 2; }
     int nchunks() const { return (np + 255) / 256; }
@@ -401,7 +383,7 @@ struct Engine : EngineBase {
         if ((rc = dX.ensure((size_t)np * d * sizeof(T)))) return rc;  // sized by the padded row count: stable while np is
         if ((rc = dY.ensure((size_t)np * sizeof(T)))) return rc;
         if (!same_shape || oldx != dX.p || oldy != dY.p) {
-            if (same_padded && use_graph_update) {
+            if (same_padded) {
                 graph_epoch++;  // same topology: the cached graphs are patched on their next use (run_chunk)
             } else {
                 drop_graphs();
@@ -501,20 +483,17 @@ struct Engine : EngineBase {
             launches++;
             return HBEGP_OK;
         }
-        if (s == 2 * TILE && use_node128) {  // the bottom node of the tree in one launch
-            if (node_v == 2) {  // FP64 arithmetic inside for both precisions (node_mma.cuh)
-                CUDA_TRY(launch_prio(k_node128_v2<false, T>, dim3(1, 1, cnt), dim3(256), node128_v2_smem_bytes(), st, Ab, Wb, mstride(), np, r0,
-                                     (T*)ldp.p + (size_t)s0 * (np / TILE), np / TILE, (int*)d_status.p + s0, (long long*)nullptr));
-                launches++;
-                return HBEGP_OK;
-            }
-            CUDA_TRY(launch_prio(k_node128<T>, dim3(1, 1, cnt), dim3(256), node128_smem_bytes<T>(), st, Ab, Wb, mstride(), np, r0,
-                                 (T*)ldp.p + (size_t)s0 * (np / TILE), np / TILE, (int*)d_status.p + s0));
+        if (s == 2 * TILE) {  // the bottom node of the tree in one launch, FP64 arithmetic inside for both precisions
+            CUDA_TRY(launch_prio(k_node128_v2<false, T>, dim3(1, 1, cnt), dim3(256), node128_v2_smem_bytes(), st, Ab, Wb, mstride(), np, r0,
+                                 (T*)ldp.p + (size_t)s0 * (np / TILE), np / TILE, (int*)d_status.p + s0, (long long*)nullptr));
             launches++;
             return HBEGP_OK;
         }
+        // The large blocks are kept multiples of 128 and k_node128_v2 zeroes the (0,1) block of every bottom node, so every
+        // 128-wide diagonal tile of W has exact zeros above its diagonal: the invariant the 128-wide tcgen05 tiles (f32)
+        // need for their triangular k ranges.
         int q = s / TILE, q1 = (q + 1) / 2;
-        if (q >= 4 && (q1 & 1)) q1 += 1;  // keep the large blocks multiples of 128 for the 128x128 GEMM tile
+        if (q >= 4 && (q1 & 1)) q1 += 1;
         if (q1 >= q) q1 = q - 1;
         const int s1 = q1 * TILE, s2 = s - s1;
         int rc;
@@ -537,11 +516,11 @@ struct Engine : EngineBase {
         g.lda = g.ldb = g.ldc = np;
         g.sA = g.sB = g.sC = mstride();
         g.rowsumsq = nullptr;
-        g.small_ctas = np <= small_tile_np ? small_tile_ctas : 0;
+        g.small_ctas = np <= SMALL_TILE_NP ? SMALL_TILE_CTAS : 0;
         // 1. panel solve as a product with the inverse: L21 = A21 W11^T  -> W(2,1)
         g.A = A21; g.B = W11; g.C = W21; g.M = s2; g.N = s1; g.K = s1; g.kmode = K_LE_N; g.lower_only = 0;
         g.alpha = T(1); g.beta = T(0);
-        CUDA_TRY((launch_gemm_auto<T, true, true>(g, cnt, st, aligned128(), 0))); launches++;
+        CUDA_TRY((launch_gemm_auto<T, true, true>(g, cnt, st))); launches++;
         // 3. T = L21 W11 -> A(2,1); independent of step 2 and of the second half, so it may run on the side stream
         cudaStream_t st3 = st;
         if (sd.st) {
@@ -551,21 +530,26 @@ struct Engine : EngineBase {
         }
         g.A = W21; g.B = W11; g.C = A21; g.M = s2; g.N = s1; g.K = s1; g.kmode = K_GE_N; g.lower_only = 0;
         g.alpha = T(1); g.beta = T(0);
-        CUDA_TRY((launch_gemm_auto<T, true, false>(g, cnt, st3, aligned128(), 1))); launches++;
+        CUDA_TRY((launch_gemm_auto<T, true, false>(g, cnt, st3))); launches++;
         if (sd.st) CUDA_TRY(cudaEventRecord(sd.b, sd.st));
         // 2. trailing update: A22 -= L21 L21^T (lower tiles)
         g.A = W21; g.B = W21; g.C = A22; g.M = s2; g.N = s2; g.K = s1; g.kmode = K_FULL; g.lower_only = 1;
         g.alpha = T(-1); g.beta = T(1);
-        CUDA_TRY((launch_gemm_auto<T, true, true>(g, cnt, st, aligned128(), 2))); launches++;
+        CUDA_TRY((launch_gemm_auto<T, true, true>(g, cnt, st))); launches++;
         if ((rc = chol_inv(st, s0, cnt, r0 + s1, s2, sd))) return rc;
         // (a nested node may have re-recorded sd.b later on the side stream: waiting for that implies our product)
         if (sd.st) CUDA_TRY(cudaStreamWaitEvent(st, sd.b, 0));
         // 4. W21 = -W22 T
         g.A = W22; g.B = A21; g.C = W21; g.M = s2; g.N = s1; g.K = s2; g.kmode = K_LE_M; g.lower_only = 0;
         g.alpha = T(-1); g.beta = T(0);
-        CUDA_TRY((launch_gemm_auto<T, true, false>(g, cnt, st, aligned128(), 3))); launches++;
+        CUDA_TRY((launch_gemm_auto<T, true, false>(g, cnt, st))); launches++;
         return HBEGP_OK;
     }
+
+    // 32x32 GEMM tiles for grids of at most SMALL_TILE_CTAS 64x64 CTAs at n up to SMALL_TILE_NP (gemm.cuh launch_gemm),
+    // in the recursion and for K^-1 = W^T W
+    static constexpr long SMALL_TILE_CTAS = 296;
+    static constexpr int SMALL_TILE_NP = 1024;
 
     // K^-1 = W^T W on the lower tiles, written over the (dead) Cholesky factor in A
     int lauum(cudaStream_t st, T* Ab, T* Wb, int cnt) {
@@ -575,8 +559,8 @@ struct Engine : EngineBase {
         g.A = Wb; g.B = Wb; g.C = Ab; g.M = np; g.N = np; g.K = np; g.kmode = K_GE_M; g.lower_only = 1;
         g.alpha = T(1); g.beta = T(0);
         g.rowsumsq = nullptr;
-        g.small_ctas = (np <= small_tile_np && small_tile_kinv) ? small_tile_ctas : 0;
-        CUDA_TRY((launch_gemm_auto<T, false, false>(g, cnt, st, aligned128(), 4))); launches++;
+        g.small_ctas = np <= SMALL_TILE_NP ? SMALL_TILE_CTAS : 0;
+        CUDA_TRY((launch_gemm_auto<T, false, false>(g, cnt, st))); launches++;
         return HBEGP_OK;
     }
 
@@ -608,7 +592,7 @@ struct Engine : EngineBase {
         if (phase < 2) return HBEGP_OK;
         // alpha = W^T (W y)   (lml.rs:54 solves K alpha = y through the factorisation).  alpha and K^-1 = W^T W both
         // need W only: with a side stream the three latency-bound alpha kernels run beside the K^-1 product.
-        const bool split = alpha_side && sd.st && (want_grad || want_kinv);
+        const bool split = sd.st && (want_grad || want_kinv);
         cudaStream_t sa = st;
         if (split) {
             CUDA_TRY(cudaEventRecord(sd.a, st));
@@ -642,7 +626,8 @@ struct Engine : EngineBase {
 
     int pipeline(int nu2, cudaStream_t st, int s0, int cnt, bool want_grad, bool want_kinv, Side sd = Side()) {
         // large n with many matrices per group: the GEMMs fill the GPU on their own
-        if (!(use_side && (np <= 2048 || cnt <= side_max_cnt) && np > TILE)) sd = Side();
+        constexpr int SIDE_MAX_CNT = 4;  // at n > 2048 the side stream serves groups of at most this many matrices
+        if (!((np <= 2048 || cnt <= SIDE_MAX_CNT) && np > TILE)) sd = Side();
         if (nu2 == 5) return pipeline_nu<5>(st, s0, cnt, want_grad, want_kinv, sd);
         if (nu2 == 3) return pipeline_nu<3>(st, s0, cnt, want_grad, want_kinv, sd);
         return pipeline_nu<1>(st, s0, cnt, want_grad, want_kinv, sd);
@@ -650,17 +635,15 @@ struct Engine : EngineBase {
 
     int n_groups(int cnt) const {
         int g = (int)sub.size();
-        if (!streams_forced) {
-            // Re-measured in round 2 (profiles/r02_c3_streams.log, r02_streams_sweep.log; B = 33, ms per step with
-            // 1 / 2 / 4 / 8 groups): n = 512: 0.669 / 0.639 / 0.640 / 0.631; n = 1024: 2.47 / 2.32 / 2.26 / 2.20;
-            // n = 2048: 12.59 / 12.23 / 12.07 / 11.89 -- the latency-bound bottom nodes of one group (a few dozen CTAs on
-            // 148 SMs) overlap another group's GEMMs.  With the faster bottom node (node_mma.cuh) up to 16 groups of as few
-            // as 2 matrices (1 from n = 1024 up) pay off (profiles/r02_group_min.log: n = 1024 B = 33 1.786 -> 1.750 ms,
-            // n = 2048 B = 9 3.70 -> 3.39, n = 500 B = 3 unchanged).
-            const int gm = group_min > 0 ? group_min : (np >= 1024 ? 1 : 2);
-            if (np <= 2048) g = std::min(g, std::max(1, cnt / gm));
-            else g = std::min(g, 4);
-        }
+        // Re-measured in round 2 (profiles/r02_c3_streams.log, r02_streams_sweep.log; B = 33, ms per step with
+        // 1 / 2 / 4 / 8 groups): n = 512: 0.669 / 0.639 / 0.640 / 0.631; n = 1024: 2.47 / 2.32 / 2.26 / 2.20;
+        // n = 2048: 12.59 / 12.23 / 12.07 / 11.89 -- the latency-bound bottom nodes of one group (a few dozen CTAs on
+        // 148 SMs) overlap another group's GEMMs.  With the faster bottom node (node_mma.cuh) up to 16 groups of as few
+        // as 2 matrices (1 from n = 1024 up) pay off (profiles/r02_group_min.log: n = 1024 B = 33 1.786 -> 1.750 ms,
+        // n = 2048 B = 9 3.70 -> 3.39, n = 500 B = 3 unchanged).
+        const int gm = np >= 1024 ? 1 : 2;  // fewest matrices per stream group
+        if (np <= 2048) g = std::min(g, std::max(1, cnt / gm));
+        else g = std::min(g, 4);
         return std::max(1, std::min(g, cnt));
     }
 
@@ -703,7 +686,7 @@ struct Engine : EngineBase {
         // ~1000-node graph for every distinct batch size of a fit costs more than it saves (measured: 10.2 s
         // with graphs vs 9.5 s without for the north-star fit; 0.37 s vs 0.39 s at n = 1024).
         const bool legacy = (stream == nullptr || stream == cudaStreamLegacy);
-        if (!use_graphs || legacy || np > 2048) {
+        if (legacy || np > 2048) {
             int rc = issue_chunk(nu2, cnt, want_grad, want_kinv);
             if (rc) return rc;
             CUDA_TRY(cudaStreamSynchronize(stream));
@@ -770,7 +753,7 @@ struct Engine : EngineBase {
         if (B < 0 || (B > 0 && (!theta || !lml))) return fail(HBEGP_ERR_INVALID, "lml_grad_batch: bad arguments");
         if (B == 0) return HBEGP_OK;
         CUDA_TRY(cudaSetDevice(device));
-        if ((rc = ensure_capacity((use_graphs && pad_batches && np <= 2048 && B > 4) ? (B + 3) / 4 * 4 : B))) return rc;
+        if ((rc = ensure_capacity((np <= 2048 && B > 4) ? (B + 3) / 4 * 4 : B))) return rc;
         last_eval_cnt = (B <= cap) ? B : -1;
         for (int b0 = 0; b0 < B; b0 += cap) {
             int cnt = std::min(cap, B - b0);
@@ -1049,8 +1032,8 @@ struct ModelT : Model {
             // The variance kernel is chosen from np alone, never from the row count: a candidate's variance then has
             // the same bits however many rows are predicted with it (f32: 3xTF32 or FFMA sum in different orders).
             // rows is a multiple of 128, so the TF32 tiles are full in M even when rows < 256.
-            const bool tf = gemm_uses_tf32<T>(np, np, w_aligned128, 5);
-            const int bn = tf ? 128 : pick_gemm_tile<T>(128, np);
+            const bool tf = gemm_uses_tf32<T>(np, np);
+            const int bn = tf ? 128 : 64;
             const int ntile = (np + bn - 1) / bn;
             T* pm = nullptr;
             if (ns > 1) {
@@ -1365,7 +1348,6 @@ int Engine<T>::finish_model(int nu2, Model** out, double* lml, void* alpha_out, 
     m->c = (double)h_prm[1];
     m->prm_h.assign(h_prm, h_prm + p());
     m->noise_clamped = next_model_noise;
-    m->w_aligned128 = aligned128();
     auto bail = [&](int code) { delete m; return code; };
     if ((rc = m->W.ensure((size_t)np * np * sizeof(T)))) return bail(rc);
     if ((rc = m->alpha.ensure((size_t)np * sizeof(T)))) return bail(rc);
@@ -1417,7 +1399,6 @@ Model* Engine<T>::new_empty_model(int nu2, const std::vector<double>& prm_host, 
     m->c = prm_host[1];
     m->prm_h = prm_host;
     m->noise_clamped = noise_clamped;
-    m->w_aligned128 = aligned128();
     if (m->W.ensure((size_t)np * np * sizeof(T)) || m->alpha.ensure((size_t)np * sizeof(T)) || m->xsT.ensure((size_t)d * np * sizeof(T)) ||
         m->ls.ensure((size_t)d * sizeof(T)) || m->ldp.ensure((size_t)(np / TILE) * sizeof(T))) {
         delete m;
@@ -1493,7 +1474,7 @@ int Engine<T>::model_extend(Model* prior_, Model** out, double* lml, void* alpha
     // the append needs at least one complete 64-row leaf of the prior model and the old rows as a prefix
     // (a multiple of 128 rows of the prior are kept so that the appended blocks stay aligned with the 128-wide tiles)
     int r1 = (int)(std::min<long>(prior->n, n) / (2 * TILE)) * (2 * TILE);
-    if (!prior->w_aligned128 || prior->evicted) r1 = 0;  // (an evicted prior would have to be refactorised first: no gain)
+    if (prior->evicted) r1 = 0;  // (an evicted prior would have to be refactorised first: no gain)
     if (prior->n > n || !same_noise) r1 = 0;
     if (r1 > 0) {
         CUDA_TRY(cudaMemcpyAsync(prm.p, h_prm, (size_t)p() * sizeof(T), cudaMemcpyHostToDevice, stream));
@@ -1528,9 +1509,6 @@ static int configure_gemms() {
 #define HBEGP_CFG(BM, BN, WM, WN, AK, BK_)                                                                        \
     CUDA_TRY(cudaFuncSetAttribute(gemm_kernel<T, BM, BN, WM, WN, AK, BK_>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
                                   (int)GemmCfg<T, BM, BN, WM, WN, AK, BK_>::SMEM_BYTES))
-    HBEGP_CFG(128, 128, wm128<T>(), 32, true, true);
-    HBEGP_CFG(128, 128, wm128<T>(), 32, true, false);
-    HBEGP_CFG(128, 128, wm128<T>(), 32, false, false);
     HBEGP_CFG(64, 64, 32, 32, true, true);
     HBEGP_CFG(64, 64, 32, 32, true, false);
     HBEGP_CFG(64, 64, 32, 32, false, false);
@@ -1551,8 +1529,7 @@ static int configure_gemms() {
     }
     // kernels whose dynamic shared memory grows with the feature count d (two d x 64 operand tiles)
     const int big = (int)kMaxFeatureSmem;
-    CUDA_TRY(cudaFuncSetAttribute(k_leaf<T, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)leaf_smem_bytes<T>()));
-    CUDA_TRY(cudaFuncSetAttribute(k_node128<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)node128_smem_bytes<T>()));
+    CUDA_TRY(cudaFuncSetAttribute(k_leaf<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)leaf_smem_bytes<T>()));
     CUDA_TRY(cudaFuncSetAttribute(k_node128_v2<false, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)node128_v2_smem_bytes()));
     CUDA_TRY(cudaFuncSetAttribute(k_assemble<T, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
     CUDA_TRY(cudaFuncSetAttribute(k_assemble<T, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
@@ -1854,33 +1831,16 @@ int hbegp_ctx_create(int device, int dtype, void* stream, hbegp_ctx** out) {
         int rc = (dtype == HBEGP_F64) ? configure_gemms<double>() : configure_gemms<float>();
         if (rc) { delete e; return rc; }
     }
-    int nsub = 16;
-    if (const char* s = getenv("HBEGP_NSUB")) nsub = std::max(1, std::min(16, atoi(s)));
-    bool forced = false;
-    if (const char* s = getenv("HBEGP_STREAMS")) { nsub = std::max(1, std::min(16, atoi(s))); forced = true; }
-    {
-        const char* s64 = getenv("HBEGP_TILE");
-        const char* s32 = getenv("HBEGP_TILE32");
-        gemm_tile_pref() = (s64 && atoi(s64) == 128) ? 128 : 64;
-        gemm_tile_pref_f32() = (s32 && atoi(s32) == 128) ? 128 : 64;
-    }
     {
         const char* t = getenv("HBEGP_TF32");
-        const char* tm = getenv("HBEGP_TF32_MIN");
         tf32::enabled() = !(t && atoi(t) == 0);
-        tf32::min_extent() = tm ? std::max(64, atoi(tm)) : 256;
-        if (const char* cm = getenv("HBEGP_TF32_MASK")) tf32::class_mask() = atoi(cm);
-        else tf32::class_mask() = 0x3f;
         if (dtype == HBEGP_F32 && tf32::enabled() && !tf32::encode_fn()) {
             delete e;
             return fail(HBEGP_ERR_CUDA, "ctx_create: cuTensorMapEncodeTiled is not available from this driver (set HBEGP_TF32=0)");
         }
     }
-    bool graphs_on = true;
-    if (const char* s = getenv("HBEGP_GRAPHS")) graphs_on = atoi(s) != 0;
-    if (dtype == HBEGP_F64) { static_cast<Engine<double>*>(e)->streams_forced = forced; static_cast<Engine<double>*>(e)->use_graphs = graphs_on; }
-    else { static_cast<Engine<float>*>(e)->streams_forced = forced; static_cast<Engine<float>*>(e)->use_graphs = graphs_on; }
-    for (int i = 0; i < nsub; i++) {
+    constexpr int STREAM_GROUPS = 16;  // the most a batch is split into (Engine::n_groups)
+    for (int i = 0; i < STREAM_GROUPS; i++) {
         cudaStream_t s;
         cudaEvent_t ev;
         if (cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking) != cudaSuccess ||
@@ -1908,21 +1868,6 @@ int hbegp_ctx_create(int device, int dtype, void* stream, hbegp_ctx** out) {
         cudaEventCreateWithFlags(&e->main_b, cudaEventDisableTiming) != cudaSuccess) {
         delete e;
         return fail(HBEGP_ERR_CUDA, "ctx_create: side stream");
-    }
-    if (const char* s = getenv("HBEGP_SIDE")) e->use_side = atoi(s) != 0;
-    if (const char* s = getenv("HBEGP_NODE128")) e->use_node128 = atoi(s) != 0;
-    if (const char* s = getenv("HBEGP_NODE_V")) e->node_v = atoi(s);
-    if (const char* s = getenv("HBEGP_SMALL_TILE_CTAS")) e->small_tile_ctas = atol(s);
-    if (const char* s = getenv("HBEGP_GRAPH_UPDATE")) e->use_graph_update = atoi(s) != 0;
-    if (const char* s = getenv("HBEGP_ALPHA_SIDE")) e->alpha_side = atoi(s) != 0;
-    if (const char* s = getenv("HBEGP_SMALL_TILE_KINV")) e->small_tile_kinv = atoi(s) != 0;
-    if (const char* s = getenv("HBEGP_SMALL_TILE_NP")) e->small_tile_np = atoi(s);
-    if (const char* s = getenv("HBEGP_GROUP_MIN")) e->group_min = std::max(0, atoi(s));
-    if (const char* s = getenv("HBEGP_SIDE_CNT")) e->side_max_cnt = atoi(s);
-    if (const char* s = getenv("HBEGP_PAD")) {
-        const bool pad = atoi(s) != 0;
-        if (dtype == HBEGP_F64) static_cast<Engine<double>*>(e)->pad_batches = pad;
-        else static_cast<Engine<float>*>(e)->pad_batches = pad;
     }
     *out = new hbegp_ctx{e};
     return HBEGP_OK;

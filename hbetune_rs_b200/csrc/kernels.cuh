@@ -199,16 +199,16 @@ __device__ __forceinline__ double pivot_rcp<double>(double d) {
 //    update per panel.  No square root on the pivot chain: 1 / L_jj = rsqrt(u_jj) for all j at the end.
 //  * inverse: the four 16x16 diagonal blocks are inverted side by side (15 steps instead of 63), the off-diagonal
 //    blocks follow by block forward substitution W_PQ = -W_PP sum_R L_PR W_RQ (three levels of small products).
+// A variant with 8-wide register-resident panels (one barrier pair per panel instead of one barrier per pivot) measured
+// no faster in either precision: the gain needs the DMMA products and the transposed layout of node_mma.cuh.
 template <typename T>
 __host__ __device__ constexpr size_t leaf_tile_bytes() { return sizeof(T) * TILE * (TILE + 1); }
 template <typename T>
 constexpr size_t leaf_smem_bytes() { return 2 * leaf_tile_bytes<T>() + 2 * TILE * sizeof(T); }
-template <typename T>
-constexpr size_t node128_smem_bytes() { return 5 * leaf_tile_bytes<T>() + 2 * TILE * sizeof(T); }
 
 // The leaf on shared memory.  In: as = the 64x64 block (lower part, zeros above).  Out: ws = L^-1 (zeros above the
 // diagonal), dinv[i] = 1 / L_ii; *fail = 1 when a pivot is not positive.  Ends with a barrier.  `as` is scratch after.
-template <typename T, int DBG>
+template <typename T>
 __device__ __forceinline__ void leaf_core(T (*as)[TILE + 1], T (*ws)[TILE + 1], T* rdv, T* dinv, int* fail, int tid) {
     const int tx = tid & 15, ty = tid >> 4;
 #pragma unroll
@@ -219,57 +219,55 @@ __device__ __forceinline__ void leaf_core(T (*as)[TILE + 1], T (*ws)[TILE + 1], 
             ws[i][k] = (i == k) ? T(1) : T(0);
         }
     // ---- blocked Cholesky (nb = 16) on unscaled columns
-    if (!(DBG & 1)) {
-        const int pi = tid >> 2, pq = tid & 3;  // panel phase: row pi, panel columns pq, pq + 4, pq + 8, pq + 12
-        for (int P = 0; P < 4; P++) {
-            const int c0 = 16 * P;
-            __syncthreads();
-            T pv[4];
+    const int pi = tid >> 2, pq = tid & 3;  // panel phase: row pi, panel columns pq, pq + 4, pq + 8, pq + 12
+    for (int P = 0; P < 4; P++) {
+        const int c0 = 16 * P;
+        __syncthreads();
+        T pv[4];
 #pragma unroll
-            for (int t = 0; t < 4; t++) pv[t] = as[pi][c0 + pq + 4 * t];
+        for (int t = 0; t < 4; t++) pv[t] = as[pi][c0 + pq + 4 * t];
 #pragma unroll
-            for (int jj = 0; jj < 16; jj++) {
-                const int j = c0 + jj;
-                if (jj > 0) {
-                    // column j is final after step j - 1: its owners publish it for this step
-                    if (pq == (jj & 3)) as[pi][j] = pv[jj >> 2];
-                    __syncthreads();
-                }
-                T dj = as[j][j];
-                const T uij = as[pi][j];
-                T ukj[4];
-#pragma unroll
-                for (int t = jj >> 2; t < 4; t++) ukj[t] = as[c0 + pq + 4 * t][j];
-                if (!(dj > T(0)) || !(dj <= T(1e300))) {
-                    if (tid == 0) *fail = 1;
-                    dj = T(1);
-                }
-                const T rd = pivot_rcp<T>(dj);
-                if (tid == 0) rdv[j] = rd;
-                const T li = uij * rd;
-#pragma unroll
-                for (int t = jj >> 2; t < 4; t++) {
-                    const int k = pq + 4 * t;  // panel-relative column
-                    if (k > jj && c0 + k <= pi) pv[t] = fma(-li, ukj[t], pv[t]);
-                }
+        for (int jj = 0; jj < 16; jj++) {
+            const int j = c0 + jj;
+            if (jj > 0) {
+                // column j is final after step j - 1: its owners publish it for this step
+                if (pq == (jj & 3)) as[pi][j] = pv[jj >> 2];
+                __syncthreads();
             }
-            __syncthreads();
-            // rank-16 update of everything right of the panel: u_ik -= sum_{j in panel} u_ij u_kj / u_jj
+            T dj = as[j][j];
+            const T uij = as[pi][j];
+            T ukj[4];
 #pragma unroll
-            for (int q = 1; q < 4; q++) {
-                if (q > P) {
-                    T lk[16];
+            for (int t = jj >> 2; t < 4; t++) ukj[t] = as[c0 + pq + 4 * t][j];
+            if (!(dj > T(0)) || !(dj <= T(1e300))) {
+                if (tid == 0) *fail = 1;
+                dj = T(1);
+            }
+            const T rd = pivot_rcp<T>(dj);
+            if (tid == 0) rdv[j] = rd;
+            const T li = uij * rd;
 #pragma unroll
-                    for (int jj = 0; jj < 16; jj++) lk[jj] = as[tx + 16 * q][c0 + jj] * rdv[c0 + jj];
+            for (int t = jj >> 2; t < 4; t++) {
+                const int k = pq + 4 * t;  // panel-relative column
+                if (k > jj && c0 + k <= pi) pv[t] = fma(-li, ukj[t], pv[t]);
+            }
+        }
+        __syncthreads();
+        // rank-16 update of everything right of the panel: u_ik -= sum_{j in panel} u_ij u_kj / u_jj
 #pragma unroll
-                    for (int a = 1; a < 4; a++) {
-                        if (a >= q) {
-                            const int i = ty + 16 * a, k = tx + 16 * q;
-                            T acc = T(0);
+        for (int q = 1; q < 4; q++) {
+            if (q > P) {
+                T lk[16];
 #pragma unroll
-                            for (int jj = 0; jj < 16; jj++) acc = fma(as[i][c0 + jj], lk[jj], acc);
-                            if (k <= i) as[i][k] -= acc;
-                        }
+                for (int jj = 0; jj < 16; jj++) lk[jj] = as[tx + 16 * q][c0 + jj] * rdv[c0 + jj];
+#pragma unroll
+                for (int a = 1; a < 4; a++) {
+                    if (a >= q) {
+                        const int i = ty + 16 * a, k = tx + 16 * q;
+                        T acc = T(0);
+#pragma unroll
+                        for (int jj = 0; jj < 16; jj++) acc = fma(as[i][c0 + jj], lk[jj], acc);
+                        if (k <= i) as[i][k] -= acc;
                     }
                 }
             }
@@ -280,179 +278,35 @@ __device__ __forceinline__ void leaf_core(T (*as)[TILE + 1], T (*ws)[TILE + 1], 
         T dj = as[tid][tid];
         if (!(dj > T(0)) || !(dj <= T(1e300))) dj = T(1);
         dinv[tid] = T(1) / dev_sqrt<T>(dj);
-        if (DBG & 1) rdv[tid] = T(1) / dj;
     }
     // ---- inverse of the four 16x16 diagonal blocks, side by side (rows unscaled: W_true = W_u * dinv_row)
-    if (!(DBG & 2)) {
-        const int P = tid >> 6, r = (tid & 63) >> 2, cq = tid & 3, c0 = 16 * P;
-        for (int kk = 0; kk < 15; kk++) {
-            __syncthreads();
-            if (r > kk) {
-                const T lik = as[c0 + r][c0 + kk] * rdv[c0 + kk];  // L_ik / L_kk = u_ik / u_kk
-                for (int c = cq; c <= kk; c += 4) ws[c0 + r][c0 + c] = fma(-lik, ws[c0 + kk][c0 + c], ws[c0 + r][c0 + c]);
-            }
-        }
+    const int P = tid >> 6, r = (tid & 63) >> 2, cq = tid & 3, c0 = 16 * P;
+    for (int kk = 0; kk < 15; kk++) {
         __syncthreads();
-        {
-            const int i = c0 + r;
-            for (int c = cq; c <= r; c += 4) ws[i][c0 + c] *= dinv[i];
-        }
-        // ---- off-diagonal blocks by block forward substitution; S_PQ goes to the free upper part of `as`
-        const int sr = tid >> 4, sc = tid & 15;
-        for (int PP = 1; PP < 4; PP++) {
-            __syncthreads();
-            for (int Q = 0; Q < PP; Q++) {
-                T acc = T(0);
-                for (int k = 16 * Q; k < 16 * PP; k++) acc = fma(as[16 * PP + sr][k] * dinv[k], ws[k][16 * Q + sc], acc);
-                as[16 * Q + sr][16 * PP + sc] = acc;  // S_PQ (strictly upper position: Q < PP)
-            }
-            __syncthreads();
-            for (int Q = 0; Q < PP; Q++) {
-                T acc = T(0);
-                for (int k = 0; k <= sr; k++) acc = fma(ws[16 * PP + sr][16 * PP + k], as[16 * Q + k][16 * PP + sc], acc);
-                ws[16 * PP + sr][16 * Q + sc] = -acc;
-            }
+        if (r > kk) {
+            const T lik = as[c0 + r][c0 + kk] * rdv[c0 + kk];  // L_ik / L_kk = u_ik / u_kk
+            for (int c = cq; c <= kk; c += 4) ws[c0 + r][c0 + c] = fma(-lik, ws[c0 + kk][c0 + c], ws[c0 + r][c0 + c]);
         }
     }
     __syncthreads();
-}
-
-// Second-generation leaf (round 2): same contract as leaf_core, far fewer barriers.
-//
-// leaf_core pays one CTA barrier + a shared-memory round trip per pivot (64 of them, ~250 ns each) and another 15 for
-// the diagonal-block inverses.  Here the panel is 8 wide and its pivot chain runs entirely in registers: every row
-// thread holds the 8x8 diagonal block (36 values, broadcast loads) and factors it redundantly — all threads compute
-// the same bits, nobody waits for anybody — while carrying its own row of the panel through the same eliminations.
-// One barrier pair per panel (8 panels) instead of one barrier per pivot.  The inverse is recursive doubling:
-// the eight 8x8 diagonal blocks are inverted column-per-thread in registers, then 16-, 32- and 64-wide blocks follow
-// from W21 = -W22 (L21 W11), two small products per level.
-template <typename T, int DBG>
-__device__ __forceinline__ void leaf_core_nb8(T (*as)[TILE + 1], T (*ws)[TILE + 1], T* rdv, T* dinv, int* fail, int tid) {
-    constexpr int NB = 8;
-    const int tx = tid & 15, ty = tid >> 4;
-#pragma unroll
-    for (int a = 0; a < 4; a++)
-#pragma unroll
-        for (int q = 0; q < 4; q++) ws[ty + 16 * a][tx + 16 * q] = T(0);
-    // ---- Cholesky on unscaled columns u_ij = L_ij L_jj, panels of 8
-    if (!(DBG & 1)) {
-        for (int P = 0; P < TILE / NB; P++) {
-            const int c0 = NB * P;
-            __syncthreads();
-            if (tid < TILE) {  // warps 0 and 1
-                const int i = tid;
-                T U[NB][NB], x[NB], rd[NB];
-#pragma unroll
-                for (int r = 0; r < NB; r++)
-#pragma unroll
-                    for (int k = 0; k <= r; k++) U[r][k] = as[c0 + r][c0 + k];
-#pragma unroll
-                for (int k = 0; k < NB; k++) x[k] = as[i][c0 + k];
-                // the diagonal rows are overwritten below by their owners: both warps must hold their copies first
-                asm volatile("bar.sync 1, 64;" ::: "memory");
-                if (i >= c0) {
-                bool bad = false;
-#pragma unroll
-                for (int j = 0; j < NB; j++) {
-                    T dj = U[j][j];
-                    if (!(dj > T(0)) || !(dj <= T(1e300))) {
-                        bad = true;
-                        dj = T(1);
-                    }
-                    rd[j] = pivot_rcp<T>(dj);
-                    const T lx = x[j] * rd[j];
-#pragma unroll
-                    for (int k = j + 1; k < NB; k++) x[k] = fma(-lx, U[k][j], x[k]);
-#pragma unroll
-                    for (int r = j + 1; r < NB; r++) {
-                        const T l = U[r][j] * rd[j];
-#pragma unroll
-                        for (int k = j + 1; k <= r; k++) U[r][k] = fma(-l, U[k][j], U[r][k]);
-                    }
-                }
-#pragma unroll
-                for (int k = 0; k < NB; k++)
-                    if (c0 + k <= i) as[i][c0 + k] = x[k];
-                if (i == c0) {
-#pragma unroll
-                    for (int j = 0; j < NB; j++) {
-                        rdv[c0 + j] = rd[j];
-                        dinv[c0 + j] = dev_sqrt<T>(rd[j]);  // 1 / L_jj = sqrt(1 / u_jj)
-                    }
-                    if (bad) *fail = 1;
-                }
-                }
-            }
-            __syncthreads();
-            // rank-8 update of everything right of the panel: u_ik -= sum_{j in panel} u_ij u_kj / u_jj
-            if (P + 1 < TILE / NB) {
-#pragma unroll
-                for (int q = 0; q < 4; q++) {
-                    const int k = tx + 16 * q;
-                    if (k >= c0 + NB) {
-                        T lk[NB];
-#pragma unroll
-                        for (int jj = 0; jj < NB; jj++) lk[jj] = as[k][c0 + jj] * rdv[c0 + jj];
-#pragma unroll
-                        for (int a = 0; a < 4; a++) {
-                            const int i = ty + 16 * a;
-                            if (i >= k) {
-                                T acc = T(0);
-#pragma unroll
-                                for (int jj = 0; jj < NB; jj++) acc = fma(as[i][c0 + jj], lk[jj], acc);
-                                as[i][k] -= acc;
-                            }
-                        }
-                    }
-                }
-            }
-        }
-    } else {
-        __syncthreads();
-        if (tid < TILE) {
-            T dj = as[tid][tid];
-            if (!(dj > T(0)) || !(dj <= T(1e300))) dj = T(1);
-            rdv[tid] = T(1) / dj;
-            dinv[tid] = T(1) / dev_sqrt<T>(dj);
-        }
-        __syncthreads();
+    {
+        const int i = c0 + r;
+        for (int c = cq; c <= r; c += 4) ws[i][c0 + c] *= dinv[i];
     }
-    // here: as (lower) = u, rdv = 1 / u_jj, dinv = 1 / L_jj, all visible (the loop ends on a barrier)
-    if (!(DBG & 2)) {
-        // ---- level 0: the eight 8x8 diagonal blocks, one column of the inverse per thread, in registers:
-        // x_i = (delta_ic - sum_{k < i} u_ik z_k) dinv_i with z_k = dinv_k x_k  (L_ik = u_ik dinv_k)
-        if (tid < TILE) {
-            const int c0 = tid & ~(NB - 1), c = tid & (NB - 1);
-            T z[NB];
-#pragma unroll
-            for (int i = 0; i < NB; i++) {
-                T s = (i == c) ? T(1) : T(0);
-#pragma unroll
-                for (int k = 0; k < i; k++) s = fma(-as[c0 + i][c0 + k], z[k], s);
-                const T di = dinv[c0 + i];
-                const T xi = s * di;
-                z[i] = xi * di;
-                if (i >= c) ws[c0 + i][c0 + c] = xi;
-            }
+    // ---- off-diagonal blocks by block forward substitution; S_PQ goes to the free upper part of `as`
+    const int sr = tid >> 4, sc = tid & 15;
+    for (int PP = 1; PP < 4; PP++) {
+        __syncthreads();
+        for (int Q = 0; Q < PP; Q++) {
+            T acc = T(0);
+            for (int k = 16 * Q; k < 16 * PP; k++) acc = fma(as[16 * PP + sr][k] * dinv[k], ws[k][16 * Q + sc], acc);
+            as[16 * Q + sr][16 * PP + sc] = acc;  // S_PQ (strictly upper position: Q < PP)
         }
-        // ---- levels 1..3: half-width h = 8, 16, 32.  S = L21 W11 goes to the free upper-right block of `as`.
-#pragma unroll
-        for (int h = NB; h < TILE; h *= 2) {
-            const int cells = (TILE / (2 * h)) * h * h;  // 32 h: 256, 512, 1024
-            __syncthreads();
-            for (int e = tid; e < cells; e += 256) {
-                const int pr = e / (h * h), rc = e % (h * h), r = rc / h, c = rc % h, o = 2 * h * pr;
-                T acc = T(0);
-                for (int k = c; k < h; k++) acc = fma(as[o + h + r][o + k] * dinv[o + k], ws[o + k][o + c], acc);
-                as[o + r][o + h + c] = acc;
-            }
-            __syncthreads();
-            for (int e = tid; e < cells; e += 256) {
-                const int pr = e / (h * h), rc = e % (h * h), r = rc / h, c = rc % h, o = 2 * h * pr;
-                T acc = T(0);
-                for (int k = 0; k <= r; k++) acc = fma(ws[o + h + r][o + h + k], as[o + k][o + h + c], acc);
-                ws[o + h + r][o + c] = -acc;
-            }
+        __syncthreads();
+        for (int Q = 0; Q < PP; Q++) {
+            T acc = T(0);
+            for (int k = 0; k <= sr; k++) acc = fma(ws[16 * PP + sr][16 * PP + k], as[16 * Q + k][16 * PP + sc], acc);
+            ws[16 * PP + sr][16 * Q + sc] = -acc;
         }
     }
     __syncthreads();
@@ -470,19 +324,7 @@ __device__ __forceinline__ void leaf_logdet(const T* dinv, int tid, T* out) {
     }
 }
 
-// Leaf algorithm of k_leaf / k_node128: 0 = leaf_core, 1 = leaf_core_nb8 (register-resident 8-wide panels with FMA-pipe
-// updates: measured no faster than leaf_core in either precision, probes/leaf2_bench.cu — the gain needs the DMMA
-// products and the transposed layout of node_mma.cuh, which is what the f64 path runs)
-#ifndef HBEGP_LEAF_V
-#define HBEGP_LEAF_V 0
-#endif
-template <typename T, int DBG, int LV>
-__device__ __forceinline__ void leaf_core_sel(T (*as)[TILE + 1], T (*ws)[TILE + 1], T* rdv, T* dinv, int* fail, int tid) {
-    if constexpr (LV == 1) leaf_core_nb8<T, DBG>(as, ws, rdv, dinv, fail, tid);
-    else leaf_core<T, DBG>(as, ws, rdv, dinv, fail, tid);
-}
-
-template <typename T, int DBG = 0, int LV = HBEGP_LEAF_V>  // DBG: probe-only switch (1: skip the Cholesky loops, 2: skip the inverse)
+template <typename T>
 __global__ void __launch_bounds__(256) k_leaf(T* __restrict__ A, T* __restrict__ W, long mstride, int np, int r0,
                                               T* __restrict__ ldp, int ldp_stride, int* __restrict__ status) {
     extern __shared__ __align__(16) unsigned char leaf_smem_raw[];
@@ -503,7 +345,7 @@ __global__ void __launch_bounds__(256) k_leaf(T* __restrict__ A, T* __restrict__
             const int i = ty + 16 * a, k = tx + 16 * q;
             as[i][k] = (k <= i) ? Ab[(long)i * np + k] : T(0);
         }
-    leaf_core_sel<T, DBG, LV>(as, ws, rdv, dinv, &fail, tid);
+    leaf_core<T>(as, ws, rdv, dinv, &fail, tid);
 #pragma unroll
     for (int a = 0; a < 4; a++)
 #pragma unroll
@@ -512,123 +354,6 @@ __global__ void __launch_bounds__(256) k_leaf(T* __restrict__ A, T* __restrict__
             Wb[(long)i * np + k] = (k <= i) ? ws[i][k] : T(0);
         }
     leaf_logdet<T>(dinv, tid, ldp + (long)b * ldp_stride + r0 / TILE);
-    if (tid == 0 && fail) status[b] = 1;
-}
-
-// acc[a][q] += sum_k Am[ty + 16a][k] * (BT ? Bm[tx + 16q][k] : Bm[k][tx + 16q]): a 64x64x64 product of shared-memory
-// tiles on the FP64/FP32 FMA pipe (on sm_100a the DFMA rate equals the DMMA rate; ~2 us per product)
-template <typename T, bool BT>
-__device__ __forceinline__ void mm64(const T (*Am)[TILE + 1], const T (*Bm)[TILE + 1], T acc[4][4], int tx, int ty) {
-#pragma unroll 4
-    for (int k = 0; k < TILE; k++) {
-        T av[4], bv[4];
-#pragma unroll
-        for (int a = 0; a < 4; a++) av[a] = Am[ty + 16 * a][k];
-#pragma unroll
-        for (int q = 0; q < 4; q++) bv[q] = BT ? Bm[tx + 16 * q][k] : Bm[k][tx + 16 * q];
-#pragma unroll
-        for (int a = 0; a < 4; a++)
-#pragma unroll
-            for (int q = 0; q < 4; q++) acc[a][q] = fma(av[a], bv[q], acc[a][q]);
-    }
-}
-
-// A whole 128-wide node of the recursion in one CTA (two leaves and the four 64^3 products between them), so that
-// the bottom level of the tree costs one launch instead of six dependent ones:
-//   W11 = leaf(A11); L21 = A21 W11^T; T = L21 W11; A22 -= L21 L21^T; W22 = leaf(A22); W21 = -W22 T.
-template <typename T, int LV = HBEGP_LEAF_V>
-__global__ void __launch_bounds__(256) k_node128(T* __restrict__ A, T* __restrict__ W, long mstride, int np, int r0,
-                                                 T* __restrict__ ldp, int ldp_stride, int* __restrict__ status) {
-    extern __shared__ __align__(16) unsigned char leaf_smem_raw[];
-    typedef T Row[TILE + 1];
-    Row* as = reinterpret_cast<Row*>(leaf_smem_raw);
-    Row* w1 = reinterpret_cast<Row*>(leaf_smem_raw + 1 * leaf_tile_bytes<T>());
-    Row* w2 = reinterpret_cast<Row*>(leaf_smem_raw + 2 * leaf_tile_bytes<T>());
-    Row* pm = reinterpret_cast<Row*>(leaf_smem_raw + 3 * leaf_tile_bytes<T>());  // A21, later T
-    Row* qm = reinterpret_cast<Row*>(leaf_smem_raw + 4 * leaf_tile_bytes<T>());  // L21
-    T* rdv = reinterpret_cast<T*>(leaf_smem_raw + 5 * leaf_tile_bytes<T>());
-    T* dinv = rdv + TILE;
-    __shared__ int fail;
-    const int b = blockIdx.z, tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
-    T* Ab = A + (long)b * mstride + (long)r0 * np + r0;
-    T* Wb = W + (long)b * mstride + (long)r0 * np + r0;
-    T* ld = ldp + (long)b * ldp_stride + r0 / TILE;
-    if (tid == 0) fail = 0;
-#pragma unroll
-    for (int a = 0; a < 4; a++)
-#pragma unroll
-        for (int q = 0; q < 4; q++) {
-            const int i = ty + 16 * a, k = tx + 16 * q;
-            as[i][k] = (k <= i) ? Ab[(long)i * np + k] : T(0);
-            pm[i][k] = Ab[(long)(i + TILE) * np + k];  // A21
-        }
-    leaf_core_sel<T, 0, LV>(as, w1, rdv, dinv, &fail, tid);
-    leaf_logdet<T>(dinv, tid, ld);
-    T acc[4][4];
-    // L21 = A21 W11^T
-#pragma unroll
-    for (int a = 0; a < 4; a++)
-#pragma unroll
-        for (int q = 0; q < 4; q++) acc[a][q] = T(0);
-    mm64<T, true>(pm, w1, acc, tx, ty);
-#pragma unroll
-    for (int a = 0; a < 4; a++)
-#pragma unroll
-        for (int q = 0; q < 4; q++) qm[ty + 16 * a][tx + 16 * q] = acc[a][q];
-    // A22 (lower) into `as` while L21 settles
-#pragma unroll
-    for (int a = 0; a < 4; a++)
-#pragma unroll
-        for (int q = 0; q < 4; q++) {
-            const int i = ty + 16 * a, k = tx + 16 * q;
-            acc[a][q] = (k <= i) ? Ab[(long)(i + TILE) * np + TILE + k] : T(0);
-        }
-    __syncthreads();
-    // A22 -= L21 L21^T  (negated accumulation: acc holds A22, subtract the product)
-    {
-        T prod[4][4];
-#pragma unroll
-        for (int a = 0; a < 4; a++)
-#pragma unroll
-            for (int q = 0; q < 4; q++) prod[a][q] = T(0);
-        mm64<T, true>(qm, qm, prod, tx, ty);
-#pragma unroll
-        for (int a = 0; a < 4; a++)
-#pragma unroll
-            for (int q = 0; q < 4; q++) {
-                const int i = ty + 16 * a, k = tx + 16 * q;
-                as[i][k] = (k <= i) ? acc[a][q] - prod[a][q] : T(0);
-            }
-    }
-    // T = L21 W11 -> pm (A21 is dead: every thread finished reading it before the barrier above)
-#pragma unroll
-    for (int a = 0; a < 4; a++)
-#pragma unroll
-        for (int q = 0; q < 4; q++) acc[a][q] = T(0);
-    mm64<T, false>(qm, w1, acc, tx, ty);
-#pragma unroll
-    for (int a = 0; a < 4; a++)
-#pragma unroll
-        for (int q = 0; q < 4; q++) pm[ty + 16 * a][tx + 16 * q] = acc[a][q];
-    __syncthreads();
-    leaf_core_sel<T, 0, LV>(as, w2, rdv, dinv, &fail, tid);
-    leaf_logdet<T>(dinv, tid, ld + 1);
-    // W21 = -W22 T
-#pragma unroll
-    for (int a = 0; a < 4; a++)
-#pragma unroll
-        for (int q = 0; q < 4; q++) acc[a][q] = T(0);
-    mm64<T, false>(w2, pm, acc, tx, ty);
-#pragma unroll
-    for (int a = 0; a < 4; a++)
-#pragma unroll
-        for (int q = 0; q < 4; q++) {
-            const int i = ty + 16 * a, k = tx + 16 * q;
-            Wb[(long)i * np + k] = (k <= i) ? w1[i][k] : T(0);
-            Wb[(long)i * np + TILE + k] = T(0);  // (0,1) block: read by the 128-wide GEMM tiles' triangular k ranges
-            Wb[(long)(i + TILE) * np + k] = -acc[a][q];
-            Wb[(long)(i + TILE) * np + TILE + k] = (k <= i) ? w2[i][k] : T(0);
-        }
     if (tid == 0 && fail) status[b] = 1;
 }
 

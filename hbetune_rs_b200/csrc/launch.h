@@ -11,7 +11,6 @@
 #pragma once
 #include <cuda_runtime.h>
 
-#include <cstdlib>
 #include <utility>
 
 namespace hbegp {
@@ -27,13 +26,11 @@ struct LaunchPriority {
     // Priority for a grid of `ctas` CTAs.
     int for_grid(long ctas) const {
         if (small_ctas <= 0 || ctas > small_ctas) return least;
-        if (!graded) return greatest;
         // shortest first: every halving of the grid below the threshold is one level up (numerically down)
         int pr = least - 1;
         for (long c = small_ctas / 2; ctas <= c && pr > greatest; c /= 2) pr--;
         return pr < greatest ? greatest : pr;
     }
-    bool graded = true;
 
 private:
     static LaunchPriority make() {
@@ -44,9 +41,7 @@ private:
         }
         // One resident wave of the 64 x 64 GEMM tile is 3 CTAs x 148 SMs; anything that fits in it is latency bound.
         p.small_ctas = 444;
-        if (const char* s = getenv("HBEGP_PRIO_CTAS")) p.small_ctas = atol(s);
-        if (const char* s = getenv("HBEGP_PRIO_GRADED")) p.graded = atoi(s) != 0;
-        if (p.least == p.greatest) p.small_ctas = 0;
+        if (p.least == p.greatest) p.small_ctas = 0;  // no priority range on this device: feature off
         return p;
     }
 };

@@ -1,9 +1,10 @@
 // The 128-wide bottom node of the factor + inverse recursion, second generation (round 2).  FP64 arithmetic; the matrices
 // in global memory are double or (--use-32) float.
 //
-// k_node128 (kernels.cuh) spends its 59 us on (i) two 64-pivot chains with a CTA barrier and a shared-memory round
-// trip per pivot, (ii) 15 more barrier steps for the diagonal-block inverses and (iii) four 64^3 products whose operand
-// fetches saturate the shared-memory pipe (one 8-byte LDS per FMA and thread).  This kernel keeps the same contract
+// The first-generation node (two leaf_core leaves of kernels.cuh and four 64^3 FMA-pipe products in one CTA) spent its
+// 59 us on (i) two 64-pivot chains with a CTA barrier and a shared-memory round trip per pivot, (ii) 15 more barrier
+// steps for the diagonal-block inverses and (iii) four 64^3 products whose operand fetches saturate the shared-memory
+// pipe (one 8-byte LDS per FMA and thread).  This kernel keeps the same contract
 // (W11, W21, W22 = the inverse of the Cholesky factor of the 128-wide diagonal block, sum ln L_ii per 64-wide half,
 // status = 1 on a non-positive pivot) and removes all three:
 //  * Cholesky in panels of 8 whose pivot chain lives in registers: every row thread holds the panel's 8x8 diagonal
@@ -341,7 +342,7 @@ __device__ __forceinline__ void prod_w_b(const RowT* Wl, const RowT* Bm, double 
 //   W11 = leaf(A11); L21 = A21 W11^T; A22 -= L21 L21^T; T = L21 W11; W22 = leaf(A22); W21 = -W22 T.
 // TIO is the type of the matrices in global memory.  The arithmetic inside the node is FP64 in both cases: for --use-32
 // (TIO = float) the block is widened on load and rounded once on store — the node is latency bound, not FP64-rate bound,
-// so this costs nothing (35 us against 52 us for the FP32 k_node128) and the bottom of the recursion adds no FP32
+// so this costs nothing (35 us against 52 us for the first-generation node in FP32) and the bottom of the recursion adds no FP32
 // rounding of its own.
 template <bool PROF = false, typename TIO = double>
 __global__ void __launch_bounds__(256) k_node128_v2(TIO* __restrict__ A, TIO* __restrict__ W, long mstride, int np, int r0g,
