@@ -224,6 +224,11 @@ struct Model {
     // prm_h[0] is the unclamped value the fit evaluated (fit.rs:96 does not clamp); they differ only when the optimum
     // sits outside the noise bounds by rounding.
     double noise_clamped = 0.0;
+    // How W was computed, which rebuild_nu replays to get the same bits: the recursion over np0 rows of the evaluation
+    // that started the chain, then merge_node(r1, np_k - r1) of each append (model_extend) as (r1, np_k).  An append
+    // recomputes every row of W from its r1 on, so the entries it supersedes (r1_k >= r1) are dropped.
+    int np0 = 0;
+    std::vector<std::pair<int, int>> appends;
     // Retained-model policy (SURVEY F10 / H6: the minimizer keeps EVERY generation's model, minimize.rs:331, :407): only
     // the newest few models of a context keep their n x n factor W = L^-1 on the device.  An older one gives W and its
     // prediction scratch back to the pool (O(n d) stays: X^T / l, alpha, the parameters) and refactorises on its next
@@ -1086,9 +1091,11 @@ struct ModelT : Model {
     int predict_acquisition(int mode, const hbegp_ynorm* yn, long m, const void* xs, double param, void* out1, void* out2,
                             long* best, long* n_below) override;
 
-    // Rebuilds the evicted factor: K from the model's own scaled inputs and parameters, the recursion of the fit, W back
-    // into the model.  The engine's workspaces are used when they are large enough for this model's size, temporary ones
-    // otherwise; the context's current training data is not touched.
+    // Rebuilds the evicted factor: K from the model's own scaled inputs and parameters, then the launches that computed W
+    // (the recursion over np0 rows, and each append's merge_node on K re-assembled from its tile row r1 / 64), W back
+    // into the model.  Rows of W above r1 depend only on rows of K above r1, so the rows of K that were padding when
+    // np0 or an earlier append ran and hold data now do not change them.  The engine's workspaces are used when they are
+    // large enough for this model's size, temporary ones otherwise; the context's current training data is not touched.
     template <int NU2>
     int rebuild_nu() {
         Engine<T>* e = static_cast<Engine<T>*>(eng);
@@ -1119,15 +1126,20 @@ struct ModelT : Model {
         e->n = n; e->np = np; e->d = this->d;  // the recursion reads the matrix size from the engine
         cudaError_t ce = cudaMemcpyAsync(tprm.p, prm_host.data(), (size_t)p * sizeof(T), cudaMemcpyHostToDevice, st);
         if (ce == cudaSuccess) ce = cudaMemsetAsync(e->d_status.p, 0, sizeof(int), st);
-        if (ce == cudaSuccess) {
-            const int nt = (np / TILE) * (np / TILE + 1) / 2;
-            k_assemble<T, NU2><<<dim3(nt, 1, 1), 256, 2 * (size_t)feat_chunk(this->d) * TILE * sizeof(T), st>>>((const T*)xsT.p, (int)n, this->d, np, (const T*)tprm.p, p,
-                                                                                                   (T*)e->A.p, (long)np * np, 0);
+        auto assemble = [&](int row0) {  // the lower tiles of K from tile row row0 / TILE on
+            const int q = row0 / TILE, tile0 = q * (q + 1) / 2, nt = (np / TILE) * (np / TILE + 1) / 2;
+            k_assemble<T, NU2><<<dim3(nt - tile0, 1, 1), 256, 2 * (size_t)feat_chunk(this->d) * TILE * sizeof(T), st>>>(
+                (const T*)xsT.p, (int)n, this->d, np, (const T*)tprm.p, p, (T*)e->A.p, (long)np * np, tile0);
             e->launches++;
-            ce = cudaGetLastError();
-        }
+            return cudaGetLastError();
+        };
+        if (ce == cudaSuccess) ce = assemble(0);
         rc = HBEGP_OK;
-        if (ce == cudaSuccess) rc = e->chol_inv(st, 0, 1, 0, np);
+        if (ce == cudaSuccess) rc = e->chol_inv(st, 0, 1, 0, np0);
+        for (const auto& a : appends) {
+            if (ce != cudaSuccess || rc != HBEGP_OK || a.second == a.first) continue;
+            if ((ce = assemble(a.first)) == cudaSuccess) rc = e->merge_node(st, 0, 1, 0, a.first, a.second - a.first, typename Engine<T>::Side());
+        }
         int hs = 1;
         if (ce == cudaSuccess && rc == HBEGP_OK) ce = cudaMemcpyAsync(W.p, e->W.p, msz, cudaMemcpyDeviceToDevice, st);
         if (ce == cudaSuccess && rc == HBEGP_OK) ce = cudaMemcpyAsync(&hs, e->d_status.p, sizeof(int), cudaMemcpyDeviceToHost, st);
@@ -1344,6 +1356,7 @@ int Engine<T>::finish_model(int nu2, Model** out, double* lml, void* alpha_out, 
     m->n = n;
     m->d = d;
     m->np = np;
+    m->np0 = np;
     m->nu2 = nu2;
     m->c = (double)h_prm[1];
     m->prm_h.assign(h_prm, h_prm + p());
@@ -1395,6 +1408,7 @@ Model* Engine<T>::new_empty_model(int nu2, const std::vector<double>& prm_host, 
     m->n = n;
     m->d = d;
     m->np = np;
+    m->np0 = np;
     m->nu2 = nu2;
     m->c = prm_host[1];
     m->prm_h = prm_host;
@@ -1500,7 +1514,15 @@ int Engine<T>::model_extend(Model* prior_, Model** out, double* lml, void* alpha
         if (appended) *appended = 1;
     }
     if (g_trace_model) fprintf(stderr, "[hbegp] model_extend: %s %.3f ms\n", r1 ? "append" : "full evaluation", now_ms() - t_start);
-    return finish_model(nu2, out, lml, alpha_out, kinv_out);
+    if ((rc = finish_model(nu2, out, lml, alpha_out, kinv_out))) return rc;
+    if (r1 > 0) {
+        Model* m = *out;
+        m->np0 = prior->np0;
+        for (const auto& a : prior->appends)
+            if (a.first < r1) m->appends.push_back(a);
+        m->appends.emplace_back(r1, np);
+    }
+    return HBEGP_OK;
 }
 
 // cudaFuncSetAttribute for every GEMM instantiation up front (never inside a stream capture)
@@ -2604,6 +2626,8 @@ int hbegp_multi_model_create(hbegp_multi* mm, double nu, const double* theta, co
             hbegp_multi_model_destroy(h);
             return fail(HBEGP_ERR_NOMEM, "multi_model_create: could not allocate the replica on GPU " + std::to_string(i));
         }
+        r->np0 = src->np0;
+        r->appends = src->appends;
         h->models.push_back(new hbegp_model{r});
     }
     struct Part {
