@@ -31,9 +31,12 @@
 #include <stdint.h>
 
 #include "gemm.cuh"
+#include "tcgen05.cuh"
 
 namespace hbegp {
 namespace tf32 {
+
+using namespace tc;
 
 // What bounds the main loop now is shared-memory bandwidth: per 32-k block TMA writes 32 KB, the transform reads 32 KB and
 // writes 64 KB, and the twelve MMAs read 96 KB of operands -- 224 KB at 128 B/cycle = 1750 cycles against ~2000 measured
@@ -70,53 +73,6 @@ struct Params {
     int raster_group;
 };
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "WAIT_%=:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-        "@p bra DONE_%=;\n\t"
-        "bra WAIT_%=;\n\t"
-        "DONE_%=:\n\t"
-        "}\n" ::"r"(smem_u32(bar)),
-        "r"(parity)
-        : "memory");
-}
-
-__device__ __forceinline__ void tma_load_3d(const CUtensorMap* map, uint64_t* bar, void* dst, int c0, int c1, int c2) {
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::"r"(
-            smem_u32(dst)),
-        "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
-        : "memory");
-}
-
-// Shared-memory matrix descriptor (tcgen05, version 1); offsets in bytes.  layout: 2 = SWIZZLE_128B (16-byte chunks
-// XOR row mod 8; K-major operands), 1 = SWIZZLE_128B_BASE32B (32-byte chunks XOR row mod 4) -- the only layout the
-// tensor core accepts for MN-major 32-bit operands (it transposes 32-bit elements, so the swizzle granule is 32 bytes);
-// TMA writes it with CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B.
-__device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo, uint32_t sbo, uint32_t layout) {
-    uint64_t d = 0;
-    d |= (uint64_t)((saddr >> 4) & 0x3FFF);
-    d |= (uint64_t)((lbo >> 4) & 0x3FFF) << 16;
-    d |= (uint64_t)((sbo >> 4) & 0x3FFF) << 32;
-    d |= (uint64_t)1 << 46;  // descriptor version (Blackwell)
-    d |= (uint64_t)layout << 61;
-    return d;
-}
-
 // Instruction descriptor: D fp32, A / B tf32, M = 128, N = 128; a_major / b_major: 0 = K-major, 1 = MN-major.
 __host__ __device__ constexpr uint32_t make_idesc(bool a_kmajor, bool b_kmajor, int n) {
     return (1u << 4) | (2u << 7) | (2u << 10) | ((a_kmajor ? 0u : 1u) << 15) | ((b_kmajor ? 0u : 1u) << 16) |
@@ -133,22 +89,6 @@ __device__ __forceinline__ void mma_tf32(uint32_t tmem_d, uint64_t adesc, uint64
         "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
         : "memory");
 }
-__device__ __forceinline__ void mma_commit(uint64_t* bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float* v) {
-    uint32_t* r = reinterpret_cast<uint32_t*>(v);
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, %17, "
-        "%18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
-          "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]), "=r"(r[18]),
-          "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]),
-          "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-        : "r"(taddr));
-}
-
 // Round to TF32 (11 significand bits), nearest with ties away from zero -- what cvt.rna.tf32.f32 does -- as two integer
 // operations.  nvcc expands cvt.rna.tf32.f32 into ~7 instructions on sm_100a (shift / add / mask plus Inf-NaN
 // special-casing, see the SASS), and with 128 elements per thread and k-block the four transform warps were ISSUE
@@ -352,7 +292,7 @@ __global__ void __launch_bounds__(THREADS, 1) gemm_tf32x3_kernel(const __grid_co
 #pragma unroll
             for (int c0 = 0; c0 < BN; c0 += 32) {
                 float v[32];
-                tmem_ld32(lane_addr + buf * BN + c0, v);
+                tmem_ld32(lane_addr + buf * BN + c0, reinterpret_cast<uint32_t*>(v));
                 asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 #pragma unroll
                 for (int j = 0; j < 32; j++) acc[c0 + j] += v[j];
@@ -370,7 +310,7 @@ __global__ void __launch_bounds__(THREADS, 1) gemm_tf32x3_kernel(const __grid_co
         for (int c0 = 0; c0 < BN; c0 += 32) {
             float small[32];
             if (nk > 0) {
-                tmem_ld32(lane_addr + NBUF * BN + c0, small);
+                tmem_ld32(lane_addr + NBUF * BN + c0, reinterpret_cast<uint32_t*>(small));
                 asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
             } else {
 #pragma unroll
@@ -412,21 +352,6 @@ __global__ void __launch_bounds__(THREADS, 1) gemm_tf32x3_kernel(const __grid_co
 }
 
 // ---- host side -------------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-inline EncodeTiledFn encode_fn() {
-    static EncodeTiledFn fn = []() -> EncodeTiledFn {
-        void* f = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess)
-            return nullptr;
-        return reinterpret_cast<EncodeTiledFn>(f);
-    }();
-    return fn;
-}
-
 // Tensor map of one operand: `rows` x `kdim` elements of which the k-major flavour has k contiguous (X[r * ld + k]) and
 // the other has rows contiguous (X[k * ld + r]); third dimension = batch.  Boxes: (BK k, 128 rows) resp. (32 rows, BK k).
 inline bool make_operand_map(CUtensorMap* map, const float* base, bool kmajor, int rows, int kdim, long ld, long batch_stride, int batch) {

@@ -27,6 +27,7 @@
 #include "../../include/hbegp.h"
 #include "gemm.cuh"
 #include "gemm_tf32.cuh"
+#include "gemm_i8.cuh"
 #include "kernels.cuh"
 #include "node_mma.cuh"
 #include "lbfgs.h"
@@ -298,6 +299,7 @@ struct Engine : EngineBase {
     // batched workspaces (capacity `cap` evaluations)
     int cap = 0;
     DevBuf A, W, xsT, prm, u, alpha, ldp, tpart, gpart, d_lml, d_grad, d_status;
+    DevBuf oz;  // residue planes of the emulated K^-1 product (gemm_i8.cuh), oz::slot_bytes(np) per evaluation
     // CUDA graphs of whole batched evaluations, keyed by (nu2, count, want_grad, want_kinv, phase): the fit
     // loop replays the same launch sequence hundreds of times, and at small n the host launch rate (hundreds
     // of kernels per evaluation) would otherwise be the bottleneck.
@@ -351,7 +353,7 @@ struct Engine : EngineBase {
 
     ~Engine() override {
         drop_graphs();
-        for (DevBuf* b : {&dX, &dY, &A, &W, &xsT, &prm, &u, &alpha, &ldp, &tpart, &gpart, &d_lml, &d_grad, &d_status})
+        for (DevBuf* b : {&dX, &dY, &A, &W, &xsT, &prm, &u, &alpha, &ldp, &tpart, &gpart, &d_lml, &d_grad, &d_status, &oz})
             b->release();
         if (h_prm) cudaFreeHost(h_prm);
         if (h_out) cudaFreeHost(h_out);
@@ -409,6 +411,7 @@ struct Engine : EngineBase {
         s += (size_t)d * np * sizeof(T) + (size_t)p() * sizeof(T) + 2 * (size_t)np * sizeof(T);
         s += (size_t)(np / TILE) * sizeof(T) + (size_t)nchunks() * np * sizeof(T);
         s += (size_t)ntiles_lower() * p() * sizeof(double) + (size_t)(p() + 1) * sizeof(double) + sizeof(int);
+        if (kinv_emulated()) s += oz::slot_bytes(np);
         return s;
     }
 
@@ -419,7 +422,7 @@ struct Engine : EngineBase {
         size_t fr = 0, tot = 0;
         CUDA_TRY(cudaMemGetInfo(&fr, &tot));
         // memory already held by the current workspaces (and parked in the model pool) is reusable
-        const size_t held = A.bytes + W.bytes + gpart.bytes + tpart.bytes + xsT.bytes;
+        const size_t held = A.bytes + W.bytes + gpart.bytes + tpart.bytes + xsT.bytes + oz.bytes;
         if (limit == 0) limit = (size_t)((double)(fr + held + model_pool.held) * 0.7);
         size_t per = per_slot_bytes();
         int fit = (int)std::min<size_t>(limit / per, 4096);
@@ -442,6 +445,7 @@ struct Engine : EngineBase {
         if ((rc = d_lml.ensure(c * sizeof(double)))) return rc;
         if ((rc = d_grad.ensure(c * p() * sizeof(double)))) return rc;
         if ((rc = d_status.ensure(((size_t)c + 1) * sizeof(int)))) return rc;  // + the prefix check of model_extend
+        if (kinv_emulated() && (rc = oz.ensure(c * oz::slot_bytes(np)))) return rc;
         if (h_prm_bytes < c * p() * sizeof(T)) {
             if (h_prm) cudaFreeHost(h_prm);
             h_prm_bytes = c * p() * sizeof(T);
@@ -556,8 +560,26 @@ struct Engine : EngineBase {
     static constexpr long SMALL_TILE_CTAS = 296;
     static constexpr int SMALL_TILE_NP = 1024;
 
+    // The f64 K^-1 = W^T W runs on the integer tensor cores (Ozaki scheme II, gemm_i8.cuh) from this padded size on;
+    // below it the DMMA kernel is faster.  Measured (B200, 1000 W; probes/kinv_emul_bench.py, hbegp_bench_phase 5, ms
+    // DMMA / emulated): B = 65: n = 1536 2.62 / 3.25, 2048 5.90 / 5.77, 3072 18.9 / 14.4, 4096 43.7 / 27.2; B = 1:
+    // n = 1536 0.111 / 0.142, 2048 0.178 / 0.210, 4096 0.715 / 0.612.  K^-1 feeds only the gradient contraction and the
+    // caller's kinv, so the LML, alpha, W and every prediction keep their bits either way.  Depends on T and np alone,
+    // so that a batch, its B = 1 evaluations, graph replays, models and debug_factor agree.
+    static constexpr int OZ_MIN_NP = 2048;
+    bool kinv_emulated() const { return std::is_same<T, double>::value && np >= OZ_MIN_NP; }
+
     // K^-1 = W^T W on the lower tiles, written over the (dead) Cholesky factor in A
-    int lauum(cudaStream_t st, T* Ab, T* Wb, int cnt) {
+    int lauum(cudaStream_t st, int s0, int cnt) {
+        T* Ab = (T*)A.p + (size_t)s0 * mstride();
+        T* Wb = (T*)W.p + (size_t)s0 * mstride();
+        if constexpr (std::is_same<T, double>::value) {
+            if (kinv_emulated()) {
+                CUDA_TRY(oz::launch_kinv(Wb, Ab, mstride(), np, cnt, (unsigned char*)oz.p + (size_t)s0 * oz::slot_bytes(np), st));
+                launches += 4;
+                return HBEGP_OK;
+            }
+        }
         GemmArgs<T> g{};
         g.lda = g.ldb = g.ldc = np;
         g.sA = g.sB = g.sC = mstride();
@@ -585,7 +607,7 @@ struct Engine : EngineBase {
         T* tp = (T*)tpart.p + (size_t)s0 * nchunks() * np;
         double* gp = (double*)gpart.p + (size_t)s0 * ntiles_lower() * p();
         const size_t xsm = 2 * (size_t)feat_chunk(d) * TILE * sizeof(T);
-        if (phase == 5) return lauum(st, Ab, Wb, cnt);  // benchmark only: the K^-1 product on the W of the last evaluation
+        if (phase == 5) return lauum(st, s0, cnt);  // benchmark only: the K^-1 product on the W of the last evaluation
         k_scale_x<T><<<dim3((np + 255) / 256, d, cnt), 256, 0, st>>>((const T*)dX.p, (int)n, d, np, pr, p(), xs);
         launches++;
         k_assemble<T, NU2><<<dim3(ntiles_lower(), 1, cnt), 256, xsm, st>>>(xs, (int)n, d, np, pr, p(), Ab, mstride(), 0);
@@ -612,7 +634,7 @@ struct Engine : EngineBase {
         launches++;
         if (split) CUDA_TRY(cudaEventRecord(sd.b, sd.st));
         if (want_grad || want_kinv) {
-            if ((rc = lauum(st, Ab, Wb, cnt))) return rc;
+            if ((rc = lauum(st, s0, cnt))) return rc;
         }
         if (split) CUDA_TRY(cudaStreamWaitEvent(st, sd.b, 0));
         if (phase < 3) return HBEGP_OK;
@@ -918,6 +940,7 @@ struct Engine : EngineBase {
         CUDA_TRY(cudaSetDevice(device));
         if (A.p) CUDA_TRY(cudaMemsetAsync(A.p, 0xFF, A.bytes, stream));
         if (W.p) CUDA_TRY(cudaMemsetAsync(W.p, 0xFF, W.bytes, stream));
+        if (oz.p) CUDA_TRY(cudaMemsetAsync(oz.p, 0xFF, oz.bytes, stream));
         CUDA_TRY(cudaStreamSynchronize(stream));
         return HBEGP_OK;
     }
@@ -949,7 +972,7 @@ struct Engine : EngineBase {
         if ((rc = chol_inv(stream, 0, 1, 0, np))) { tmp.release(); return rc; }
         if (w && (rc = copy_out((T*)W.p, w, 1))) { tmp.release(); return rc; }
         if (kinv) {
-            if ((rc = lauum(stream, (T*)A.p, (T*)W.p, 1))) { tmp.release(); return rc; }
+            if ((rc = lauum(stream, 0, 1))) { tmp.release(); return rc; }
             if ((rc = copy_out((T*)A.p, kinv, 0))) { tmp.release(); return rc; }
         }
         int hs = 0;
@@ -1451,7 +1474,7 @@ int Engine<T>::append_nu(ModelT<T>* prior, int r1, bool want_kinv) {
     launches++;
     k_sum_chunks<T><<<dim3((np + 255) / 256, 1, 1), 256, 0, st>>>((T*)tpart.p, nchunks(), np, (T*)alpha.p, np);
     launches++;
-    if (want_kinv && (rc = lauum(st, Ab, Wb, 1))) return rc;
+    if (want_kinv && (rc = lauum(st, 0, 1))) return rc;
     k_finish<T><<<1, 256, 0, st>>>((const T*)dY.p, (T*)alpha.p, np, (int)n, np, (T*)ldp.p, np / TILE, (double*)gpart.p,
                                   (long)ntiles_lower() * p(), ntiles_lower(), p(), (int*)d_status.p, (double*)d_lml.p,
                                   (double*)d_grad.p, 0);
@@ -1548,6 +1571,8 @@ static int configure_gemms() {
         CUDA_TRY((tf32::configure<true, true>()));
         CUDA_TRY((tf32::configure<true, false>()));
         CUDA_TRY((tf32::configure<false, false>()));
+    } else {
+        CUDA_TRY(oz::configure());
     }
     // kernels whose dynamic shared memory grows with the feature count d (two d x 64 operand tiles)
     const int big = (int)kMaxFeatureSmem;
