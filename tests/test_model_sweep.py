@@ -18,6 +18,7 @@ from oracle.gpr import BoundedValue
 from tests.test_dispatch_sweep import (DTYPES, EPS32, FLOOR, RATIO, TILE, _check_predict, _ctx, _gemm_kind, _lapack_f32,
                                        _name, _note, _np, _predict_path, _predict_truth, _recursion, _reference,
                                        _rounded, _split, _thetas, _worst_tile)
+from tests.test_kinv_emulation import _emulated
 from tests.util import oracle_kernel, oracle_lml, random_thetas, synth
 
 # ------------------------------------------------------------------------------------------------ dispatch restated
@@ -63,6 +64,8 @@ def _append_plan(n_prior, n, f32):
         v.add("r1 < n_prior")
     for op in _append_ops(n_prior, n):
         v.add(op[0] if op[0] != "gemm" else (op[1], _gemm_kind(np_, op[2], op[3], op[4], 1, f32)))
+    if _emulated(np_, f32):  # the lauum on the integer tensor cores (tests/test_kinv_bits.py)
+        v.add("K^-1 emulated")
     return v
 
 
@@ -75,6 +78,8 @@ APPEND_SHAPES = [
     (1000, 1100),  # np 1152: 64x64 tiles; r1 = 896 < 1000
     (1100, 1600),  # r1 = 1024, np 1600: 64x64 tiles and ragged 3xTF32 tiles
     (640, 640),    # np = r1: only the copy of W11, alpha and K^-1
+    (1900, 2100),  # prior np 1920, np 2112: K^-1 emulated, the workspace of the emulation first allocated by extend
+    (2100, 2300),  # r1 = 2048, np 2304: both sides emulated, b = 48
 ]
 
 
@@ -85,7 +90,7 @@ def test_append_shapes_reach_every_variant():
         for f32 in (False, True):
             for v in _append_plan(n_prior, n, f32):
                 reached.setdefault(v, set()).add((n_prior, n, "f32" if f32 else "f64"))
-    req = {"leaf", "node", "s2 = 0", "prior np not a multiple of 128", "r1 < n_prior"}
+    req = {"leaf", "node", "s2 = 0", "prior np not a multiple of 128", "r1 < n_prior", "K^-1 emulated"}
     for cls in range(5):
         req |= {(cls, "32x32"), (cls, "64x64"), (cls, "tf32"), (cls, "tf32 ragged")}
     missing = sorted(map(str, req - set(reached)))
@@ -102,6 +107,7 @@ def test_append_shapes_reach_every_variant():
     assert all((c, "64x64") in _append_plan(1000, 1100, False) for c in range(5)) and _r1(1000, 1100) == 896
     assert {(c, "tf32 ragged") for c in range(5)} <= _append_plan(1100, 1600, True)
     assert _append_ops(640, 640, False) == []
+    assert not _emulated(_np(1900)) and _emulated(_np(2100)) and _r1(2100, 2300) == 2048 and _emulated(2048)
 
 
 def test_append_falls_back_to_the_full_evaluation():
