@@ -166,16 +166,18 @@ def _kernel_f64(x1, x2, c, ls, nu):
     return c * (1 + t + t * t / 3) * np.exp(-t)
 
 
-def _reference(theta, x, y, nu=2.5):
+def _reference(theta, x, y, nu=2.5, k=None):
     """LML, gradient, alpha, K, W = L^-1 and K^-1 in f64 (cho_factor / dtrtri).  Gradient component k is
-    1/2 tr((alpha alpha^T - K^-1) dK/dtheta_k), one n x n slice at a time (matern_kernel.rs:83-135)."""
+    1/2 tr((alpha alpha^T - K^-1) dK/dtheta_k), one n x n slice at a time (matern_kernel.rs:83-135).  A given K
+    (the symmetric matrix the GPU assembled, say) replaces the host's kc + noise I in the LAPACK steps."""
     x = np.asarray(x, dtype=np.float64)
     y = np.asarray(y, dtype=np.float64)
     n, d = x.shape
     noise, c, ls = math.exp(theta[0]), math.exp(theta[1]), np.exp(np.asarray(theta[2:], dtype=np.float64))
     kc = _kernel_f64(x, x, c, ls, nu)
-    k = kc.copy()
-    k[np.diag_indices(n)] += noise
+    if k is None:
+        k = kc.copy()
+        k[np.diag_indices(n)] += noise
     low, _ = cho_factor(k, lower=True)
     low = np.tril(low)
     r = SimpleNamespace(k=k)
