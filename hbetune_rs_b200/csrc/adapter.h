@@ -119,8 +119,9 @@ static inline double norm_pdf(double z) { return std::exp(-0.5 * z * z) / std::s
 
 // expected_improvement (acquisition.rs:141-171); NaN signals the reference's assertion failures
 static inline double expected_improvement(double mean, double std, double fmin) {
-    if (!std::isfinite(mean) || !std::isfinite(std) || !std::isfinite(fmin)) return std::numeric_limits<double>::quiet_NaN();
-    if (ei_std_is_zero(std)) return mean < fmin ? -(mean - fmin) : 0.0;  // kernels.cuh (shared with k_acquisition)
+    // both predicates live in kernels.cuh, shared with k_acquisition
+    if (!ei_inputs_finite(mean, std, fmin)) return std::numeric_limits<double>::quiet_NaN();
+    if (ei_std_is_zero(std)) return mean < fmin ? -(mean - fmin) : 0.0;
     const double z = -(mean - fmin) / std;
     return -(mean - fmin) * norm_cdf(z) + std * norm_pdf(z);
 }

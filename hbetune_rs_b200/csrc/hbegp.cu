@@ -250,7 +250,7 @@ struct Model {
     void release_all() {
         W.release(); alpha.release(); xsT.release(); ls.release(); ldp.release();
         kstar.release(); part.release(); pmean.release(); nbelow.release(); xs_tmp.release(); mean_tmp.release(); var_tmp.release();
-        acq1.release(); acq2.release(); argv.release(); argi.release(); warn_rows.release(); warn_vals.release();
+        acq1.release(); acq2.release(); argws.release(); warn_rows.release(); warn_vals.release();
     }
     virtual ~Model() {
         release_all();
@@ -261,10 +261,10 @@ struct Model {
     virtual int predict_sharded(long m, const void* xs, void* mean, void* var, long* n_below) = 0;
     virtual int predict_acquisition(int mode, const hbegp_ynorm* yn, long m, const void* xs, double param, void* out1,
                                     void* out2, long* best, long* n_below) = 0;
-    DevBuf acq1, acq2, argv, argi;
+    DevBuf acq1, acq2, argws;  // argws: the arg-best index, then launch_argbest's workspace
     void use_pool(BufPool* pl) {
         for (DevBuf* b : {&W, &alpha, &xsT, &ls, &ldp, &kstar, &part, &pmean, &nbelow, &xs_tmp, &mean_tmp, &var_tmp, &acq1, &acq2,
-                          &argv, &argi, &warn_rows, &warn_vals})
+                          &argws, &warn_rows, &warn_vals})
             b->pool = pl;
     }
 };
@@ -1306,9 +1306,7 @@ int ModelT<T>::predict_acquisition(int mode, const hbegp_ynorm* yn, long m, cons
     if ((rc = var_tmp.ensure((size_t)m * sizeof(T)))) return rc;
     if ((rc = acq1.ensure((size_t)m * sizeof(T)))) return rc;
     if ((rc = acq2.ensure((size_t)m * sizeof(T)))) return rc;
-    const int nparts = (int)std::min<long>(1024, (m + 255) / 256);
-    if ((rc = argv.ensure((size_t)nparts * sizeof(T)))) return rc;
-    if ((rc = argi.ensure((size_t)(nparts + 1) * sizeof(long)))) return rc;
+    if ((rc = argws.ensure(sizeof(long) + argbest_ws_bytes(m)))) return rc;
     CUDA_TRY(cudaMemcpyAsync(xs_tmp.p, xs, (size_t)m * d * sizeof(T), cudaMemcpyHostToDevice, st));
     if ((rc = predict_device(m, xs_tmp.p, mean_tmp.p, var_tmp.p, nullptr))) return rc;
     YNorm<T> y;
@@ -1325,10 +1323,10 @@ int ModelT<T>::predict_acquisition(int mode, const hbegp_ynorm* yn, long m, cons
     const T* key = (mode == 0) ? (const T*)acq2.p : (const T*)acq1.p;
     long hbest = -1;
     if (best) {
-        k_argbest_part<T><<<nparts, 256, 0, st>>>(key, m, mode == 0 ? 1 : 0, (T*)argv.p, (long*)argi.p);
-        k_argbest_final<T><<<1, 32, 0, st>>>((const T*)argv.p, (const long*)argi.p, nparts, mode == 0 ? 1 : 0, (long*)argi.p + nparts);
+        long* dbest = (long*)argws.p;
+        CUDA_TRY(launch_argbest<T>(key, m, mode == 0 ? 1 : 0, dbest + 1, dbest, st));
         e->launches += 2;
-        CUDA_TRY(cudaMemcpyAsync(&hbest, (long*)argi.p + nparts, sizeof(long), cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaMemcpyAsync(&hbest, dbest, sizeof(long), cudaMemcpyDeviceToHost, st));
     }
     CUDA_TRY(cudaGetLastError());
     if (out1) CUDA_TRY(cudaMemcpyAsync(out1, acq1.p, (size_t)m * sizeof(T), cudaMemcpyDeviceToHost, st));

@@ -20,6 +20,11 @@ __host__ __device__ inline int feat_chunk(int d) { return d < kFeatChunk ? d : k
 // epsilon = f64::EPSILON first, so any |std| <= 2.2e-16 takes the trivial branch (the ULP test that follows can only
 // add denormals, which the first test already covers).  Shared by the host adapter and k_acquisition.
 __host__ __device__ inline bool ei_std_is_zero(double sd) { return sd <= 0.0 || fabs(sd) <= 2.220446049250313e-16; }
+// The reference asserts that mean, std and fmin are finite before anything else (acquisition.rs:141-171); where one is
+// not, expected_improvement is NaN on the host and on the device alike, the std-zero branch included.
+__host__ __device__ inline bool ei_inputs_finite(double mean, double sd, double fmin) {
+    return fabs(mean) <= 1.7976931348623157e308 && fabs(sd) <= 1.7976931348623157e308 && fabs(fmin) <= 1.7976931348623157e308;
+}
 
 // Per-evaluation hyper-parameters, already clamped and rounded to T on the host
 // (src/gpr/fit.rs:94-96): prm[0] = noise, prm[1] = c, prm[2 + k] = l_k.
@@ -851,7 +856,9 @@ __global__ void k_acquisition(const T* __restrict__ mean, const T* __restrict__ 
     if (mode == 0) {
         const double mean_d = (double)mu, std_d = (double)sd;
         double ei;
-        if (ei_std_is_zero(std_d)) {
+        if (!ei_inputs_finite(mean_d, std_d, fmin_n)) {
+            ei = __longlong_as_double(0x7FF8000000000000LL);  // NaN, as the host expected_improvement
+        } else if (ei_std_is_zero(std_d)) {
             ei = mean_d < fmin_n ? -(mean_d - fmin_n) : 0.0;
         } else {
             const double z = -(mean_d - fmin_n) / std_d;
@@ -925,6 +932,27 @@ __global__ void k_argbest_final(const T* __restrict__ pv, const long* __restrict
         }
     }
     *out = bi;
+}
+
+// The arg-best plan: up to kArgbestParts parts of chunk = ceil(m / nparts) elements, one 256-thread block per part, so
+// from m = 256 * 1024 + 1 on a thread sees several elements of its part and trailing parts can be empty.
+constexpr int kArgbestParts = 1024, kArgbestThreads = 256;
+inline int argbest_parts(long m) {
+    const long p = (m + kArgbestThreads - 1) / kArgbestThreads;
+    return (int)(p < kArgbestParts ? (p > 0 ? p : 1) : kArgbestParts);
+}
+// Workspace of launch_argbest: one index and one value per part.
+inline size_t argbest_ws_bytes(long m) { return (size_t)argbest_parts(m) * (sizeof(long) + 8); }
+
+// *out (device) = the arg-best of key[0, m) under the rules of k_argbest_part; asynchronous on `st`.
+template <typename T>
+inline cudaError_t launch_argbest(const T* key, long m, int want_max, void* ws, long* out, cudaStream_t st) {
+    const int nparts = argbest_parts(m);
+    long* pi = static_cast<long*>(ws);
+    T* pv = reinterpret_cast<T*>(pi + nparts);
+    k_argbest_part<T><<<nparts, kArgbestThreads, 0, st>>>(key, m, want_max, pv, pi);
+    k_argbest_final<T><<<1, 32, 0, st>>>(pv, pi, nparts, want_max, out);
+    return cudaGetLastError();
 }
 
 // out[i][j] = (i >= j) ? in[i][j] : in[j][i] for i, j < n  (hermitian fill of potri, lml.rs:62), packed n x n

@@ -233,7 +233,10 @@ struct hbegp_ynorm;
 /* predict_mean_ei_a (src/core/gpr.rs:179-212) for m candidates in one call: mean_out[m] = de-normalised mean,
  * ei_out[m] = expected improvement (acquisition.rs:141-171, evaluated in f64) against fmin given in NATURAL
  * units (it is projected into normalised space in A first, gpr.rs:192-196).  best_index (may be NULL) receives
- * find_best_candidate_by_ei's argmax (acquisition.rs:177-202: the LAST maximum wins).  Any output may be NULL. */
+ * find_best_candidate_by_ei's argmax (acquisition.rs:177-202: the LAST maximum wins).  Any output may be NULL.
+ * ei_out[i] is NaN exactly where hbegp_expected_improvement is: where the mean, sqrt(variance) or the projected fmin
+ * is NaN or infinite (the log projection of fmin <= expected, say), whatever the variance.  NaN rows never win, so
+ * best_index is -1 when every row is NaN; a caller should check it before using it. */
 int hbegp_predict_mean_ei(hbegp_model* model, const struct hbegp_ynorm* yn, long m, const void* xs, double fmin,
                           void* mean_out, void* ei_out, long* best_index, long* n_below_warn);
 /* predict_confidence_bound (src/core/gpr.rs:94-112) for m points: out[m] = location_from(mean + sqrt(var) * cb);
