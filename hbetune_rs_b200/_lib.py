@@ -101,6 +101,12 @@ PROTOTYPES = {
                                         C.c_void_p, C.POINTER(C.c_long), C.POINTER(C.c_long)]),
     "hbegp_predict_confidence_bound": (C.c_int, [C.c_void_p, C.POINTER(YNorm), C.c_long, C.c_void_p, C.c_double,
                                                  C.c_void_p, C.POINTER(C.c_long), C.POINTER(C.c_long)]),
+    "hbegp_predict_grad": (C.c_int, [C.c_void_p, C.c_long, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                     C.POINTER(C.c_long)]),
+    "hbegp_predict_mean_ei_grad": (C.c_int, [C.c_void_p, C.POINTER(YNorm), C.c_long, C.c_void_p, C.c_double, C.c_void_p,
+                                             C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_long)]),
+    "hbegp_predict_confidence_bound_grad": (C.c_int, [C.c_void_p, C.POINTER(YNorm), C.c_long, C.c_void_p, C.c_double,
+                                                      C.c_void_p, C.c_void_p, C.POINTER(C.c_long)]),
     "hbegp_minimize_by_gradient": (C.c_int, [OBJECTIVE_FN, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                              C.c_int, C.POINTER(C.c_double)]),
     "hbegp_rng_seed": (None, [C.c_ulonglong, C.POINTER(C.c_ulonglong)]),

@@ -237,7 +237,7 @@ struct Model {
     bool evicted = false;
     void evict() {
         W.release(); kstar.release(); part.release(); pmean.release(); xs_tmp.release(); mean_tmp.release(); var_tmp.release();
-        acq1.release(); acq2.release();
+        acq1.release(); acq2.release(); gu.release(); gpart.release(); dmean_tmp.release(); dvar_tmp.release();
         evicted = true;
     }
     virtual int ensure_resident() = 0;
@@ -251,6 +251,7 @@ struct Model {
         W.release(); alpha.release(); xsT.release(); ls.release(); ldp.release();
         kstar.release(); part.release(); pmean.release(); nbelow.release(); xs_tmp.release(); mean_tmp.release(); var_tmp.release();
         acq1.release(); acq2.release(); argws.release(); warn_rows.release(); warn_vals.release();
+        gu.release(); gpart.release(); dmean_tmp.release(); dvar_tmp.release();
     }
     virtual ~Model() {
         release_all();
@@ -259,12 +260,16 @@ struct Model {
     virtual int predict_device(long m, const void* xs, void* mean, void* var, long* n_below_device) = 0;
     virtual int predict_host(long m, const void* xs, void* mean, void* var, long* n_below) = 0;
     virtual int predict_sharded(long m, const void* xs, void* mean, void* var, long* n_below) = 0;
+    // dout1 / dout2 (may be NULL): gradients in the candidate of out1 / out2 (hbegp_predict_*_grad)
     virtual int predict_acquisition(int mode, const hbegp_ynorm* yn, long m, const void* xs, double param, void* out1,
-                                    void* out2, long* best, long* n_below) = 0;
+                                    void* out2, long* best, long* n_below, void* dout1, void* dout2) = 0;
+    virtual int predict_grad_host(long m, const void* xs, void* mean, void* var, void* dmean, void* dvar, long* n_below) = 0;
     DevBuf acq1, acq2, argws;  // argws: the arg-best index, then launch_argbest's workspace
+    // gradient path: U = k* W^T (one chunk), the split partials of k_kstar_grad, the gradients of the host entry points
+    DevBuf gu, gpart, dmean_tmp, dvar_tmp;
     void use_pool(BufPool* pl) {
         for (DevBuf* b : {&W, &alpha, &xsT, &ls, &ldp, &kstar, &part, &pmean, &nbelow, &xs_tmp, &mean_tmp, &var_tmp, &acq1, &acq2,
-                          &argws, &warn_rows, &warn_vals})
+                          &argws, &warn_rows, &warn_vals, &gu, &gpart, &dmean_tmp, &dvar_tmp})
             b->pool = pl;
     }
 };
@@ -994,6 +999,7 @@ struct ModelT : Model {
     }
 
     // m <= 64: latency path (see k_kstar_small)
+    bool predicts_small(long m) const { return m <= 64 && (size_t)m * d * sizeof(T) <= 40 * 1024; }
     template <int NU2>
     int predict_small(int m, const T* xs, T* mean, T* var, unsigned long long* nb) {
         Engine<T>* e = static_cast<Engine<T>*>(eng);
@@ -1022,7 +1028,7 @@ struct ModelT : Model {
     int predict_impl(long m, const T* xs, T* mean, T* var, unsigned long long* nb) {
         Engine<T>* e = static_cast<Engine<T>*>(eng);
         cudaStream_t st = e->stream;
-        if (m <= 64 && (size_t)m * d * sizeof(T) <= 40 * 1024) return predict_small<NU2>((int)m, xs, mean, var, nb);
+        if (predicts_small(m)) return predict_small<NU2>((int)m, xs, mean, var, nb);
         const size_t ksm = (2 * (size_t)feat_chunk(d) * TILE + TILE) * sizeof(T);
         const int ttiles = np / TILE;
         // The train tiles are split over grid.y in FIXED groups of 16 (1024 training rows); the partial means are summed
@@ -1112,7 +1118,128 @@ struct ModelT : Model {
     }
 
     int predict_acquisition(int mode, const hbegp_ynorm* yn, long m, const void* xs, double param, void* out1, void* out2,
-                            long* best, long* n_below) override;
+                            long* best, long* n_below, void* dout1, void* dout2) override;
+
+    // Gradients in the candidate of the mean and (dvar != nullptr) the variance of the rows that predict_device(m, xs,
+    // mean, var) has just predicted with var != nullptr; var is that call's output (dvar is 0 where it is 0).  The values
+    // are never recomputed here, so they keep the bits of the plain prediction.
+    //   m <= 64 (predict_small): k* of these rows is still in `kstar`; u = W k* (k_wmatvec_small_store), v = W^T u in
+    //   split partials (k_wtmatvec_small), the gradient kernel over one train tile per CTA, partials summed in tile order.
+    //   m > 64, per chunk: k* again (k_kstar_mean), U = k* W^T (the variance GEMM with C stored), V = U W (K_GE_N) over
+    //   k*, the gradient kernel over the fixed groups of 16 train tiles of k_kstar_mean, partials summed in group order.
+    template <int NU2>
+    int predict_grad_impl(long m, const T* xs, const T* var, T* dmean, T* dvar) {
+        Engine<T>* e = static_cast<Engine<T>*>(eng);
+        cudaStream_t st = e->stream;
+        const int ttiles = np / TILE;
+        const size_t gsm = kstar_grad_smem<T>(d);
+        int rc;
+        if (predicts_small(m)) {
+            const int split_rows = (ttiles + 7) / 8 * TILE, nsplit = (np + split_rows - 1) / split_rows;
+            const int groups = (int)((m + 15) / 16);
+            if ((rc = gpart.ensure((size_t)ttiles * 2 * 64 * d * sizeof(T)))) return rc;
+            if (dvar) {
+                if ((rc = gu.ensure(((size_t)64 + (size_t)nsplit * 64) * np * sizeof(T)))) return rc;
+                T* u = (T*)gu.p;
+                T* pv = u + (size_t)64 * np;
+                k_wmatvec_small_store<T><<<dim3(np / 8, groups), 256, 0, st>>>((const T*)W.p, np, (const T*)kstar.p, (int)m, u);
+                k_wtmatvec_small<T><<<dim3(ttiles, nsplit, groups), 256, 0, st>>>((const T*)W.p, np, u, (int)m, split_rows, pv);
+                e->launches += 2;
+            }
+            const T* pv = dvar ? (const T*)gu.p + (size_t)64 * np : nullptr;
+            k_kstar_grad<T, NU2><<<dim3(1, ttiles), 256, gsm, st>>>(xs, m, 0, d, (const T*)xsT.p, (int)n, np, (const T*)ls.p,
+                                                                   (const T*)alpha.p, pv, nsplit, (long)64 * np, 1, (T*)gpart.p, 64);
+            k_grad_finish<T><<<(unsigned)((m * d + 255) / 256), 256, 0, st>>>((const T*)gpart.p, ttiles, 64, m, m, 0, d, (T)c,
+                                                                             (const T*)ls.p, var, dmean, dvar);
+            e->launches += 2;
+            CUDA_TRY(cudaGetLastError());
+            return HBEGP_OK;
+        }
+        const size_t ksm = (2 * (size_t)feat_chunk(d) * TILE + TILE) * sizeof(T);
+        const int tpc = 16, ns = (ttiles + tpc - 1) / tpc;  // k_kstar_mean's fixed train-tile groups
+        const int chunk = (int)std::min<long>(predict_chunk_rows(), round_up(m, 128));
+        if ((rc = gpart.ensure((size_t)ns * 2 * chunk * d * sizeof(T)))) return rc;
+        if (dvar) {
+            if ((rc = kstar.ensure((size_t)chunk * np * sizeof(T)))) return rc;
+            if ((rc = gu.ensure((size_t)chunk * np * sizeof(T)))) return rc;
+            if ((rc = pmean.ensure((size_t)ns * chunk * sizeof(T)))) return rc;  // k_kstar_mean's mean partials, unused
+        }
+        const bool tf = gemm_uses_tf32<T>(np, np);
+        const int bn = tf ? 128 : 64;
+        for (long row0 = 0; row0 < m; row0 += chunk) {
+            const int rows = (int)std::min<long>(chunk, round_up(m - row0, 128));
+            if (dvar) {
+                k_kstar_mean<T, NU2><<<dim3(rows / TILE, ns), 256, ksm, st>>>(xs, m, row0, d, (const T*)xsT.p, (int)n, np, (const T*)ls.p,
+                                                                           (T)c, (const T*)alpha.p, (T*)kstar.p, nullptr, tpc,
+                                                                           (T*)pmean.p, rows);
+                GemmArgs<T> g{};
+                g.A = (const T*)kstar.p; g.lda = np;
+                g.B = (const T*)W.p; g.ldb = np;
+                g.C = (T*)gu.p; g.ldc = np;
+                g.M = rows; g.N = np; g.K = np; g.kmode = K_LE_N;
+                g.alpha = T(1); g.beta = T(0);
+                g.raster_group = (int)std::max<size_t>(1, ((size_t)48 << 20) / ((size_t)bn * np * sizeof(T)));
+                GemmArgs<T> h{};
+                h.A = (const T*)gu.p; h.lda = np;
+                h.B = (const T*)W.p; h.ldb = np;
+                h.C = (T*)kstar.p; h.ldc = np;
+                h.M = rows; h.N = np; h.K = np; h.kmode = K_GE_N;
+                h.alpha = T(1); h.beta = T(0);
+                if constexpr (std::is_same<T, float>::value) {
+                    if (tf) {
+                        CUDA_TRY((tf32::launch<true, true>(g, 1, st)));
+                        CUDA_TRY((tf32::launch<true, false>(h, 1, st)));
+                    } else {
+                        CUDA_TRY((launch_gemm<T, true, true>(g, 1, st)));
+                        CUDA_TRY((launch_gemm<T, true, false>(h, 1, st)));
+                    }
+                } else {
+                    CUDA_TRY((launch_gemm<T, true, true>(g, 1, st)));
+                    CUDA_TRY((launch_gemm<T, true, false>(h, 1, st)));
+                }
+                e->launches += 3;
+            }
+            k_kstar_grad<T, NU2><<<dim3(rows / TILE, ns), 256, gsm, st>>>(xs, m, row0, d, (const T*)xsT.p, (int)n, np, (const T*)ls.p,
+                                                                       (const T*)alpha.p, dvar ? (const T*)kstar.p : nullptr, 1, 0, tpc,
+                                                                       (T*)gpart.p, rows);
+            k_grad_finish<T><<<(unsigned)(((long)rows * d + 255) / 256), 256, 0, st>>>((const T*)gpart.p, ns, rows, rows, m, row0, d, (T)c,
+                                                                                      (const T*)ls.p, var, dmean, dvar);
+            e->launches += 2;
+            CUDA_TRY(cudaGetLastError());
+        }
+        return HBEGP_OK;
+    }
+
+    int predict_grad_device(long m, const T* xs, const T* var, T* dmean, T* dvar) {
+        if (nu2 == 5) return predict_grad_impl<5>(m, xs, var, dmean, dvar);
+        if (nu2 == 3) return predict_grad_impl<3>(m, xs, var, dmean, dvar);
+        return predict_grad_impl<1>(m, xs, var, dmean, dvar);
+    }
+
+    int predict_grad_host(long m, const void* xs, void* mean, void* var, void* dmean, void* dvar, long* n_below) override {
+        if (m < 0 || (m > 0 && (!xs || !mean || !dmean))) return fail(HBEGP_ERR_INVALID, "predict_grad: bad arguments");
+        if (n_below) *n_below = 0;
+        if (m == 0) return HBEGP_OK;
+        Engine<T>* e = static_cast<Engine<T>*>(eng);
+        CUDA_TRY(cudaSetDevice(e->device));
+        const size_t md = (size_t)m * d * sizeof(T);
+        int rc;
+        if ((rc = xs_tmp.ensure(md)) || (rc = mean_tmp.ensure((size_t)m * sizeof(T))) || (rc = var_tmp.ensure((size_t)m * sizeof(T))) ||
+            (rc = dmean_tmp.ensure(md)) || (dvar && (rc = dvar_tmp.ensure(md))))
+            return rc;
+        CUDA_TRY(cudaMemcpyAsync(xs_tmp.p, xs, md, cudaMemcpyHostToDevice, e->stream));
+        if ((rc = predict_device(m, xs_tmp.p, mean_tmp.p, var_tmp.p, nullptr))) return rc;
+        if ((rc = predict_grad_device(m, (const T*)xs_tmp.p, (const T*)var_tmp.p, (T*)dmean_tmp.p, dvar ? (T*)dvar_tmp.p : nullptr))) return rc;
+        CUDA_TRY(cudaMemcpyAsync(mean, mean_tmp.p, (size_t)m * sizeof(T), cudaMemcpyDeviceToHost, e->stream));
+        if (var) CUDA_TRY(cudaMemcpyAsync(var, var_tmp.p, (size_t)m * sizeof(T), cudaMemcpyDeviceToHost, e->stream));
+        CUDA_TRY(cudaMemcpyAsync(dmean, dmean_tmp.p, md, cudaMemcpyDeviceToHost, e->stream));
+        if (dvar) CUDA_TRY(cudaMemcpyAsync(dvar, dvar_tmp.p, md, cudaMemcpyDeviceToHost, e->stream));
+        unsigned long long hb = 0;
+        CUDA_TRY(cudaMemcpyAsync(&hb, nbelow.p, sizeof(hb), cudaMemcpyDeviceToHost, e->stream));
+        CUDA_TRY(cudaStreamSynchronize(e->stream));
+        if (n_below) *n_below = (long)hb;
+        return fetch_warn_list((long)hb);
+    }
 
     // Rebuilds the evicted factor: K from the model's own scaled inputs and parameters, then the launches that computed W
     // (the recursion over np0 rows, and each append's merge_node on K re-assembled from its tile row r1 / 64), W back
@@ -1292,7 +1419,7 @@ struct ModelT : Model {
 // predict + acquisition epilogue + arg-best, all on the device; only the requested vectors come back
 template <typename T>
 int ModelT<T>::predict_acquisition(int mode, const hbegp_ynorm* yn, long m, const void* xs, double param, void* out1,
-                                   void* out2, long* best, long* n_below) {
+                                   void* out2, long* best, long* n_below, void* dout1, void* dout2) {
     if (!yn || m < 0 || (m > 0 && !xs) || (mode != 0 && mode != 1)) return fail(HBEGP_ERR_INVALID, "predict_acquisition: bad arguments");
     if (best) *best = -1;
     if (n_below) *n_below = 0;
@@ -1307,6 +1434,9 @@ int ModelT<T>::predict_acquisition(int mode, const hbegp_ynorm* yn, long m, cons
     if ((rc = acq1.ensure((size_t)m * sizeof(T)))) return rc;
     if ((rc = acq2.ensure((size_t)m * sizeof(T)))) return rc;
     if ((rc = argws.ensure(sizeof(long) + argbest_ws_bytes(m)))) return rc;
+    const bool grad = dout1 || dout2;
+    const size_t md = (size_t)m * d * sizeof(T);
+    if (grad && ((rc = dmean_tmp.ensure(md)) || (rc = dvar_tmp.ensure(md)))) return rc;
     CUDA_TRY(cudaMemcpyAsync(xs_tmp.p, xs, (size_t)m * d * sizeof(T), cudaMemcpyHostToDevice, st));
     if ((rc = predict_device(m, xs_tmp.p, mean_tmp.p, var_tmp.p, nullptr))) return rc;
     YNorm<T> y;
@@ -1331,6 +1461,17 @@ int ModelT<T>::predict_acquisition(int mode, const hbegp_ynorm* yn, long m, cons
     CUDA_TRY(cudaGetLastError());
     if (out1) CUDA_TRY(cudaMemcpyAsync(out1, acq1.p, (size_t)m * sizeof(T), cudaMemcpyDeviceToHost, st));
     if (out2 && mode == 0) CUDA_TRY(cudaMemcpyAsync(out2, acq2.p, (size_t)m * sizeof(T), cudaMemcpyDeviceToHost, st));
+    if (grad) {
+        // dvar is always needed: EI and the confidence bound depend on sqrt(var)
+        if ((rc = predict_grad_device(m, (const T*)xs_tmp.p, (const T*)var_tmp.p, (T*)dmean_tmp.p, (T*)dvar_tmp.p))) return rc;
+        k_acquisition_grad<T><<<(unsigned)((m + 255) / 256), 256, 0, st>>>((const T*)mean_tmp.p, (const T*)var_tmp.p, m, d, mode,
+                                                                          y.projection, y.amplitude, fmin_n, cb, (T*)dmean_tmp.p,
+                                                                          (T*)dvar_tmp.p);
+        e->launches++;
+        CUDA_TRY(cudaGetLastError());
+        if (dout1) CUDA_TRY(cudaMemcpyAsync(dout1, dmean_tmp.p, md, cudaMemcpyDeviceToHost, st));
+        if (dout2 && mode == 0) CUDA_TRY(cudaMemcpyAsync(dout2, dvar_tmp.p, md, cudaMemcpyDeviceToHost, st));
+    }
     unsigned long long hb = 0;
     CUDA_TRY(cudaMemcpyAsync(&hb, nbelow.p, sizeof(hb), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
@@ -1585,6 +1726,9 @@ static int configure_gemms() {
     CUDA_TRY(cudaFuncSetAttribute(k_kstar_mean<T, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
     CUDA_TRY(cudaFuncSetAttribute(k_kstar_mean<T, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
     CUDA_TRY(cudaFuncSetAttribute(k_kstar_mean<T, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
+    CUDA_TRY(cudaFuncSetAttribute(k_kstar_grad<T, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
+    CUDA_TRY(cudaFuncSetAttribute(k_kstar_grad<T, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
+    CUDA_TRY(cudaFuncSetAttribute(k_kstar_grad<T, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
     return HBEGP_OK;
 }
 
@@ -2350,14 +2494,34 @@ int hbegp_predict_mean_ei(hbegp_model* model, const hbegp_ynorm* yn, long m, con
                           void* ei_out, long* best_index, long* n_below_warn) {
     if (!model) return fail(HBEGP_ERR_INVALID, "null model");
     if (!model->m->eng) return fail(HBEGP_ERR_INVALID, "the model's context has been destroyed");
-    return model->m->predict_acquisition(0, yn, m, xs, fmin, mean_out, ei_out, best_index, n_below_warn);
+    return model->m->predict_acquisition(0, yn, m, xs, fmin, mean_out, ei_out, best_index, n_below_warn, nullptr, nullptr);
 }
 
 int hbegp_predict_confidence_bound(hbegp_model* model, const hbegp_ynorm* yn, long m, const void* xs, double cb, void* out,
                                    long* best_index, long* n_below_warn) {
     if (!model) return fail(HBEGP_ERR_INVALID, "null model");
     if (!model->m->eng) return fail(HBEGP_ERR_INVALID, "the model's context has been destroyed");
-    return model->m->predict_acquisition(1, yn, m, xs, cb, out, nullptr, best_index, n_below_warn);
+    return model->m->predict_acquisition(1, yn, m, xs, cb, out, nullptr, best_index, n_below_warn, nullptr, nullptr);
+}
+
+int hbegp_predict_grad(hbegp_model* model, long m, const void* xs, void* mean, void* var, void* dmean, void* dvar, long* n_below_warn) {
+    if (!model) return fail(HBEGP_ERR_INVALID, "null model");
+    if (!model->m->eng) return fail(HBEGP_ERR_INVALID, "the model's context has been destroyed");
+    return model->m->predict_grad_host(m, xs, mean, var, dmean, dvar, n_below_warn);
+}
+
+int hbegp_predict_mean_ei_grad(hbegp_model* model, const hbegp_ynorm* yn, long m, const void* xs, double fmin, void* mean_out,
+                               void* ei_out, void* dmean_out, void* dei_out, long* n_below_warn) {
+    if (!model) return fail(HBEGP_ERR_INVALID, "null model");
+    if (!model->m->eng) return fail(HBEGP_ERR_INVALID, "the model's context has been destroyed");
+    return model->m->predict_acquisition(0, yn, m, xs, fmin, mean_out, ei_out, nullptr, n_below_warn, dmean_out, dei_out);
+}
+
+int hbegp_predict_confidence_bound_grad(hbegp_model* model, const hbegp_ynorm* yn, long m, const void* xs, double cb, void* out,
+                                        void* dout, long* n_below_warn) {
+    if (!model) return fail(HBEGP_ERR_INVALID, "null model");
+    if (!model->m->eng) return fail(HBEGP_ERR_INVALID, "the model's context has been destroyed");
+    return model->m->predict_acquisition(1, yn, m, xs, cb, out, nullptr, nullptr, n_below_warn, dout, nullptr);
 }
 
 int hbegp_minimize_by_gradient(hbegp_objective_fn objective, void* user, int n, double* x, const double* lo,

@@ -823,6 +823,208 @@ __global__ void k_var_finish(const T* __restrict__ part, int ld, int ntiles, lon
     var[row0 + r] = v;
 }
 
+// ------------------------------------------------------------------------------- predict gradients
+// Gradients of the predictive mean and variance in the candidate x (caller's units).  With x~_k = x_k / l_k,
+// X~_jk = X_jk / l_k (division first, as everywhere), s_j = sum_k (x~_k - X~_jk)^2 and dk_factor = -2 dM/ds of
+// matern_grad_terms:  d k*_j / d x_k = -c dk_factor(s_j) (x~_k - X~_jk) / l_k, so
+//   dmean_k = -(c / l_k) sum_j alpha_j dk_factor_j (x~_k - X~_jk),
+//   dvar_k  =  (2 c / l_k) sum_j v_j dk_factor_j (x~_k - X~_jk),   v = K^-1 k* = W^T (W k*).
+// At s = 0 (a candidate on a training point) every Matern order contributes 0 (nu = 1/2: dk_factor is 0 there).
+
+// u[r][i] = sum_{k <= i} W[i][k] k*[r][k] for the 16 candidates of group blockIdx.y: k_wmatvec_small with u stored
+// instead of squared (latency path of the variance gradient).
+template <typename T>
+__global__ void __launch_bounds__(256) k_wmatvec_small_store(const T* __restrict__ W, int np, const T* __restrict__ kstar, int m,
+                                                             T* __restrict__ u) {
+    const int row = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    const int r0 = blockIdx.y * 16;
+    const T* wr = W + (long)row * np;
+    T acc[16];
+#pragma unroll
+    for (int q = 0; q < 16; q++) acc[q] = T(0);
+    for (int k = lane; k <= row; k += 32) {
+        const T wv = wr[k];
+#pragma unroll
+        for (int q = 0; q < 16; q++)
+            if (r0 + q < m) acc[q] = fma(wv, kstar[(long)(r0 + q) * np + k], acc[q]);
+    }
+#pragma unroll
+    for (int q = 0; q < 16; q++) {
+        T v = acc[q];
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+        if (lane == 0 && r0 + q < m) u[(long)(r0 + q) * np + row] = v;
+    }
+}
+
+// v = W^T u for the 16 candidates of group blockIdx.z, the 64 columns of blockIdx.x and the rows
+// [blockIdx.y * split_rows, +split_rows) of W: pv[blockIdx.y][r][col] = sum_{i in split, i >= col} W[i][col] u[r][i].
+// Rows of W are read along the row (64 consecutive columns per step); the 4 row groups of a CTA are summed in order, the
+// splits later by the consumer (k_kstar_grad), also in order.
+template <typename T>
+__global__ void __launch_bounds__(256) k_wtmatvec_small(const T* __restrict__ W, int np, const T* __restrict__ u, int m,
+                                                        int split_rows, T* __restrict__ pv) {
+    __shared__ T red[4][16][TILE];
+    const int tid = threadIdx.x, cl = tid & 63, rg = tid >> 6;
+    const int col = blockIdx.x * TILE + cl, r0 = blockIdx.z * 16;
+    const int ibeg = max(blockIdx.y * split_rows, (int)blockIdx.x * TILE), iend = min(np, (int)(blockIdx.y + 1) * split_rows);
+    T acc[16];
+#pragma unroll
+    for (int q = 0; q < 16; q++) acc[q] = T(0);
+    for (int i = ibeg + rg; i < iend; i += 4) {
+        const T wv = (i >= col) ? W[(long)i * np + col] : T(0);
+#pragma unroll
+        for (int q = 0; q < 16; q++)
+            if (r0 + q < m) acc[q] = fma(wv, u[(long)(r0 + q) * np + i], acc[q]);
+    }
+#pragma unroll
+    for (int q = 0; q < 16; q++) red[rg][q][cl] = acc[q];
+    __syncthreads();
+    for (int e = tid; e < 16 * TILE; e += 256) {
+        const int q = e / TILE, c = e % TILE;
+        if (r0 + q < m)
+            pv[((long)blockIdx.y * 64 + r0 + q) * np + blockIdx.x * TILE + c] = ((red[0][q][c] + red[1][q][c]) + red[2][q][c]) + red[3][q][c];
+    }
+}
+
+constexpr int kGradFeat = 16;  // features per pass of k_kstar_grad (4 per thread)
+
+// Per 64 candidates (grid.x) and the train tiles [blockIdx.y * tiles_per_cta, +tiles_per_cta): re-forms the distances
+// like k_kstar_mean, then gpart[y][0][r][k] = sum_j alpha_j dk_factor_j (x~_rk - X~_jk) and, when V != nullptr,
+// gpart[y][1][r][k] = the same with v_rj = sum_{s < vsplit} V[s * vstride + r * np + j] (summed in split order) in place
+// of alpha_j.  Feature passes of kGradFeat features each; a pass re-forms the distances.  Fixed tiles_per_cta makes a
+// candidate's partials independent of the other rows predicted with it.
+template <typename T>
+__host__ __device__ inline size_t kstar_grad_smem(int d) {
+    return ((size_t)2 * feat_chunk(d) * TILE + 2 * TILE * (TILE + 1) + kGradFeat * TILE) * sizeof(T);
+}
+template <typename T, int NU2>
+__global__ void __launch_bounds__(256) k_kstar_grad(const T* __restrict__ xs, long m, long row0, int d,
+                                                    const T* __restrict__ xsT_train, int n, int np,
+                                                    const T* __restrict__ ls, const T* __restrict__ alpha,
+                                                    const T* __restrict__ V, int vsplit, long vstride, int tiles_per_cta,
+                                                    T* __restrict__ gpart, long gp_rows) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int dc = feat_chunk(d);
+    T* xc = reinterpret_cast<T*>(smem_raw);  // [dc][64] candidates (scaled)
+    T* xt = xc + dc * TILE;                  // [dc][64] train tile
+    T* wm = xt + dc * TILE;                  // [64][65] alpha_j dk_factor
+    T* wv = wm + TILE * (TILE + 1);          // [64][65] v_rj dk_factor
+    T* xg = wv + TILE * (TILE + 1);          // [kGradFeat][64] the pass's features of the train tile
+    const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
+    const int pr = tid & 63, pk = tid >> 6;  // feature pass: candidate row pr, features pk + 4 i
+    const long r0 = (long)blockIdx.x * TILE;
+    const bool want_v = V != nullptr;
+    auto load_candidates = [&](int c0, int dl) {
+        for (int e = tid; e < dl * TILE; e += 256) {
+            int r = e / dl, k = e % dl;
+            long gr = row0 + r0 + r;
+            xc[k * TILE + r] = (gr < m) ? xs[gr * d + c0 + k] / ls[c0 + k] : T(0);
+        }
+    };
+    const int jbeg = blockIdx.y * tiles_per_cta * TILE, jend = min(np, jbeg + tiles_per_cta * TILE);
+    const long gpr = row0 + r0 + pr;
+    if (d <= dc) load_candidates(0, d);  // one chunk: the candidate tile stays for every pass and train tile
+    for (int f0 = 0; f0 < d; f0 += kGradFeat) {
+        T xr[4], am[4], av[4];
+#pragma unroll
+        for (int i = 0; i < 4; i++) {
+            const int k = f0 + pk + 4 * i;
+            xr[i] = (gpr < m && k < d) ? xs[gpr * d + k] / ls[k] : T(0);
+            am[i] = T(0);
+            av[i] = T(0);
+        }
+        for (int j0 = jbeg; j0 < jend; j0 += TILE) {
+            T acc[4][4];
+#pragma unroll
+            for (int a = 0; a < 4; a++)
+#pragma unroll
+                for (int q = 0; q < 4; q++) acc[a][q] = T(0);
+            for (int c0 = 0; c0 < d; c0 += dc) {
+                const int dl = min(dc, d - c0);
+                __syncthreads();
+                for (int e = tid; e < dl * TILE; e += 256) {
+                    int k = e / TILE, r = e % TILE;
+                    xt[e] = xsT_train[(long)(c0 + k) * np + j0 + r];
+                }
+                if (d > dc) load_candidates(c0, dl);
+                __syncthreads();
+                for (int k = 0; k < dl; k++) {
+                    T vi[4], vj[4];
+#pragma unroll
+                    for (int a = 0; a < 4; a++) vi[a] = xc[k * TILE + ty + 16 * a];
+#pragma unroll
+                    for (int q = 0; q < 4; q++) vj[q] = xt[k * TILE + tx + 16 * q];
+#pragma unroll
+                    for (int a = 0; a < 4; a++)
+#pragma unroll
+                        for (int q = 0; q < 4; q++) {
+                            T df = vi[a] - vj[q];
+                            acc[a][q] += df * df;
+                        }
+                }
+            }
+#pragma unroll
+            for (int a = 0; a < 4; a++)
+#pragma unroll
+                for (int q = 0; q < 4; q++) {
+                    const int lr = ty + 16 * a, lj = tx + 16 * q, gj = j0 + lj;
+                    T kval, dkf;
+                    matern_grad_terms<T, NU2>(acc[a][q], kval, dkf);
+                    wm[lr * (TILE + 1) + lj] = (gj < n) ? alpha[gj] * dkf : T(0);
+                    if (want_v) {
+                        T v = T(0);
+                        for (int s = 0; s < vsplit; s++) v += V[s * vstride + (r0 + lr) * (long)np + gj];
+                        wv[lr * (TILE + 1) + lj] = (gj < n) ? v * dkf : T(0);
+                    }
+                }
+            for (int e = tid; e < kGradFeat * TILE; e += 256) {
+                const int k = f0 + e / TILE;
+                xg[e] = (k < d) ? xsT_train[(long)k * np + j0 + e % TILE] : T(0);
+            }
+            __syncthreads();
+            for (int j = 0; j < TILE; j++) {
+                const T w1 = wm[pr * (TILE + 1) + j];
+                const T w2 = want_v ? wv[pr * (TILE + 1) + j] : T(0);
+#pragma unroll
+                for (int i = 0; i < 4; i++) {
+                    const T df = xr[i] - xg[(pk + 4 * i) * TILE + j];
+                    am[i] += w1 * df;
+                    av[i] += w2 * df;
+                }
+            }
+        }
+        T* gm = gpart + ((long)blockIdx.y * 2) * gp_rows * d;
+#pragma unroll
+        for (int i = 0; i < 4; i++) {
+            const int k = f0 + pk + 4 * i;
+            if (k < d) {
+                gm[(r0 + pr) * d + k] = am[i];
+                if (want_v) gm[(gp_rows + r0 + pr) * d + k] = av[i];
+            }
+        }
+    }
+}
+
+// Sums the split partials of k_kstar_grad in split order and scales them: dmean[row0 + r][k] = -c S_mean / l_k,
+// dvar = 2 c S_var / l_k, and dvar = 0 where the predicted variance is 0 (clamped, or a pre-clamp value of exactly 0).  One thread per (row, feature).
+template <typename T>
+__global__ void k_grad_finish(const T* __restrict__ gpart, int nsplit, long gp_rows, long rows, long m, long row0, int d, T c,
+                              const T* __restrict__ ls, const T* __restrict__ var, T* __restrict__ dmean, T* __restrict__ dvar) {
+    const long e = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    const long r = e / d;
+    const int k = (int)(e % d);
+    if (r >= rows || row0 + r >= m) return;
+    T sm = T(0), sv = T(0);
+    for (int y = 0; y < nsplit; y++) {
+        const T* g = gpart + (long)y * 2 * gp_rows * d;
+        sm += g[r * d + k];
+        if (dvar != nullptr) sv += g[(gp_rows + r) * d + k];
+    }
+    dmean[(row0 + r) * d + k] = -(c * sm) / ls[k];
+    if (dvar != nullptr) dvar[(row0 + r) * d + k] = (var[row0 + r] == T(0)) ? T(0) : (T(2) * c * sv) / ls[k];
+}
+
 template <typename T>
 __device__ __forceinline__ T mul_rn(T a, T b);
 template <>
@@ -870,6 +1072,46 @@ __global__ void k_acquisition(const T* __restrict__ mean, const T* __restrict__ 
         out2[r] = (T)ei;
     } else {
         out1[r] = location_from(add_rn<T>(mu, mul_rn<T>(sd, cb)));
+    }
+}
+
+// Chain rules of k_acquisition on (mean, var, dmean, dvar) of one row per thread, in place over the gradients:
+//   dsd = dvar / (2 sd) where sd > 0, else 0;  d location_from(y) = amplitude * dy (linear),
+//   amplitude * exp(y * amplitude) * dy (logarithmic).
+//   mode 0: dmean <- d location_from(mean); dvar <- dEI in f64: -Phi(z) dmean + phi(z) dsd, in the std-zero branch
+//           -dmean where mean < fmin_n and 0 otherwise, NaN in every component where EI is NaN;
+//   mode 1: dmean <- d location_from(mean + cb sd) with dy = dmean + cb dsd.
+template <typename T>
+__global__ void k_acquisition_grad(const T* __restrict__ mean, const T* __restrict__ var, long m, int d, int mode, int proj,
+                                   T amplitude, double fmin_n, T cb, T* __restrict__ dmean, T* __restrict__ dvar) {
+    long r = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= m) return;
+    const T mu = mean[r], sd = dev_sqrt<T>(var[r]);
+    const T y = (mode == 0) ? mu : add_rn<T>(mu, mul_rn<T>(sd, cb));
+    const T lf = proj == 0 ? amplitude : amplitude * dev_exp<T>(mul_rn<T>(y, amplitude));
+    T* gm = dmean + r * d;
+    T* gv = dvar + r * d;
+    const double mean_d = (double)mu, std_d = (double)sd;
+    const bool finite = ei_inputs_finite(mean_d, std_d, fmin_n), zero = ei_std_is_zero(std_d);
+    double cdf = 0.0, pdf = 0.0;
+    if (mode == 0 && finite && !zero) {
+        const double z = -(mean_d - fmin_n) / std_d;
+        cdf = 0.5 * erfc(-z * 0.70710678118654752440);
+        pdf = exp(-0.5 * z * z) * 0.39894228040143267794;
+    }
+    for (int k = 0; k < d; k++) {
+        const T dm = gm[k];
+        const T dsd = (sd > T(0)) ? gv[k] / (T(2) * sd) : T(0);
+        if (mode == 0) {
+            double dei;
+            if (!finite) dei = __longlong_as_double(0x7FF8000000000000LL);
+            else if (zero) dei = mean_d < fmin_n ? -(double)dm : 0.0;
+            else dei = -cdf * (double)dm + pdf * (double)dsd;
+            gm[k] = lf * dm;
+            gv[k] = (T)dei;
+        } else {
+            gm[k] = lf * (dm + cb * dsd);
+        }
     }
 }
 

@@ -171,6 +171,30 @@ class SurrogateModelGPR:
               "hbegp_predict_confidence_bound")
         return out, best.value
 
+    def predict_mean_ei_grad(self, x, fmin):
+        """``hbegp_predict_mean_ei_grad``: (mean, ei, dmean, dei) for the rows of x, the values as
+        ``predict_mean_ei_device`` and the gradients in the candidate of shape (m, d) (dmean de-normalised, dei in
+        normalised units)."""
+        x = np.ascontiguousarray(x, dtype=self.A)
+        m, d = x.shape
+        mean, ei = np.empty(m, dtype=self.A), np.empty(m, dtype=self.A)
+        dmean, dei = np.empty((m, d), dtype=self.A), np.empty((m, d), dtype=self.A)
+        nb = C.c_long(0)
+        check(lib.hbegp_predict_mean_ei_grad(self.fitted.model.single_handle(), C.byref(self.y_norm._raw), m, _ptr(x), float(fmin),
+                                             _ptr(mean), _ptr(ei), _ptr(dmean), _ptr(dei), C.byref(nb)), "hbegp_predict_mean_ei_grad")
+        return mean, ei, dmean, dei
+
+    def predict_confidence_bound_grad(self, x, cb):
+        """``hbegp_predict_confidence_bound_grad``: (bounds, dbounds) for the rows of x, dbounds of shape (m, d)."""
+        x = np.ascontiguousarray(x, dtype=self.A)
+        m, d = x.shape
+        out, dout = np.empty(m, dtype=self.A), np.empty((m, d), dtype=self.A)
+        nb = C.c_long(0)
+        check(lib.hbegp_predict_confidence_bound_grad(self.fitted.model.single_handle(), C.byref(self.y_norm._raw), m, _ptr(x),
+                                                      float(cb), _ptr(out), _ptr(dout), C.byref(nb)),
+              "hbegp_predict_confidence_bound_grad")
+        return out, dout
+
     def predict_mean_ei(self, x, fmin):
         mean, ei = self.predict_mean_ei_a(np.asarray(x)[None, :], fmin)
         return mean[0], ei[0]

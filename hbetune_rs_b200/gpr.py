@@ -376,6 +376,22 @@ class Model:
                   + ", ".join(f"{v:.2e}" for v in vals) + more, file=sys.stderr)
         return mean, var
 
+    def predict_grad(self, xs: np.ndarray, want_variance: bool = True):
+        """``hbegp_predict_grad``: (mean, var, dmean, dvar) with dmean / dvar of shape (m, d), the gradients in the
+        candidate (normalised units; var and dvar are None unless wanted).  Values as ``predict``."""
+        xs = np.ascontiguousarray(xs, dtype=self.A)
+        assert xs.ndim == 2 and xs.shape[1] == self.d
+        m = xs.shape[0]
+        mean = np.empty(m, dtype=self.A)
+        var = np.empty(m, dtype=self.A) if want_variance else None
+        dmean = np.empty((m, self.d), dtype=self.A)
+        dvar = np.empty((m, self.d), dtype=self.A) if want_variance else None
+        nb = C.c_long(0)
+        check(lib.hbegp_predict_grad(self._h, m, _ptr(xs), _ptr(mean), _ptr(var), _ptr(dmean), _ptr(dvar), C.byref(nb)),
+              "hbegp_predict_grad")
+        self.n_below_warn = nb.value
+        return mean, var, dmean, dvar
+
     def single_handle(self):
         return self._h
 

@@ -245,6 +245,34 @@ int hbegp_predict_mean_ei(hbegp_model* model, const struct hbegp_ynorm* yn, long
 int hbegp_predict_confidence_bound(hbegp_model* model, const struct hbegp_ynorm* yn, long m, const void* xs,
                                    double cb, void* out, long* best_index, long* n_below_warn);
 
+/* ---- gradients in the candidate ----------------------------------------------------------------------
+ * x is in the caller's units, as the row-major candidates of hbegp_predict.  With x~_k = x_k / l_k, X~_jk = X_jk / l_k
+ * and s_j = sum_k (x~_k - X~_jk)^2, d k*_j / d x_k = -c dk_factor(s_j) (x~_k - X~_jk) / l_k, dk_factor = -2 dM/ds, so
+ *   dmean = sum_j alpha_j grad k*_j,   dvar = -2 sum_j v_j grad k*_j,  v = K^-1 k*  (normalised units).
+ * Definitions where the functions are not smooth:
+ *   - a term with s_j = 0 (the candidate on a training point) contributes 0, for every nu (for nu = 1/2 the
+ *     derivative does not exist there; the reference's non-finite -> 0 rule gives 0);
+ *   - where the variance is clamped to 0 (its pre-clamp value is < 0, or exactly 0), dvar = 0;
+ *   - d sqrt(var) = dvar / (2 sqrt(var)) where sqrt(var) > 0, else 0;
+ *   - EI (f64, normalised units): -Phi(z) dmean + phi(z) d sqrt(var); in the std-zero branch -dmean where
+ *     mean < fmin and 0 otherwise; NaN in every component where EI is NaN;
+ *   - de-normalisation: amplitude * dy (linear projection), amplitude * exp(y * amplitude) * dy (logarithmic), with
+ *     y = mean for the mean and y = mean + cb sqrt(var) (dy = dmean + cb d sqrt(var)) for the confidence bound.
+ * The values returned equal those of hbegp_predict / _mean_ei / _confidence_bound bit for bit, the calls count as the
+ * last prediction for hbegp_predict_warn_values, and an evicted model is rebuilt first.  A candidate's gradients do not
+ * depend on the other rows predicted with it, among m > 64 rows; the m <= 64 path agrees with it to rounding. */
+/* Gradients of hbegp_predict's outputs: dmean[m*d] (required) and dvar[m*d] (may be NULL), row-major, in the data
+ * type; mean[m] (required) and var[m] (may be NULL) as hbegp_predict. */
+int hbegp_predict_grad(hbegp_model* model, long m, const void* xs, void* mean, void* var, void* dmean, void* dvar,
+                       long* n_below_warn);
+/* hbegp_predict_mean_ei plus dmean_out[m*d] (de-normalised mean) and dei_out[m*d] (EI, normalised units).  Any output
+ * may be NULL. */
+int hbegp_predict_mean_ei_grad(hbegp_model* model, const struct hbegp_ynorm* yn, long m, const void* xs, double fmin,
+                               void* mean_out, void* ei_out, void* dmean_out, void* dei_out, long* n_below_warn);
+/* hbegp_predict_confidence_bound plus dout[m*d].  Either output may be NULL. */
+int hbegp_predict_confidence_bound_grad(hbegp_model* model, const struct hbegp_ynorm* yn, long m, const void* xs,
+                                        double cb, void* out, void* dout, long* n_below_warn);
+
 /* ---- host-side pieces of the reference interface (no GPU needed) -------------------------------- */
 /* Bounded L-BFGS used by hbegp_fit_runs, exposed with a callback objective
  * (objective(x, grad_out, user) -> f), mirroring minimize_by_gradient (src/util/gradmin.rs:35-60).

@@ -223,6 +223,21 @@ std::vector<A> predict(const FittedKernel<A>& fk, const std::vector<A>& x, long 
 
 enum class Projection { Linear = HBEGP_PROJ_LINEAR, Logarithmic = HBEGP_PROJ_LOG };
 
+// hbegp_predict_grad: the mean (returned), its gradient in the candidate (m x d, row-major) into *dmean and, when
+// `variance` is given, the variance and its gradient into *variance / *dvar (normalised units)
+template <typename A>
+std::vector<A> predict_grad(const FittedKernel<A>& fk, const std::vector<A>& x, long m, int d, std::vector<A>* dmean,
+                            std::vector<A>* variance = nullptr, std::vector<A>* dvar = nullptr) {
+    std::vector<A> mean(m);
+    dmean->assign((size_t)m * d, A(0));
+    if (variance) variance->assign(m, A(0));
+    if (dvar) dvar->assign((size_t)m * d, A(0));
+    check(hbegp_predict_grad(fk.model->h, m, x.data(), mean.data(), variance ? variance->data() : nullptr, dmean->data(),
+                             dvar ? dvar->data() : nullptr, nullptr),
+          "hbegp_predict_grad");
+    return mean;
+}
+
 // src/core/ynormalize.rs:158-288
 template <typename A>
 class YNormalize {
@@ -295,6 +310,27 @@ public:
         std::vector<A> out(m);
         check(hbegp_predict_confidence_bound(fitted_.model->h, &y_norm_.raw(), m, x.data(), (double)cb, out.data(), best, nullptr),
               "hbegp_predict_confidence_bound");
+        return out;
+    }
+    // hbegp_predict_mean_ei_grad: (mean, ei) as predict_mean_ei_a, and their gradients in the candidate (m x d,
+    // row-major; dmean de-normalised, dei in normalised units) into *dmean / *dei
+    std::pair<std::vector<A>, std::vector<A>> predict_mean_ei_grad(const std::vector<A>& x, long m, A fmin, std::vector<A>* dmean,
+                                                                   std::vector<A>* dei) const {
+        std::vector<A> mean(m), ei(m);
+        if (dmean) dmean->assign((size_t)m * d_, A(0));
+        if (dei) dei->assign((size_t)m * d_, A(0));
+        check(hbegp_predict_mean_ei_grad(fitted_.model->h, &y_norm_.raw(), m, x.data(), (double)fmin, mean.data(), ei.data(),
+                                         dmean ? dmean->data() : nullptr, dei ? dei->data() : nullptr, nullptr),
+              "hbegp_predict_mean_ei_grad");
+        return {mean, ei};
+    }
+    // hbegp_predict_confidence_bound_grad: the bounds of m points, their gradients (m x d) into *dout
+    std::vector<A> predict_confidence_bound_grad(const std::vector<A>& x, long m, A cb, std::vector<A>* dout) const {
+        std::vector<A> out(m);
+        if (dout) dout->assign((size_t)m * d_, A(0));
+        check(hbegp_predict_confidence_bound_grad(fitted_.model->h, &y_norm_.raw(), m, x.data(), (double)cb, out.data(),
+                                                  dout ? dout->data() : nullptr, nullptr),
+              "hbegp_predict_confidence_bound_grad");
         return out;
     }
     A predict_confidence_bound(const std::vector<A>& x, A cb) const {

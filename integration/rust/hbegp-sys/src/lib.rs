@@ -206,6 +206,19 @@ extern "C" {
         out: *mut c_void, best_index: *mut c_long, n_below_warn: *mut c_long,
     ) -> c_int;
 
+    pub fn hbegp_predict_grad(
+        model: *mut hbegp_model, m: c_long, xs: *const c_void, mean: *mut c_void, var: *mut c_void, dmean: *mut c_void,
+        dvar: *mut c_void, n_below_warn: *mut c_long,
+    ) -> c_int;
+    pub fn hbegp_predict_mean_ei_grad(
+        model: *mut hbegp_model, yn: *const hbegp_ynorm, m: c_long, xs: *const c_void, fmin: c_double,
+        mean_out: *mut c_void, ei_out: *mut c_void, dmean_out: *mut c_void, dei_out: *mut c_void, n_below_warn: *mut c_long,
+    ) -> c_int;
+    pub fn hbegp_predict_confidence_bound_grad(
+        model: *mut hbegp_model, yn: *const hbegp_ynorm, m: c_long, xs: *const c_void, cb: c_double,
+        out: *mut c_void, dout: *mut c_void, n_below_warn: *mut c_long,
+    ) -> c_int;
+
     pub fn hbegp_minimize_by_gradient(
         objective: hbegp_objective_fn, user: *mut c_void, n: c_int, x: *mut c_double, lo: *const c_double,
         hi: *const c_double, maxeval: c_int, f_out: *mut c_double,
