@@ -24,6 +24,16 @@ class RunResult(C.Structure):
     ]
 
 
+class AcqResult(C.Structure):
+    _fields_ = [
+        ("best_value", C.c_double),
+        ("best_eval", C.c_longlong),
+        ("n_evals", C.c_longlong),
+        ("status", C.c_int),
+        ("reserved", C.c_int),
+    ]
+
+
 class YNorm(C.Structure):
     _fields_ = [("amplitude", C.c_double), ("expected", C.c_double), ("projection", C.c_int), ("dtype", C.c_int)]
 
@@ -107,6 +117,12 @@ PROTOTYPES = {
                                              C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_long)]),
     "hbegp_predict_confidence_bound_grad": (C.c_int, [C.c_void_p, C.POINTER(YNorm), C.c_long, C.c_void_p, C.c_double,
                                                       C.c_void_p, C.c_void_p, C.POINTER(C.c_long)]),
+    "hbegp_acquire_ei": (C.c_int, [C.c_void_p, C.POINTER(YNorm), C.c_double, C.c_long, C.c_void_p, C.c_void_p, C.c_void_p,
+                                   C.c_int, C.c_void_p, C.c_void_p, C.POINTER(AcqResult), C.POINTER(C.c_long),
+                                   C.POINTER(C.c_longlong)]),
+    "hbegp_acquire_confidence_bound": (C.c_int, [C.c_void_p, C.POINTER(YNorm), C.c_double, C.c_long, C.c_void_p, C.c_void_p,
+                                                 C.c_void_p, C.c_int, C.c_void_p, C.POINTER(AcqResult), C.POINTER(C.c_long),
+                                                 C.POINTER(C.c_longlong)]),
     "hbegp_minimize_by_gradient": (C.c_int, [OBJECTIVE_FN, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                              C.c_int, C.POINTER(C.c_double)]),
     "hbegp_rng_seed": (None, [C.c_ulonglong, C.POINTER(C.c_ulonglong)]),

@@ -264,6 +264,10 @@ struct Model {
     virtual int predict_acquisition(int mode, const hbegp_ynorm* yn, long m, const void* xs, double param, void* out1,
                                     void* out2, long* best, long* n_below, void* dout1, void* dout2) = 0;
     virtual int predict_grad_host(long m, const void* xs, void* mean, void* var, void* dmean, void* dvar, long* n_below) = 0;
+    // hbegp_acquire_ei (mode 0) / hbegp_acquire_confidence_bound (mode 1)
+    virtual int acquire(int mode, const hbegp_ynorm* yn, double param, long S, const void* starts, const double* lo,
+                        const double* hi, int maxeval, void* x_out, void* mean_out, hbegp_acq_result* results, long* best_index,
+                        long long* n_rounds) = 0;
     DevBuf acq1, acq2, argws;  // argws: the arg-best index, then launch_argbest's workspace
     // gradient path: U = k* W^T (one chunk), the split partials of k_kstar_grad, the gradients of the host entry points
     DevBuf gu, gpart, dmean_tmp, dvar_tmp;
@@ -1119,6 +1123,10 @@ struct ModelT : Model {
 
     int predict_acquisition(int mode, const hbegp_ynorm* yn, long m, const void* xs, double param, void* out1, void* out2,
                             long* best, long* n_below, void* dout1, void* dout2) override;
+    int ensure_acquisition_rows(long m, bool grad);
+    int acquisition_device(int mode, const YNorm<T>& y, long m, double fmin_n, T cb, bool grad);
+    int acquire(int mode, const hbegp_ynorm* yn, double param, long S, const void* starts, const double* lo, const double* hi,
+                int maxeval, void* x_out, void* mean_out, hbegp_acq_result* results, long* best_index, long long* n_rounds) override;
 
     // Gradients in the candidate of the mean and (dvar != nullptr) the variance of the rows that predict_device(m, xs,
     // mean, var) has just predicted with var != nullptr; var is that call's output (dvar is 0 where it is 0).  The values
@@ -1416,6 +1424,68 @@ struct ModelT : Model {
     }
 };
 
+// The winning start of an acquisition search: the largest EI with the last maximum winning (find_best_candidate_by_ei,
+// acquisition.rs:192-200, max_by) or the smallest bound with the first minimum winning (minimize.rs:680-714, strict `<`);
+// starts without a finite value never win.  -1 if no start has one.
+static long acq_best_index(int mode, long S, const hbegp_acq_result* results) {
+    long best = -1;
+    for (long i = 0; i < S; i++) {
+        if (results[i].status != HBEGP_OK) continue;
+        const double v = results[i].best_value;
+        if (best < 0 || (mode == 0 ? v >= results[best].best_value : v < results[best].best_value)) best = i;
+    }
+    return best;
+}
+
+// The device half of predict_acquisition on the m rows in xs_tmp: predict_device -> k_acquisition and, with grad,
+// predict_grad_device -> k_acquisition_grad.  The buffers must hold m rows already.  Leaves the values in acq1 / acq2
+// and the gradients in dmean_tmp / dvar_tmp (see k_acquisition, k_acquisition_grad); issues no copy and no
+// synchronisation, so that the acquisition search can capture it in a graph.
+template <typename T>
+int ModelT<T>::acquisition_device(int mode, const YNorm<T>& y, long m, double fmin_n, T cb, bool grad) {
+    Engine<T>* e = static_cast<Engine<T>*>(eng);
+    cudaStream_t st = e->stream;
+    int rc;
+    if ((rc = predict_device(m, xs_tmp.p, mean_tmp.p, var_tmp.p, nullptr))) return rc;
+    k_acquisition<T><<<(unsigned)((m + 255) / 256), 256, 0, st>>>((const T*)mean_tmp.p, (const T*)var_tmp.p, m, mode, y.projection,
+                                                                 y.amplitude, y.expected, fmin_n, cb, (T*)acq1.p, (T*)acq2.p);
+    e->launches++;
+    CUDA_TRY(cudaGetLastError());
+    if (!grad) return HBEGP_OK;
+    // dvar is always needed: EI and the confidence bound depend on sqrt(var)
+    if ((rc = predict_grad_device(m, (const T*)xs_tmp.p, (const T*)var_tmp.p, (T*)dmean_tmp.p, (T*)dvar_tmp.p))) return rc;
+    k_acquisition_grad<T><<<(unsigned)((m + 255) / 256), 256, 0, st>>>((const T*)mean_tmp.p, (const T*)var_tmp.p, m, d, mode,
+                                                                      y.projection, y.amplitude, fmin_n, cb, (T*)dmean_tmp.p,
+                                                                      (T*)dvar_tmp.p);
+    e->launches++;
+    CUDA_TRY(cudaGetLastError());
+    return HBEGP_OK;
+}
+
+// The normalisation record in the data type, and the parameter of mode 0 (fmin projected into normalised space in A,
+// gpr.rs:192-196) or mode 1 (the confidence-bound factor in A).
+template <typename T>
+static void acquisition_params(int mode, const hbegp_ynorm* yn, double param, YNorm<T>* y, double* fmin_n, T* cb) {
+    y->amplitude = (T)yn->amplitude;
+    y->expected = (T)yn->expected;
+    y->projection = yn->projection;
+    *fmin_n = 0.0;
+    *cb = T(0);
+    if (mode == 0) *fmin_n = (double)y->into((T)param);
+    else *cb = (T)param;
+}
+
+template <typename T>
+int ModelT<T>::ensure_acquisition_rows(long m, bool grad) {
+    const size_t md = (size_t)m * d * sizeof(T);
+    int rc;
+    if ((rc = xs_tmp.ensure(md)) || (rc = mean_tmp.ensure((size_t)m * sizeof(T))) || (rc = var_tmp.ensure((size_t)m * sizeof(T))) ||
+        (rc = acq1.ensure((size_t)m * sizeof(T))) || (rc = acq2.ensure((size_t)m * sizeof(T))))
+        return rc;
+    if (grad && ((rc = dmean_tmp.ensure(md)) || (rc = dvar_tmp.ensure(md)))) return rc;
+    return HBEGP_OK;
+}
+
 // predict + acquisition epilogue + arg-best, all on the device; only the requested vectors come back
 template <typename T>
 int ModelT<T>::predict_acquisition(int mode, const hbegp_ynorm* yn, long m, const void* xs, double param, void* out1,
@@ -1428,28 +1498,16 @@ int ModelT<T>::predict_acquisition(int mode, const hbegp_ynorm* yn, long m, cons
     CUDA_TRY(cudaSetDevice(e->device));
     cudaStream_t st = e->stream;
     int rc;
-    if ((rc = xs_tmp.ensure((size_t)m * d * sizeof(T)))) return rc;
-    if ((rc = mean_tmp.ensure((size_t)m * sizeof(T)))) return rc;
-    if ((rc = var_tmp.ensure((size_t)m * sizeof(T)))) return rc;
-    if ((rc = acq1.ensure((size_t)m * sizeof(T)))) return rc;
-    if ((rc = acq2.ensure((size_t)m * sizeof(T)))) return rc;
-    if ((rc = argws.ensure(sizeof(long) + argbest_ws_bytes(m)))) return rc;
     const bool grad = dout1 || dout2;
     const size_t md = (size_t)m * d * sizeof(T);
-    if (grad && ((rc = dmean_tmp.ensure(md)) || (rc = dvar_tmp.ensure(md)))) return rc;
-    CUDA_TRY(cudaMemcpyAsync(xs_tmp.p, xs, (size_t)m * d * sizeof(T), cudaMemcpyHostToDevice, st));
-    if ((rc = predict_device(m, xs_tmp.p, mean_tmp.p, var_tmp.p, nullptr))) return rc;
+    if ((rc = ensure_acquisition_rows(m, grad))) return rc;
+    if ((rc = argws.ensure(sizeof(long) + argbest_ws_bytes(m)))) return rc;
+    CUDA_TRY(cudaMemcpyAsync(xs_tmp.p, xs, md, cudaMemcpyHostToDevice, st));
     YNorm<T> y;
-    y.amplitude = (T)yn->amplitude;
-    y.expected = (T)yn->expected;
-    y.projection = yn->projection;
-    double fmin_n = 0.0;
-    T cb = T(0);
-    if (mode == 0) fmin_n = (double)y.into((T)param);  // gpr.rs:192-196: fmin projected into normalised space in A
-    else cb = (T)param;
-    k_acquisition<T><<<(unsigned)((m + 255) / 256), 256, 0, st>>>((const T*)mean_tmp.p, (const T*)var_tmp.p, m, mode, y.projection,
-                                                                 y.amplitude, y.expected, fmin_n, cb, (T*)acq1.p, (T*)acq2.p);
-    e->launches++;
+    double fmin_n;
+    T cb;
+    acquisition_params<T>(mode, yn, param, &y, &fmin_n, &cb);
+    if ((rc = acquisition_device(mode, y, m, fmin_n, cb, grad))) return rc;
     const T* key = (mode == 0) ? (const T*)acq2.p : (const T*)acq1.p;
     long hbest = -1;
     if (best) {
@@ -1458,26 +1516,189 @@ int ModelT<T>::predict_acquisition(int mode, const hbegp_ynorm* yn, long m, cons
         e->launches += 2;
         CUDA_TRY(cudaMemcpyAsync(&hbest, dbest, sizeof(long), cudaMemcpyDeviceToHost, st));
     }
-    CUDA_TRY(cudaGetLastError());
     if (out1) CUDA_TRY(cudaMemcpyAsync(out1, acq1.p, (size_t)m * sizeof(T), cudaMemcpyDeviceToHost, st));
     if (out2 && mode == 0) CUDA_TRY(cudaMemcpyAsync(out2, acq2.p, (size_t)m * sizeof(T), cudaMemcpyDeviceToHost, st));
-    if (grad) {
-        // dvar is always needed: EI and the confidence bound depend on sqrt(var)
-        if ((rc = predict_grad_device(m, (const T*)xs_tmp.p, (const T*)var_tmp.p, (T*)dmean_tmp.p, (T*)dvar_tmp.p))) return rc;
-        k_acquisition_grad<T><<<(unsigned)((m + 255) / 256), 256, 0, st>>>((const T*)mean_tmp.p, (const T*)var_tmp.p, m, d, mode,
-                                                                          y.projection, y.amplitude, fmin_n, cb, (T*)dmean_tmp.p,
-                                                                          (T*)dvar_tmp.p);
-        e->launches++;
-        CUDA_TRY(cudaGetLastError());
-        if (dout1) CUDA_TRY(cudaMemcpyAsync(dout1, dmean_tmp.p, md, cudaMemcpyDeviceToHost, st));
-        if (dout2 && mode == 0) CUDA_TRY(cudaMemcpyAsync(dout2, dvar_tmp.p, md, cudaMemcpyDeviceToHost, st));
-    }
+    if (dout1) CUDA_TRY(cudaMemcpyAsync(dout1, dmean_tmp.p, md, cudaMemcpyDeviceToHost, st));
+    if (dout2 && mode == 0) CUDA_TRY(cudaMemcpyAsync(dout2, dvar_tmp.p, md, cudaMemcpyDeviceToHost, st));
     unsigned long long hb = 0;
     CUDA_TRY(cudaMemcpyAsync(&hb, nbelow.p, sizeof(hb), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     if (best) *best = hbest;
     if (n_below) *n_below = (long)hb;
     return fetch_warn_list((long)hb);
+}
+
+// Rounds of the acquisition search between two looks of the host at the live count (HBEGP_ACQ_ROUNDS overrides it for
+// measurements): each look is a device-to-host copy and a synchronisation; up to R - 1 rounds after the last start
+// finished are wasted once per search.
+static int acq_rounds_per_look() {
+    const char* v = getenv("HBEGP_ACQ_ROUNDS");
+    const int r = v ? atoi(v) : 0;
+    return r > 0 ? r : 4;
+}
+
+template <typename T>
+int ModelT<T>::acquire(int mode, const hbegp_ynorm* yn, double param, long S, const void* starts, const double* lo,
+                       const double* hi, int maxeval, void* x_out, void* mean_out, hbegp_acq_result* results, long* best_index,
+                       long long* n_rounds) {
+    const char* what = mode == 0 ? "acquire_ei" : "acquire_confidence_bound";
+    if (!yn || !lo || !hi || S < 0 || maxeval < 0 || (S > 0 && (!starts || !x_out || !results)) || !best_index || !n_rounds)
+        return fail(HBEGP_ERR_INVALID, std::string(what) + ": bad arguments");
+    for (int k = 0; k < d; k++)
+        if (!std::isfinite(lo[k]) || !std::isfinite(hi[k]) || lo[k] > hi[k])
+            return fail(HBEGP_ERR_INVALID, std::string(what) + ": the bounds must be finite with lo <= hi");
+    const T* x0 = (const T*)starts;
+    for (size_t t = 0; t < (size_t)S * d; t++)
+        if (!std::isfinite((double)x0[t])) return fail(HBEGP_ERR_INVALID, std::string(what) + ": a start point is not finite");
+    *best_index = -1;
+    *n_rounds = 0;
+    if (S == 0) return HBEGP_OK;
+    const size_t Sd = (size_t)S * d;
+    // the clamped starts (BoundedLbfgs's constructor) and the records of a start that evaluated nothing
+    std::vector<double> xt0(Sd);
+    for (size_t t = 0; t < Sd; t++) xt0[t] = std::min(std::max((double)x0[t], lo[t % d]), hi[t % d]);
+    for (long i = 0; i < S; i++) results[i] = {std::numeric_limits<double>::quiet_NaN(), -1, 0, HBEGP_NOT_PD, 0};
+    if (maxeval == 0) {
+        for (size_t t = 0; t < Sd; t++) ((T*)x_out)[t] = (T)xt0[t];
+        if (mean_out && mode == 0)
+            for (long i = 0; i < S; i++) ((T*)mean_out)[i] = std::numeric_limits<T>::quiet_NaN();
+        return HBEGP_OK;
+    }
+    Engine<T>* e = static_cast<Engine<T>*>(eng);
+    CUDA_TRY(cudaSetDevice(e->device));
+    cudaStream_t st = e->stream;
+    int rc;
+    if ((rc = ensure_resident())) return rc;
+    if ((rc = ensure_acquisition_rows(S, true))) return rc;
+    // one device buffer: scalars | x g xt dir (S d) | s y (S M d) | a (S M) | lo hi (d) | best x (S d, T) | best mean (S, T)
+    // | free flags (S d) | live count; set up on the host and copied up once
+    const int M = kAcqMemory;
+    const size_t n_sc = (size_t)S * sizeof(AcqScalars), n_vec = Sd * sizeof(double), n_mem = Sd * M * sizeof(double);
+    const size_t o_x = n_sc, o_g = o_x + n_vec, o_xt = o_g + n_vec, o_dir = o_xt + n_vec, o_s = o_dir + n_vec, o_y = o_s + n_mem,
+                 o_a = o_y + n_mem, o_lo = o_a + (size_t)S * M * sizeof(double), o_hi = o_lo + d * sizeof(double),
+                 o_bx = o_hi + d * sizeof(double), o_bm = o_bx + (Sd * sizeof(T) + 7) / 8 * 8,
+                 o_fr = o_bm + ((size_t)S * sizeof(T) + 7) / 8 * 8, o_live = o_fr + (Sd + 7) / 8 * 8, total = o_live + 8;
+    std::vector<unsigned char> h(total, 0);
+    AcqScalars* sc = (AcqScalars*)h.data();
+    for (long i = 0; i < S; i++) {
+        sc[i].f = std::numeric_limits<double>::infinity();
+        sc[i].alpha = 1.0;
+        sc[i].best_f = std::numeric_limits<double>::quiet_NaN();
+        sc[i].best_eval = -1;
+        sc[i].steepest = 1;
+    }
+    std::memcpy(h.data() + o_xt, xt0.data(), n_vec);
+    std::memcpy(h.data() + o_lo, lo, d * sizeof(double));
+    std::memcpy(h.data() + o_hi, hi, d * sizeof(double));
+    std::vector<T> rows(Sd), bm((size_t)S, std::numeric_limits<T>::quiet_NaN());
+    for (size_t t = 0; t < Sd; t++) rows[t] = (T)xt0[t];
+    std::memcpy(h.data() + o_bx, rows.data(), Sd * sizeof(T));
+    std::memcpy(h.data() + o_bm, bm.data(), (size_t)S * sizeof(T));
+    const int live0 = (int)S;
+    std::memcpy(h.data() + o_live, &live0, sizeof(int));
+    DevBuf sbuf;
+    sbuf.pool = &e->model_pool;
+    struct Release {
+        DevBuf& b;
+        ~Release() { b.release(); }
+    } release{sbuf};
+    if ((rc = sbuf.ensure(total))) return rc;
+    unsigned char* dp = (unsigned char*)sbuf.p;
+    CUDA_TRY(cudaMemcpyAsync(dp, h.data(), total, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(xs_tmp.p, rows.data(), Sd * sizeof(T), cudaMemcpyHostToDevice, st));
+    AcqState as{(AcqScalars*)dp, (double*)(dp + o_x), (double*)(dp + o_g), (double*)(dp + o_xt), (double*)(dp + o_dir),
+                (double*)(dp + o_s), (double*)(dp + o_y), (double*)(dp + o_a), dp + o_fr, (const double*)(dp + o_lo),
+                (const double*)(dp + o_hi)};
+    T* best_x = (T*)(dp + o_bx);
+    T* best_m = (T*)(dp + o_bm);
+    int* live = (int*)(dp + o_live);
+    YNorm<T> y;
+    double fmin_n;
+    T cb;
+    acquisition_params<T>(mode, yn, param, &y, &fmin_n, &cb);
+    const double ftol = lbfgs_tolerances().ftol, gtol = lbfgs_tolerances().gtol;
+    const T* val = (mode == 0) ? (const T*)acq2.p : (const T*)acq1.p;
+    const T* grd = (mode == 0) ? (const T*)dvar_tmp.p : (const T*)dmean_tmp.p;
+    // one round: all S rows evaluated (the batch has the same shape, and takes the same prediction path, every round),
+    // then one optimiser step per start
+    auto round = [&]() -> int {
+        int r;
+        if ((r = acquisition_device(mode, y, S, fmin_n, cb, true))) return r;
+        k_acq_step<T><<<(unsigned)((S + 127) / 128), 128, 0, st>>>((int)S, d, mode, maxeval, ftol, gtol, val, grd,
+                                                                  (const T*)acq1.p, (T*)xs_tmp.p, as, best_x, best_m, live);
+        e->launches++;
+        CUDA_TRY(cudaGetLastError());
+        return HBEGP_OK;
+    };
+    auto read_live = [&](int* out) -> int {
+        CUDA_TRY(cudaMemcpyAsync(out, live, sizeof(int), cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+        return HBEGP_OK;
+    };
+    // the first round runs as it is: it sizes every buffer a round uses, so the graph below captures final pointers
+    if ((rc = round())) return rc;
+    int hl = 0;
+    if ((rc = read_live(&hl))) return rc;
+    const int R = acq_rounds_per_look();
+    const bool legacy = (st == nullptr || st == cudaStreamLegacy);
+    cudaGraphExec_t exec = nullptr;
+    struct GraphRelease {
+        cudaGraphExec_t& g;
+        ~GraphRelease() { if (g) cudaGraphExecDestroy(g); }
+    } graph_release{exec};
+    long long kernels = 0;
+    while (hl > 0) {
+        if (legacy) {  // no capture on the legacy stream: the same launches, issued one by one
+            for (int k = 0; k < R; k++)
+                if ((rc = round())) return rc;
+        } else {
+            if (!exec) {
+                const long long before = e->launches;
+                CUDA_TRY(cudaStreamBeginCapture(st, cudaStreamCaptureModeRelaxed));
+                int crc = HBEGP_OK;
+                for (int k = 0; k < R && crc == HBEGP_OK; k++) crc = round();
+                cudaGraph_t graph = nullptr;
+                cudaError_t ce = cudaStreamEndCapture(st, &graph);
+                kernels = e->launches - before;
+                e->launches = before;
+                if (crc) {
+                    if (graph) cudaGraphDestroy(graph);
+                    return crc;
+                }
+                if (ce != cudaSuccess) return fail(HBEGP_ERR_CUDA, std::string("cudaStreamEndCapture: ") + cudaGetErrorString(ce));
+                ce = cudaGraphInstantiate(&exec, graph, 0);
+                cudaGraphDestroy(graph);
+                if (ce != cudaSuccess) {
+                    exec = nullptr;
+                    return fail(HBEGP_ERR_CUDA, std::string("cudaGraphInstantiate: ") + cudaGetErrorString(ce));
+                }
+            }
+            CUDA_TRY(cudaGraphLaunch(exec, st));
+            e->launches += kernels;
+        }
+        if ((rc = read_live(&hl))) return rc;
+    }
+    // results: the scalars, the best points and means
+    std::vector<AcqScalars> hsc((size_t)S);
+    CUDA_TRY(cudaMemcpyAsync(hsc.data(), dp, n_sc, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(x_out, best_x, Sd * sizeof(T), cudaMemcpyDeviceToHost, st));
+    if (mean_out && mode == 0) CUDA_TRY(cudaMemcpyAsync(mean_out, best_m, (size_t)S * sizeof(T), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    long long nr = 0;
+    for (long i = 0; i < S; i++) {
+        hbegp_acq_result& res = results[i];
+        const AcqScalars& c = hsc[i];
+        res.n_evals = c.evals;
+        res.best_eval = c.best_eval;
+        if (c.best_eval >= 0) {
+            res.status = HBEGP_OK;
+            res.best_value = (mode == 0) ? -c.best_f : c.best_f;
+        }
+        nr = std::max<long long>(nr, c.rounds);
+    }
+    *n_rounds = nr;
+    *best_index = acq_best_index(mode, S, results);
+    return HBEGP_OK;
 }
 
 template <typename T>
@@ -2522,6 +2743,22 @@ int hbegp_predict_confidence_bound_grad(hbegp_model* model, const hbegp_ynorm* y
     if (!model) return fail(HBEGP_ERR_INVALID, "null model");
     if (!model->m->eng) return fail(HBEGP_ERR_INVALID, "the model's context has been destroyed");
     return model->m->predict_acquisition(1, yn, m, xs, cb, out, nullptr, nullptr, n_below_warn, dout, nullptr);
+}
+
+int hbegp_acquire_ei(hbegp_model* model, const hbegp_ynorm* yn, double fmin, long n_starts, const void* starts, const double* lo,
+                     const double* hi, int maxeval, void* x_out, void* mean_out, hbegp_acq_result* results, long* best_index,
+                     long long* n_rounds) {
+    if (!model || !model->m) return fail(HBEGP_ERR_INVALID, "null model");
+    if (!model->m->eng) return fail(HBEGP_ERR_INVALID, "the model's context has been destroyed");
+    return model->m->acquire(0, yn, fmin, n_starts, starts, lo, hi, maxeval, x_out, mean_out, results, best_index, n_rounds);
+}
+
+int hbegp_acquire_confidence_bound(hbegp_model* model, const hbegp_ynorm* yn, double cb, long n_starts, const void* starts,
+                                   const double* lo, const double* hi, int maxeval, void* x_out, hbegp_acq_result* results,
+                                   long* best_index, long long* n_rounds) {
+    if (!model || !model->m) return fail(HBEGP_ERR_INVALID, "null model");
+    if (!model->m->eng) return fail(HBEGP_ERR_INVALID, "the model's context has been destroyed");
+    return model->m->acquire(1, yn, cb, n_starts, starts, lo, hi, maxeval, x_out, nullptr, results, best_index, n_rounds);
 }
 
 int hbegp_minimize_by_gradient(hbegp_objective_fn objective, void* user, int n, double* x, const double* lo,

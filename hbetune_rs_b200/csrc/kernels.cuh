@@ -1257,6 +1257,253 @@ __global__ void k_pack_round(const double* __restrict__ lml, const double* __res
     }
 }
 
+// ---- the acquisition search (hbegp_acquire_ei / hbegp_acquire_confidence_bound): BoundedLbfgs of lbfgs.h restated for
+// the device, one thread per start, so that the whole search loop stays on the device.  Every operation is the one
+// lbfgs.h performs on the host (built with -ffp-contract=off), in the same order: explicit round-to-nearest double
+// operations keep nvcc from contracting them into FMAs, and std::min / std::max are written as libstdc++'s ternaries
+// (NaN behaviour included).  lbfgs.h's rho is never read there and is not kept here.
+constexpr int kAcqMemory = 10;  // BoundedLbfgs's default memory
+
+// Per-start scalars of the optimiser and of the capture.
+struct AcqScalars {
+    double f, alpha, best_f;
+    long long best_eval;
+    int evals, ls_iter, stall, k, head, have_x, done, steepest, rounds, pad;
+};
+
+// Device state of S starts; arrays are per start, contiguous (d or kAcqMemory * d values each).
+struct AcqState {
+    AcqScalars* sc;
+    double *x, *g, *xt, *dir, *s, *y, *a;  // dir doubles as the two-loop recursion's q, as it is overwritten from it
+    unsigned char* fr;                     // free flags
+    const double *lo, *hi;
+};
+
+__device__ __forceinline__ double acq_min(double a, double b) { return (b < a) ? b : a; }  // std::min
+__device__ __forceinline__ double acq_max(double a, double b) { return (a < b) ? b : a; }  // std::max
+
+struct AcqRun {  // the view of one start: BoundedLbfgs's members
+    AcqScalars& c;
+    double *x, *g, *xt, *dir, *s, *y, *a;
+    unsigned char* fr;
+    const double *lo, *hi;
+    int n, maxeval;
+    double ftol, gtol;
+
+    __device__ double* S(int j) const { return s + (size_t)((c.head + j) % kAcqMemory) * n; }  // j = 0: oldest pair
+    __device__ double* Y(int j) const { return y + (size_t)((c.head + j) % kAcqMemory) * n; }
+    __device__ void clear() { c.k = 0; c.head = 0; }
+    __device__ bool finish() {
+        c.done = 1;
+        return true;
+    }
+
+    __device__ bool make_trial() {
+        if (c.evals >= maxeval) return finish();
+        bool moved = false;
+        for (int i = 0; i < n; i++) {
+            double v = __dadd_rn(x[i], __dmul_rn(c.alpha, dir[i]));
+            v = acq_min(acq_max(v, lo[i]), hi[i]);
+            xt[i] = v;
+            if (v != x[i]) moved = true;
+        }
+        if (!moved) return finish();
+        return false;
+    }
+
+    __device__ bool next_direction(bool force_steepest) {
+        if (c.evals >= maxeval) return finish();
+        double pgmax = 0.0;
+        int nfree = 0;
+        for (int i = 0; i < n; i++) {
+            const bool at_lo = x[i] <= lo[i] && g[i] > 0.0;
+            const bool at_hi = x[i] >= hi[i] && g[i] < 0.0;
+            fr[i] = !(at_lo || at_hi);
+            if (fr[i]) {
+                nfree++;
+                pgmax = acq_max(pgmax, fabs(g[i]));
+            }
+        }
+        if (nfree == 0 || pgmax <= (gtol > 0 ? gtol : 0.0)) return finish();
+        c.steepest = force_steepest || c.k == 0;
+        double* q = dir;
+        for (int i = 0; i < n; i++) q[i] = fr[i] ? g[i] : 0.0;
+        if (!c.steepest) {
+            const int k = c.k;
+            for (int j = k - 1; j >= 0; j--) {
+                const double *Sj = S(j), *Yj = Y(j);
+                double sq = 0, sy = 0;
+                for (int i = 0; i < n; i++)
+                    if (fr[i]) {
+                        sq = __dadd_rn(sq, __dmul_rn(Sj[i], q[i]));
+                        sy = __dadd_rn(sy, __dmul_rn(Sj[i], Yj[i]));
+                    }
+                if (!(sy > 0)) {
+                    a[j] = 0;
+                    continue;
+                }
+                a[j] = __ddiv_rn(sq, sy);
+                for (int i = 0; i < n; i++)
+                    if (fr[i]) q[i] = __dsub_rn(q[i], __dmul_rn(a[j], Yj[i]));
+            }
+            {
+                const double *Sl = S(k - 1), *Yl = Y(k - 1);
+                double sy = 0, yy = 0;
+                for (int i = 0; i < n; i++)
+                    if (fr[i]) {
+                        sy = __dadd_rn(sy, __dmul_rn(Sl[i], Yl[i]));
+                        yy = __dadd_rn(yy, __dmul_rn(Yl[i], Yl[i]));
+                    }
+                const double gamma = (sy > 0 && yy > 0) ? __ddiv_rn(sy, yy) : 1.0;
+                for (int i = 0; i < n; i++) q[i] = __dmul_rn(q[i], gamma);
+            }
+            for (int j = 0; j < k; j++) {
+                const double *Sj = S(j), *Yj = Y(j);
+                double yq = 0, sy = 0;
+                for (int i = 0; i < n; i++)
+                    if (fr[i]) {
+                        yq = __dadd_rn(yq, __dmul_rn(Yj[i], q[i]));
+                        sy = __dadd_rn(sy, __dmul_rn(Sj[i], Yj[i]));
+                    }
+                if (!(sy > 0)) continue;
+                const double beta = __ddiv_rn(yq, sy);
+                for (int i = 0; i < n; i++)
+                    if (fr[i]) q[i] = __dadd_rn(q[i], __dmul_rn(__dsub_rn(a[j], beta), Sj[i]));
+            }
+        }
+        double gd = 0, gnorm1 = 0;
+        for (int i = 0; i < n; i++) {
+            dir[i] = fr[i] ? -q[i] : 0.0;
+            gd = __dadd_rn(gd, __dmul_rn(g[i], dir[i]));
+            if (fr[i]) gnorm1 = __dadd_rn(gnorm1, fabs(g[i]));
+        }
+        if (!(gd < 0) || !isfinite(gd)) {
+            c.steepest = 1;
+            gd = 0;
+            for (int i = 0; i < n; i++) {
+                dir[i] = fr[i] ? -g[i] : 0.0;
+                gd = __dadd_rn(gd, __dmul_rn(g[i], dir[i]));
+            }
+        }
+        c.alpha = c.steepest ? acq_min(1.0, __ddiv_rn(1.0, gnorm1)) : 1.0;
+        c.ls_iter = 0;
+        return make_trial();
+    }
+
+    // BoundedLbfgs::tell; gt(i) is component i of the gradient at xt
+    template <typename G>
+    __device__ bool tell(double ft, const G& gt) {
+        if (c.done) return true;
+        c.evals++;
+        const bool finite = isfinite(ft);
+        if (!c.have_x) {
+            for (int i = 0; i < n; i++) x[i] = xt[i];
+            c.f = ft;
+            c.have_x = 1;
+            if (!finite) return finish();
+            for (int i = 0; i < n; i++) g[i] = gt(i);
+            return next_direction(true);
+        }
+        double dec = 0.0;
+        for (int i = 0; i < n; i++) dec = __dadd_rn(dec, __dmul_rn(g[i], __dsub_rn(xt[i], x[i])));
+        if (!(dec < 0.0)) {
+            if (c.k > 0 || !c.steepest) {
+                clear();
+                return next_direction(true);
+            }
+            return finish();
+        }
+        if (finite && ft <= __dadd_rn(c.f, __dmul_rn(1e-4, dec))) {
+            double sy = 0, ss = 0, yy = 0;
+            for (int i = 0; i < n; i++) {
+                const double si = __dsub_rn(xt[i], x[i]), yi = __dsub_rn(gt(i), g[i]);
+                sy = __dadd_rn(sy, __dmul_rn(si, yi));
+                ss = __dadd_rn(ss, __dmul_rn(si, si));
+                yy = __dadd_rn(yy, __dmul_rn(yi, yi));
+            }
+            if (sy > __dmul_rn(1e-10, __dsqrt_rn(__dmul_rn(ss, yy))) && sy > 0) {
+                // push_back, dropping the oldest pair when the memory is full; s and y are recomputed with the same
+                // operations, so the ring keeps the bits lbfgs.h stores
+                int slot;
+                if (c.k == kAcqMemory) {
+                    slot = c.head;
+                    c.head = (c.head + 1) % kAcqMemory;
+                } else {
+                    slot = (c.head + c.k) % kAcqMemory;
+                    c.k++;
+                }
+                double* Sn = s + (size_t)slot * n;
+                double* Yn = y + (size_t)slot * n;
+                for (int i = 0; i < n; i++) {
+                    Sn[i] = __dsub_rn(xt[i], x[i]);
+                    Yn[i] = __dsub_rn(gt(i), g[i]);
+                }
+            }
+            const double fprev = c.f;
+            for (int i = 0; i < n; i++) x[i] = xt[i];
+            c.f = ft;
+            for (int i = 0; i < n; i++) g[i] = gt(i);
+            const double scale = acq_max(acq_max(fabs(fprev), fabs(c.f)), 1.0);
+            if (ftol > 0 && __dsub_rn(fprev, c.f) <= __dmul_rn(ftol, scale)) c.stall++;
+            else c.stall = 0;
+            if (c.stall >= 2) return finish();
+            return next_direction(false);
+        }
+        c.ls_iter++;
+        double anew;
+        if (finite) {
+            const double denom = __dmul_rn(2.0, __dsub_rn(__dsub_rn(ft, c.f), dec));
+            anew = (denom > 0) ? __ddiv_rn(__dmul_rn(-dec, c.alpha), denom) : __dmul_rn(0.5, c.alpha);
+            anew = acq_min(acq_max(anew, __dmul_rn(0.1, c.alpha)), __dmul_rn(0.5, c.alpha));
+        } else {
+            anew = __dmul_rn(0.25, c.alpha);
+        }
+        c.alpha = anew;
+        if (c.ls_iter > 25 || c.alpha < 1e-18) {
+            if (c.k > 0 || !c.steepest) {
+                clear();
+                return next_direction(true);
+            }
+            return finish();
+        }
+        return make_trial();
+    }
+};
+
+// One step of every start (thread i = start i) after the round evaluated the S rows of xs:
+//   mode 0: f = -EI (val = ei_out), gradient -dei (grad), mean = de-normalised mean (captured with the point);
+//   mode 1: f = the confidence bound (val), gradient grad; mean unused.
+// A live start applies the capture rule of fit_runs_impl (first finite value, then a strictly smaller f), tells the
+// optimiser, and writes its next trial point, rounded to T, back into its row; a finished start changes nothing, so its
+// row keeps its last trial point.  *live counts the starts not done yet.
+template <typename T>
+__global__ void k_acq_step(int S, int d, int mode, int maxeval, double ftol, double gtol, const T* __restrict__ val,
+                           const T* __restrict__ grad, const T* __restrict__ mean, T* __restrict__ xs, AcqState st,
+                           T* __restrict__ best_x, T* __restrict__ best_mean, int* __restrict__ live) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= S) return;
+    AcqScalars& c = st.sc[i];
+    if (c.done) return;
+    const size_t o = (size_t)i * d, om = o * kAcqMemory;
+    AcqRun r{c, st.x + o, st.g + o, st.xt + o, st.dir + o, st.s + om, st.y + om, st.a + (size_t)i * kAcqMemory, st.fr + o,
+             st.lo, st.hi, d, maxeval, ftol, gtol};
+    c.rounds++;
+    const double v = (double)val[i];
+    const double f = (mode == 0) ? -v : v;
+    T* row = xs + o;
+    if (isfinite(f) && (c.best_eval < 0 || f < c.best_f)) {
+        c.best_f = f;
+        c.best_eval = c.evals;
+        for (int k = 0; k < d; k++) best_x[o + k] = row[k];
+        if (mode == 0) best_mean[i] = mean[i];
+    }
+    const T* gr = grad + o;
+    auto gt = [&](int k) -> double { return (mode == 0) ? -(double)gr[k] : (double)gr[k]; };
+    r.tell(f, gt);
+    for (int k = 0; k < d; k++) row[k] = (T)r.xt[k];
+    if (c.done) atomicSub(live, 1);
+}
+
 template <typename T>
 __global__ void k_fill(T* __restrict__ out, long n, T v) {
     long i = (long)blockIdx.x * blockDim.x + threadIdx.x;

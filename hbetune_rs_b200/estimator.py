@@ -195,6 +195,41 @@ class SurrogateModelGPR:
               "hbegp_predict_confidence_bound_grad")
         return out, dout
 
+    def _acquire_args(self, starts, lo, hi):
+        starts = np.ascontiguousarray(np.atleast_2d(starts), dtype=self.A)
+        d = starts.shape[1]
+        lo = np.ascontiguousarray(np.broadcast_to(np.asarray(lo, dtype=np.float64), (d,)))
+        hi = np.ascontiguousarray(np.broadcast_to(np.asarray(hi, dtype=np.float64), (d,)))
+        return starts, lo, hi
+
+    def acquire_ei(self, starts, lo, hi, fmin, maxeval: int = 150):
+        """``hbegp_acquire_ei``: one bounded L-BFGS search maximising EI from each row of ``starts`` over the box
+        [lo, hi], all on the device.  Returns (x, mean, records, best_index, n_rounds): the best point of each start
+        (S x d) and the de-normalised mean there, the ``AcqResult`` records (best_value = EI in normalised units), the
+        winning start (last maximum; -1 if none) and the number of rounds."""
+        starts, lo, hi = self._acquire_args(starts, lo, hi)
+        S, d = starts.shape
+        x, mean = np.empty((S, d), dtype=self.A), np.empty(S, dtype=self.A)
+        res = (_lib.AcqResult * S)()
+        best, rounds = C.c_long(-1), C.c_longlong(0)
+        check(lib.hbegp_acquire_ei(self.fitted.model.single_handle(), C.byref(self.y_norm._raw), float(fmin), S, _ptr(starts),
+                                   _ptr(lo), _ptr(hi), maxeval, _ptr(x), _ptr(mean), res, C.byref(best), C.byref(rounds)),
+              "hbegp_acquire_ei")
+        return x, mean, list(res), best.value, rounds.value
+
+    def acquire_confidence_bound(self, starts, lo, hi, cb, maxeval: int = 150):
+        """``hbegp_acquire_confidence_bound``: one bounded L-BFGS search minimising the de-normalised confidence bound
+        from each row of ``starts``.  Returns (x, records, best_index, n_rounds) (first minimum wins)."""
+        starts, lo, hi = self._acquire_args(starts, lo, hi)
+        S, d = starts.shape
+        x = np.empty((S, d), dtype=self.A)
+        res = (_lib.AcqResult * S)()
+        best, rounds = C.c_long(-1), C.c_longlong(0)
+        check(lib.hbegp_acquire_confidence_bound(self.fitted.model.single_handle(), C.byref(self.y_norm._raw), float(cb), S,
+                                                 _ptr(starts), _ptr(lo), _ptr(hi), maxeval, _ptr(x), res, C.byref(best),
+                                                 C.byref(rounds)), "hbegp_acquire_confidence_bound")
+        return x, list(res), best.value, rounds.value
+
     def predict_mean_ei(self, x, fmin):
         mean, ei = self.predict_mean_ei_a(np.asarray(x)[None, :], fmin)
         return mean[0], ei[0]

@@ -273,6 +273,50 @@ int hbegp_predict_mean_ei_grad(hbegp_model* model, const struct hbegp_ynorm* yn,
 int hbegp_predict_confidence_bound_grad(hbegp_model* model, const struct hbegp_ynorm* yn, long m, const void* xs,
                                         double cb, void* out, void* dout, long* n_below_warn);
 
+/* ---- acquisition search on the device ------------------------------------------------------------
+ * S independent bounded L-BFGS searches over the box lo <= x <= hi (lo, hi: f64, length d), one per start point
+ * (starts[S*d], data type), advancing in lockstep: hbegp_acquire_ei maximises EI, hbegp_acquire_confidence_bound
+ * minimises the de-normalised bound.  An alternative to the reference's BOBYQA searches (SearchingAcquisition::acquire,
+ * suggest_optimum), not a restatement of them: NLopt is not available, so the chosen points are not hbetune's.
+ *  - The optimiser is BoundedLbfgs (the fit's optimiser, memory 10) with the tolerances hbegp_lbfgs_set_tolerances has
+ *    set at call time.  Its objective is -EI with gradient -dei (EI) or the bound with its gradient: the values and
+ *    gradients of hbegp_predict_mean_ei_grad / hbegp_predict_confidence_bound_grad, widened to f64.  A non-finite
+ *    value is a failed trial, as a non-PD matrix is in the fit; a start whose first value is not finite ends at once
+ *    (the log projection with fmin <= expected, a mean that is not finite).
+ *  - Every round evaluates all S rows, in start order; a finished start's row keeps its last trial point and its result
+ *    is ignored.  The batch therefore has the same shape, and takes the same prediction path, in every round: a start's
+ *    bits do not depend on when the others finish.  Each start's steps equal BoundedLbfgs of lbfgs.h bit for bit.
+ *    Starts outside the box are clamped.  f32 models: the optimiser works in f64; the point evaluated is the f64 trial
+ *    rounded to float.
+ *  - Each start keeps the best point it evaluated (the first finite value, then only a strictly better one):
+ *    x_out[S*d] holds it as evaluated, in the data type (the clamped start if there is none), and results[S] its record.
+ *    mean_out[S] (EI only, may be NULL) holds the de-normalised mean there (NaN if there is none).
+ *  - best_index: the last maximum of the EI (find_best_candidate_by_ei, max_by) or the first minimum of the bound
+ *    (minimize.rs:680-714), among the starts with status HBEGP_OK; -1 if there is none.  n_rounds: rounds in which at least
+ *    one start was live.
+ *  - n_starts = 0 is a no-op.  maxeval = 0 evaluates nothing: x_out = the clamped starts, every status HBEGP_NOT_PD,
+ *    best_index -1, n_rounds 0.  HBEGP_ERR_INVALID: a NULL required pointer (all but mean_out), n_starts < 0,
+ *    maxeval < 0, a non-finite start or bound, lo > hi.
+ *  - All rounds run on the device: a round is predict -> acquisition epilogue -> gradients -> one optimiser step per
+ *    start, and the host looks at the count of live starts only every few rounds (a CUDA graph of those rounds).  The
+ *    starts go up and the results come back once per call.
+ *  - An evicted model is rebuilt first.  The search is not a prediction for hbegp_predict_warn_values: the list of the
+ *    last prediction call stays as it was.  One GPU (on a multi model, pass a replica). */
+typedef struct hbegp_acq_result {
+    double best_value;   /* EI: largest EI seen (normalised units, as ei_out of hbegp_predict_mean_ei);
+                            bound: smallest bound seen (de-normalised, as out of hbegp_predict_confidence_bound); NaN if none */
+    long long best_eval; /* 0-based evaluation of this start that first reached it; -1 if no value was finite */
+    long long n_evals;   /* evaluations this start performed (<= maxeval) */
+    int status;          /* HBEGP_OK, or HBEGP_NOT_PD if no evaluation of this start had a finite value */
+    int reserved;
+} hbegp_acq_result;
+int hbegp_acquire_ei(hbegp_model* model, const struct hbegp_ynorm* yn, double fmin, long n_starts, const void* starts,
+                     const double* lo, const double* hi, int maxeval, void* x_out, void* mean_out, hbegp_acq_result* results,
+                     long* best_index, long long* n_rounds);
+int hbegp_acquire_confidence_bound(hbegp_model* model, const struct hbegp_ynorm* yn, double cb, long n_starts,
+                                   const void* starts, const double* lo, const double* hi, int maxeval, void* x_out,
+                                   hbegp_acq_result* results, long* best_index, long long* n_rounds);
+
 /* ---- host-side pieces of the reference interface (no GPU needed) -------------------------------- */
 /* Bounded L-BFGS used by hbegp_fit_runs, exposed with a callback objective
  * (objective(x, grad_out, user) -> f), mirroring minimize_by_gradient (src/util/gradmin.rs:35-60).

@@ -333,6 +333,37 @@ public:
               "hbegp_predict_confidence_bound_grad");
         return out;
     }
+    // hbegp_acquire_ei: S bounded L-BFGS searches maximising EI from the rows of starts (S x d) over [lo, hi]; the best
+    // point of each start into *x (S x d), the de-normalised mean there into *mean (may be NULL), the records into
+    // *results; returns the winning start (-1 if none), the rounds into *n_rounds (may be NULL)
+    long acquire_ei(const std::vector<A>& starts, long S, const std::vector<double>& lo, const std::vector<double>& hi, A fmin,
+                    int maxeval, std::vector<A>* x, std::vector<A>* mean, std::vector<hbegp_acq_result>* results,
+                    long long* n_rounds = nullptr) const {
+        x->assign((size_t)S * d_, A(0));
+        if (mean) mean->assign((size_t)S, A(0));
+        results->assign((size_t)S, hbegp_acq_result{});
+        long best = -1;
+        long long rounds = 0;
+        check(hbegp_acquire_ei(fitted_.model->h, &y_norm_.raw(), (double)fmin, S, starts.data(), lo.data(), hi.data(), maxeval,
+                               x->data(), mean ? mean->data() : nullptr, results->data(), &best, &rounds),
+              "hbegp_acquire_ei");
+        if (n_rounds) *n_rounds = rounds;
+        return best;
+    }
+    // hbegp_acquire_confidence_bound: the same, minimising the de-normalised confidence bound
+    long acquire_confidence_bound(const std::vector<A>& starts, long S, const std::vector<double>& lo, const std::vector<double>& hi,
+                                  A cb, int maxeval, std::vector<A>* x, std::vector<hbegp_acq_result>* results,
+                                  long long* n_rounds = nullptr) const {
+        x->assign((size_t)S * d_, A(0));
+        results->assign((size_t)S, hbegp_acq_result{});
+        long best = -1;
+        long long rounds = 0;
+        check(hbegp_acquire_confidence_bound(fitted_.model->h, &y_norm_.raw(), (double)cb, S, starts.data(), lo.data(), hi.data(),
+                                             maxeval, x->data(), results->data(), &best, &rounds),
+              "hbegp_acquire_confidence_bound");
+        if (n_rounds) *n_rounds = rounds;
+        return best;
+    }
     A predict_confidence_bound(const std::vector<A>& x, A cb) const {
         A out;
         check(hbegp_predict_confidence_bound(fitted_.model->h, &y_norm_.raw(), 1, x.data(), (double)cb, &out, nullptr, nullptr),

@@ -40,6 +40,16 @@ pub const HBEGP_COMM_ID_BYTES: usize = 128;
 
 #[repr(C)]
 #[derive(Clone, Copy, Debug, Default)]
+pub struct hbegp_acq_result {
+    pub best_value: c_double,
+    pub best_eval: c_longlong,
+    pub n_evals: c_longlong,
+    pub status: c_int,
+    pub reserved: c_int,
+}
+
+#[repr(C)]
+#[derive(Clone, Copy, Debug, Default)]
 pub struct hbegp_run_result {
     pub best_lml: c_double,
     pub best_eval: c_longlong,
@@ -217,6 +227,18 @@ extern "C" {
     pub fn hbegp_predict_confidence_bound_grad(
         model: *mut hbegp_model, yn: *const hbegp_ynorm, m: c_long, xs: *const c_void, cb: c_double,
         out: *mut c_void, dout: *mut c_void, n_below_warn: *mut c_long,
+    ) -> c_int;
+
+    // acquisition search on the device: S bounded L-BFGS searches in lockstep (see hbegp.h)
+    pub fn hbegp_acquire_ei(
+        model: *mut hbegp_model, yn: *const hbegp_ynorm, fmin: c_double, n_starts: c_long, starts: *const c_void,
+        lo: *const c_double, hi: *const c_double, maxeval: c_int, x_out: *mut c_void, mean_out: *mut c_void,
+        results: *mut hbegp_acq_result, best_index: *mut c_long, n_rounds: *mut c_longlong,
+    ) -> c_int;
+    pub fn hbegp_acquire_confidence_bound(
+        model: *mut hbegp_model, yn: *const hbegp_ynorm, cb: c_double, n_starts: c_long, starts: *const c_void,
+        lo: *const c_double, hi: *const c_double, maxeval: c_int, x_out: *mut c_void, results: *mut hbegp_acq_result,
+        best_index: *mut c_long, n_rounds: *mut c_longlong,
     ) -> c_int;
 
     pub fn hbegp_minimize_by_gradient(
