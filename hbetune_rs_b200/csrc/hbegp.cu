@@ -22,6 +22,7 @@
 #include <string>
 #include <thread>
 #include <tuple>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/hbegp.h"
@@ -290,14 +291,40 @@ inline void EngineBase::evict_old_models() {
     }
 }
 
+// nu -> NU2 of the kernel instantiations: 2 nu for the Matern orders 1/2, 3/2 and 5/2, kNu2Rbf for nu = +inf (the
+// squared exponential, which sklearn's Matern(nu=inf) also is).  NaN, -inf and any other nu are unsupported.
 static int nu_to_nu2(double nu, int* nu2) {
     const double eps = std::numeric_limits<double>::epsilon();
-    if (std::fabs(nu - 0.5) <= eps) *nu2 = 1;
+    if (nu == std::numeric_limits<double>::infinity()) *nu2 = kNu2Rbf;
+    else if (std::fabs(nu - 0.5) <= eps) *nu2 = 1;
     else if (std::fabs(nu - 1.5) <= eps) *nu2 = 3;
     else if (std::fabs(nu - 2.5) <= eps) *nu2 = 5;
     else return fail(HBEGP_ERR_UNSUPPORTED, "Matern kernel with arbitrary values for nu (matern_kernel.rs:79)");
     return HBEGP_OK;
 }
+
+// The NU2 values the kernels are instantiated for.  with_nu2 and for_each_nu2 are the only code that maps a nu2 to an
+// instantiation; f is called with std::integral_constant<int, NU2>.
+template <int... N>
+struct Nu2Set {
+    template <typename F>
+    static int with(int nu2, F&& f) {  // f(NU2 == nu2); HBEGP_ERR_UNSUPPORTED for a nu2 without kernels
+        int rc = HBEGP_OK;
+        const bool found = ((nu2 == N && (rc = f(std::integral_constant<int, N>()), true)) || ...);
+        return found ? rc : fail(HBEGP_ERR_UNSUPPORTED, "no kernels for nu2 = " + std::to_string(nu2));
+    }
+    template <typename F>
+    static int each(F&& f) {  // f(NU2) for every NU2 in order, up to the first error
+        int rc = HBEGP_OK;
+        ((rc = rc ? rc : f(std::integral_constant<int, N>())), ...);
+        return rc;
+    }
+};
+using KernelNu2s = Nu2Set<1, 3, 5, kNu2Rbf>;
+template <typename F>
+static int with_nu2(int nu2, F&& f) { return KernelNu2s::with(nu2, std::forward<F>(f)); }
+template <typename F>
+static int for_each_nu2(F&& f) { return KernelNu2s::each(std::forward<F>(f)); }
 
 template <typename T>
 struct ModelT;
@@ -664,9 +691,7 @@ struct Engine : EngineBase {
         // large n with many matrices per group: the GEMMs fill the GPU on their own
         constexpr int SIDE_MAX_CNT = 4;  // at n > 2048 the side stream serves groups of at most this many matrices
         if (!((np <= 2048 || cnt <= SIDE_MAX_CNT) && np > TILE)) sd = Side();
-        if (nu2 == 5) return pipeline_nu<5>(st, s0, cnt, want_grad, want_kinv, sd);
-        if (nu2 == 3) return pipeline_nu<3>(st, s0, cnt, want_grad, want_kinv, sd);
-        return pipeline_nu<1>(st, s0, cnt, want_grad, want_kinv, sd);
+        return with_nu2(nu2, [&](auto nu) { return pipeline_nu<decltype(nu)::value>(st, s0, cnt, want_grad, want_kinv, sd); });
     }
 
     int n_groups(int cnt) const {
@@ -901,9 +926,7 @@ struct Engine : EngineBase {
         if (dd <= 0 || !theta || n1 < 0 || n2 < 0 || ((n1 > 0 && n2 > 0) && (!x1 || !x2 || !out))) return fail(HBEGP_ERR_INVALID, "kernel_matrix: bad arguments");
         if (n1 == 0 || n2 == 0) return HBEGP_OK;
         CUDA_TRY(cudaSetDevice(device));
-        if (nu2 == 5) return kernel_matrix_nu<5>(dd, theta, n1, x1, n2, x2, out);
-        if (nu2 == 3) return kernel_matrix_nu<3>(dd, theta, n1, x1, n2, x2, out);
-        return kernel_matrix_nu<1>(dd, theta, n1, x1, n2, x2, out);
+        return with_nu2(nu2, [&](auto nu) { return kernel_matrix_nu<decltype(nu)::value>(dd, theta, n1, x1, n2, x2, out); });
     }
 
     // trait Kernel::theta_grad(x) -> (K (n, n), dK/dtheta (n, n, d + 1)) (kernel.rs:16-21, product_kernel.rs:40-70).
@@ -931,9 +954,11 @@ struct Engine : EngineBase {
         if (ce == cudaSuccess) ce = cudaMemcpyAsync(dls.p, ls_h.data(), (size_t)dd * sizeof(T), cudaMemcpyHostToDevice, st);
         if (ce != cudaSuccess) return done(fail(HBEGP_ERR_CUDA, std::string("kernel_theta_grad: ") + cudaGetErrorString(ce)));
         dim3 grid((unsigned)((nn + 127) / 128), (unsigned)nn);
-        if (nu2 == 5) k_kernel_theta_grad<T, 5><<<grid, 128, 0, st>>>((const T*)dx.p, (int)nn, dd, (const T*)dls.p, c, (T*)dk.p, (T*)dg.p);
-        else if (nu2 == 3) k_kernel_theta_grad<T, 3><<<grid, 128, 0, st>>>((const T*)dx.p, (int)nn, dd, (const T*)dls.p, c, (T*)dk.p, (T*)dg.p);
-        else k_kernel_theta_grad<T, 1><<<grid, 128, 0, st>>>((const T*)dx.p, (int)nn, dd, (const T*)dls.p, c, (T*)dk.p, (T*)dg.p);
+        rc = with_nu2(nu2, [&](auto nu) {
+            k_kernel_theta_grad<T, decltype(nu)::value><<<grid, 128, 0, st>>>((const T*)dx.p, (int)nn, dd, (const T*)dls.p, c, (T*)dk.p, (T*)dg.p);
+            return HBEGP_OK;
+        });
+        if (rc) return done(rc);
         launches++;
         ce = cudaGetLastError();
         if (ce == cudaSuccess && k_out) ce = cudaMemcpyAsync(k_out, dk.p, (size_t)nn * nn * sizeof(T), cudaMemcpyDeviceToHost, st);
@@ -973,9 +998,12 @@ struct Engine : EngineBase {
             return HBEGP_OK;
         };
         k_scale_x<T><<<dim3((np + 255) / 256, d, 1), 256, 0, stream>>>((const T*)dX.p, (int)n, d, np, (T*)prm.p, p(), (T*)xsT.p);
-        if (nu2 == 5) k_assemble<T, 5><<<dim3(ntiles_lower(), 1, 1), 256, xsm, stream>>>((T*)xsT.p, (int)n, d, np, (T*)prm.p, p(), (T*)A.p, mstride(), 0);
-        else if (nu2 == 3) k_assemble<T, 3><<<dim3(ntiles_lower(), 1, 1), 256, xsm, stream>>>((T*)xsT.p, (int)n, d, np, (T*)prm.p, p(), (T*)A.p, mstride(), 0);
-        else k_assemble<T, 1><<<dim3(ntiles_lower(), 1, 1), 256, xsm, stream>>>((T*)xsT.p, (int)n, d, np, (T*)prm.p, p(), (T*)A.p, mstride(), 0);
+        rc = with_nu2(nu2, [&](auto nu) {
+            k_assemble<T, decltype(nu)::value><<<dim3(ntiles_lower(), 1, 1), 256, xsm, stream>>>((T*)xsT.p, (int)n, d, np, (T*)prm.p, p(),
+                                                                                             (T*)A.p, mstride(), 0);
+            return HBEGP_OK;
+        });
+        if (rc) { tmp.release(); return rc; }
         CUDA_TRY(cudaGetLastError());
         if (k && (rc = copy_out((T*)A.p, k, 1))) { tmp.release(); return rc; }
         if ((rc = chol_inv(stream, 0, 1, 0, np))) { tmp.release(); return rc; }
@@ -1116,9 +1144,7 @@ struct ModelT : Model {
         if (var && (rc = warn_vals.ensure(kWarnCap * sizeof(T)))) return rc;
         unsigned long long* nb = n_below_device ? (unsigned long long*)n_below_device : (unsigned long long*)nbelow.p;
         if (var) CUDA_TRY(cudaMemsetAsync(nb, 0, sizeof(unsigned long long), e->stream));
-        if (nu2 == 5) return predict_impl<5>(m, (const T*)xs, (T*)mean, (T*)var, nb);
-        if (nu2 == 3) return predict_impl<3>(m, (const T*)xs, (T*)mean, (T*)var, nb);
-        return predict_impl<1>(m, (const T*)xs, (T*)mean, (T*)var, nb);
+        return with_nu2(nu2, [&](auto nu) { return predict_impl<decltype(nu)::value>(m, (const T*)xs, (T*)mean, (T*)var, nb); });
     }
 
     int predict_acquisition(int mode, const hbegp_ynorm* yn, long m, const void* xs, double param, void* out1, void* out2,
@@ -1219,9 +1245,7 @@ struct ModelT : Model {
     }
 
     int predict_grad_device(long m, const T* xs, const T* var, T* dmean, T* dvar) {
-        if (nu2 == 5) return predict_grad_impl<5>(m, xs, var, dmean, dvar);
-        if (nu2 == 3) return predict_grad_impl<3>(m, xs, var, dmean, dvar);
-        return predict_grad_impl<1>(m, xs, var, dmean, dvar);
+        return with_nu2(nu2, [&](auto nu) { return predict_grad_impl<decltype(nu)::value>(m, xs, var, dmean, dvar); });
     }
 
     int predict_grad_host(long m, const void* xs, void* mean, void* var, void* dmean, void* dvar, long* n_below) override {
@@ -1314,7 +1338,7 @@ struct ModelT : Model {
 
     int ensure_resident() override {
         if (!evicted) return HBEGP_OK;
-        int rc = (nu2 == 5) ? rebuild_nu<5>() : (nu2 == 3) ? rebuild_nu<3>() : rebuild_nu<1>();
+        int rc = with_nu2(nu2, [&](auto nu) { return rebuild_nu<decltype(nu)::value>(); });
         if (rc == HBEGP_OK) {
             // it is the most recently used model now: move it to the back and let the policy drop another one
             auto& ms = eng->models;
@@ -1890,9 +1914,7 @@ int Engine<T>::model_extend(Model* prior_, Model** out, double* lml, void* alpha
     if (r1 == 0) {  // different rows or row order: the full evaluation
         if ((rc = run_chunk(nu2, 1, false, want_kinv))) return rc;
     } else {
-        if (nu2 == 5) rc = append_nu<5>(prior, r1, want_kinv);
-        else if (nu2 == 3) rc = append_nu<3>(prior, r1, want_kinv);
-        else rc = append_nu<1>(prior, r1, want_kinv);
+        rc = with_nu2(nu2, [&](auto nu) { return append_nu<decltype(nu)::value>(prior, r1, want_kinv); });
         if (rc) return rc;
         if (appended) *appended = 1;
     }
@@ -1938,19 +1960,14 @@ static int configure_gemms() {
     const int big = (int)kMaxFeatureSmem;
     CUDA_TRY(cudaFuncSetAttribute(k_leaf<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)leaf_smem_bytes<T>()));
     CUDA_TRY(cudaFuncSetAttribute(k_node128_v2<false, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)node128_v2_smem_bytes()));
-    CUDA_TRY(cudaFuncSetAttribute(k_assemble<T, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-    CUDA_TRY(cudaFuncSetAttribute(k_assemble<T, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-    CUDA_TRY(cudaFuncSetAttribute(k_assemble<T, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-    CUDA_TRY(cudaFuncSetAttribute(k_grad_contract<T, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-    CUDA_TRY(cudaFuncSetAttribute(k_grad_contract<T, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-    CUDA_TRY(cudaFuncSetAttribute(k_grad_contract<T, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-    CUDA_TRY(cudaFuncSetAttribute(k_kstar_mean<T, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-    CUDA_TRY(cudaFuncSetAttribute(k_kstar_mean<T, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-    CUDA_TRY(cudaFuncSetAttribute(k_kstar_mean<T, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-    CUDA_TRY(cudaFuncSetAttribute(k_kstar_grad<T, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-    CUDA_TRY(cudaFuncSetAttribute(k_kstar_grad<T, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-    CUDA_TRY(cudaFuncSetAttribute(k_kstar_grad<T, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-    return HBEGP_OK;
+    return for_each_nu2([&](auto nu) {
+        constexpr int NU2 = decltype(nu)::value;
+        CUDA_TRY(cudaFuncSetAttribute(k_assemble<T, NU2>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
+        CUDA_TRY(cudaFuncSetAttribute(k_grad_contract<T, NU2>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
+        CUDA_TRY(cudaFuncSetAttribute(k_kstar_mean<T, NU2>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
+        CUDA_TRY(cudaFuncSetAttribute(k_kstar_grad<T, NU2>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
+        return HBEGP_OK;
+    });
 }
 
 // ------------------------------------------------------------------------------------ restart loop

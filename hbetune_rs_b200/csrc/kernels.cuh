@@ -47,9 +47,13 @@ __device__ __forceinline__ double dev_log<double>(double x) { return log(x); }
 template <>
 __device__ __forceinline__ float dev_log<float>(float x) { return logf(x); }
 
+// NU2 of nu = +inf, the squared exponential (RBF) kernel; every other NU2 is 2 * nu.
+constexpr int kNu2Rbf = 0;
+
 // Matern correlation from the scaled distance r (src/gpr/matern_kernel.rs:65-80).  NU2 = 2 * nu.
 template <typename T, int NU2>
 __device__ __forceinline__ T matern_corr(T r) {
+    static_assert(NU2 == 1 || NU2 == 3 || NU2 == 5, "matern_corr: finite nu only (corr_from_sq for the RBF)");
     if (NU2 == 1) return dev_exp<T>(-r);
     if (NU2 == 3) {
         T k = r * T(1.7320508075688772935);
@@ -59,12 +63,23 @@ __device__ __forceinline__ T matern_corr(T r) {
     return (T(1) + k + k * k / T(3)) * dev_exp<T>(-k);
 }
 
+// Correlation from the squared scaled distance s = sum_k (x~_ik - x~_jk)^2.  RBF: exp(-0.5 s) (sklearn's RBF; the
+// product by 0.5 is exact and no square root is taken); finite nu: exactly matern_corr(sqrt(s)).
+template <typename T, int NU2>
+__device__ __forceinline__ T corr_from_sq(T s) {
+    if constexpr (NU2 == kNu2Rbf) return dev_exp<T>(T(-0.5) * s);
+    else return matern_corr<T, NU2>(dev_sqrt<T>(s));
+}
+
 // Per-entry terms of the theta gradient (src/gpr/matern_kernel.rs:83-135) from s = sum_k d_ijk,
 // d_ijk = (x_ik - x_jk)^2 / l_k^2: kval = the correlation recomputed from t = sqrt(2 nu s), and dk_factor such that
-// dM_ij / d ln l_k = dk_factor * d_ijk.
+// dM_ij / d ln l_k = dk_factor * d_ijk.  RBF: kval = exp(-0.5 s) and dk_factor = -2 dM/ds = kval.
 template <typename T, int NU2>
 __device__ __forceinline__ void matern_grad_terms(T s, T& kval, T& dk_factor) {
-    if (NU2 == 5) {
+    if constexpr (NU2 == kNu2Rbf) {
+        kval = dev_exp<T>(T(-0.5) * s);
+        dk_factor = kval;
+    } else if (NU2 == 5) {
         const T t = dev_sqrt<T>(T(5) * s);
         const T e = dev_exp<T>(-t);
         kval = (T(1) + t + t * t / T(3)) * e;
@@ -75,6 +90,7 @@ __device__ __forceinline__ void matern_grad_terms(T s, T& kval, T& dk_factor) {
         kval = (t + T(1)) * e;
         dk_factor = T(3) * e;  // matern_kernel.rs:112-118
     } else {
+        static_assert(NU2 == 1 || NU2 == 3 || NU2 == 5, "matern_grad_terms: unknown NU2");
         const T r = dev_sqrt<T>(s);
         kval = dev_exp<T>(-r);
         dk_factor = (r > T(0)) ? kval / r : T(0);  // matern_kernel.rs:102-111 (non-finite -> 0)
@@ -167,7 +183,7 @@ __global__ void __launch_bounds__(256) k_assemble(const T* __restrict__ xsT, int
             T v;
             if (gi >= n || gj >= n) v = (gi == gj) ? T(1) : T(0);
             else {
-                v = c * matern_corr<T, NU2>(dev_sqrt<T>(acc[a][q]));
+                v = c * corr_from_sq<T, NU2>(acc[a][q]);
                 if (gi == gj) v += noise;
             }
             Kb[(long)gi * np + gj] = v;
@@ -671,7 +687,7 @@ __global__ void __launch_bounds__(256) k_kstar_mean(const T* __restrict__ xs, lo
 #pragma unroll
             for (int q = 0; q < 4; q++) {
                 const int gj = j0 + tx + 16 * q;
-                T v = (gj < n) ? c * matern_corr<T, NU2>(dev_sqrt<T>(acc[a][q])) : T(0);
+                T v = (gj < n) ? c * corr_from_sq<T, NU2>(acc[a][q]) : T(0);
                 macc[a] += v * al[tx + 16 * q];
                 if (kstar != nullptr) kstar[(r0 + ty + 16 * a) * (long)np + gj] = v;
             }
@@ -716,7 +732,7 @@ __global__ void __launch_bounds__(256) k_kstar_small(const T* __restrict__ xs, i
                 const T df = xc[r * d + k] - xsT_train[(long)k * np + j];
                 acc += df * df;
             }
-            const T v = (j < n) ? c * matern_corr<T, NU2>(dev_sqrt<T>(acc)) : T(0);
+            const T v = (j < n) ? c * corr_from_sq<T, NU2>(acc) : T(0);
             if (kstar != nullptr) kstar[(long)r * np + j] = v;
             contrib = v * aj;
         }
@@ -829,7 +845,8 @@ __global__ void k_var_finish(const T* __restrict__ part, int ld, int ntiles, lon
 // matern_grad_terms:  d k*_j / d x_k = -c dk_factor(s_j) (x~_k - X~_jk) / l_k, so
 //   dmean_k = -(c / l_k) sum_j alpha_j dk_factor_j (x~_k - X~_jk),
 //   dvar_k  =  (2 c / l_k) sum_j v_j dk_factor_j (x~_k - X~_jk),   v = K^-1 k* = W^T (W k*).
-// At s = 0 (a candidate on a training point) every Matern order contributes 0 (nu = 1/2: dk_factor is 0 there).
+// At s = 0 (a candidate on a training point) every Matern order and the RBF contribute 0 (nu = 1/2: dk_factor is 0
+// there; elsewhere x~_k - X~_jk is).
 
 // u[r][i] = sum_{k <= i} W[i][k] k*[r][k] for the 16 candidates of group blockIdx.y: k_wmatvec_small with u stored
 // instead of squared (latency path of the variance gradient).
@@ -1223,7 +1240,7 @@ __global__ void k_kernel_theta_grad(const T* __restrict__ x, int n, int d, const
         const T df = x[(long)i * d + k] / ls[k] - x[(long)j * d + k] / ls[k];  // division first (matern_kernel.rs:51-60)
         r2 += df * df;
     }
-    const T kij = c * matern_corr<T, NU2>(dev_sqrt<T>(r2));
+    const T kij = c * corr_from_sq<T, NU2>(r2);
     if (k_out) k_out[(long)i * n + j] = kij;
     if (!grad) return;
     // like k_grad_contract, d_ijk is formed from the scaled inputs ((x_ik / l_k - x_jk / l_k)^2; the reference squares

@@ -77,7 +77,8 @@ class ConstantKernel:
 
 
 class Matern:
-    """``src/gpr/matern_kernel.rs:12-187`` (parameters only; nu in {0.5, 1.5, 2.5})."""
+    """``src/gpr/matern_kernel.rs:12-187`` (parameters only; nu in {0.5, 1.5, 2.5}, or ``math.inf`` for the squared
+    exponential (RBF) kernel exp(-0.5 |x / l - x' / l|^2), sklearn's ``RBF`` and ``Matern(nu=np.inf)``)."""
 
     def __init__(self, nu: float, length_scale: Sequence[BoundedValue]):
         self.nu = nu

@@ -34,7 +34,7 @@ extern "C" {
 #define HBEGP_ERR_INVALID (-1)    /* bad argument / call order */
 #define HBEGP_ERR_CUDA (-2)       /* CUDA runtime failure (incl. no device) */
 #define HBEGP_ERR_NOMEM (-3)      /* device memory exhausted */
-#define HBEGP_ERR_UNSUPPORTED (-4)/* e.g. Matern nu other than 0.5 / 1.5 / 2.5 */
+#define HBEGP_ERR_UNSUPPORTED (-4)/* e.g. nu other than 0.5 / 1.5 / 2.5 / +INFINITY (NaN and -INFINITY included) */
 #define HBEGP_ERR_NO_CAPTURE (-5) /* fit: no evaluation succeeded (fit.rs:161 unwrap panic) */
 
 typedef struct hbegp_ctx hbegp_ctx;
@@ -72,7 +72,14 @@ int hbegp_set_data(hbegp_ctx* ctx, long n, int d, const void* x, const void* y);
 int hbegp_set_data_device(hbegp_ctx* ctx, long n, int d, const void* x_device, const void* y_device);
 
 /* ---- LML + gradient, batched over thetas ------------------------------------------------------- */
-/* B evaluations of src/gpr/lml.rs:29-79 for Product<ConstantKernel, Matern(nu)> + noise, one per theta
+/* Every `nu` argument selects the correlation M of the kernel c M + noise I: nu = 0.5, 1.5, 2.5 the Matern orders of
+ * src/gpr/matern_kernel.rs:65-80 (of r = sqrt(s)), nu = +INFINITY the squared exponential (RBF; sklearn's RBF, which
+ * sklearn's Matern(nu=inf) also is) M = exp(-0.5 s), the product by 0.5 exact and no square root taken.  In both,
+ * s = sum_k (x_ik / l_k - x_jk / l_k)^2 (division first, features summed left to right), and K_ii = c + noise.  The
+ * RBF's theta gradient is dK/d ln c = c M and dK/d ln l_k = c M (x_ik - x_jk)^2 / l_k^2 (sklearn's anisotropic RBF).  A
+ * model keeps its nu through extend, rebuild, replicas, predictions, gradients and the acquisition searches.
+ *
+ * B evaluations of src/gpr/lml.rs:29-79 for Product<ConstantKernel, Matern(nu)> + noise, one per theta
  * row.  `lo`/`hi` (natural units, length p, may be NULL) clamp exp(theta[1..]) like with_clamped_theta
  * (src/gpr/fit.rs:95; noise is not clamped).  Outputs: lml[B]; grad[B*p] (may be NULL: value only);
  * status[B] in {HBEGP_OK, HBEGP_NOT_PD}; on NOT_PD lml = -inf and grad = 0 (fit.rs:103-113 returns +inf
@@ -251,7 +258,8 @@ int hbegp_predict_confidence_bound(hbegp_model* model, const struct hbegp_ynorm*
  *   dmean = sum_j alpha_j grad k*_j,   dvar = -2 sum_j v_j grad k*_j,  v = K^-1 k*  (normalised units).
  * Definitions where the functions are not smooth:
  *   - a term with s_j = 0 (the candidate on a training point) contributes 0, for every nu (for nu = 1/2 the
- *     derivative does not exist there; the reference's non-finite -> 0 rule gives 0);
+ *     derivative does not exist there; the reference's non-finite -> 0 rule gives 0; for the other orders and the
+ *     RBF, whose dk_factor = M, 0 is the derivative);
  *   - where the variance is clamped to 0 (its pre-clamp value is < 0, or exactly 0), dvar = 0;
  *   - d sqrt(var) = dvar / (2 sqrt(var)) where sqrt(var) > 0, else 0;
  *   - EI (f64, normalised units): -Phi(z) dmean + phi(z) d sqrt(var); in the std-zero branch -dmean where
